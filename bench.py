@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline measurement of the geometric hot path on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--extras 0|1]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--extras 0|1] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1], "C2"): knn_point k=16, 16384 queries vs 16384 refs, batch 8,
 on synthetic HDL-64-shaped frame pairs (b200pc.synth, seeds fixed by pair index).  One "step" is one
@@ -57,7 +57,15 @@ def parse():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--extras", type=int, default=1, help="also time the other kernels of the path (rank 0)")
     ap.add_argument("--ref-queries", type=int, default=0, help="(--impl reference) queries per step; 0 = automatic")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, so that two builds can be "
+                         "compared output for output on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the timed CUDA path (--impl b200)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -665,9 +673,18 @@ def main():
     if rank == 0:
         sampler.start()
     ops.launch_count = 0
-    secs = timed_steps(lambda: P.knn_point(K_NN, ref, qry), args.steps, args.warmup, flush, torch.cuda.synchronize, barrier)
+    last = []
+
+    def step():
+        last[:] = [P.knn_point(K_NN, ref, qry)]
+    secs = timed_steps(step, args.steps, args.warmup, flush, torch.cuda.synchronize, barrier)
     abi_calls = ops.launch_count
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # [BATCH, NPTS, K_NN] neighbour indices of rank 0's frame pairs: 8 MB in float32, exact since they are < 2^24
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "knn_point_idx.npy"), last[0].cpu().numpy().astype(np.float32))
+    del last
     # sustained rate: the same call back to back for >= 2 s (no flush in between: the kernel reads 3 MB, it is not
     # memory bound), clocks sampled over that window
     sustained = None
