@@ -101,7 +101,7 @@ int b200pc_three_nn(const float *unknown, const float *known, int B, int N, int 
 int b200pc_three_interpolate(const float *feat, const int64_t *idx, const float *weight, int B, int S, int N,
                              int C, float *out, b200pc_stream_t stream);
 /* gradients: gfeat [B,S,C] must be zero-filled by the caller (atomic accumulation);
- * gweight [B,N,3] may be NULL. */
+ * gweight [B,N,3] may be NULL.  A neighbour out of range after one wrap gets no gradient (gweight 0, nothing into gfeat). */
 int b200pc_three_interpolate_bwd(const float *gout, const float *feat, const int64_t *idx, const float *weight,
                                  int B, int S, int N, int C, float *gfeat, float *gweight,
                                  b200pc_stream_t stream);
@@ -149,7 +149,8 @@ int b200pc_gather_bwd(const float *gout, const int64_t *idx, int B, int N, int C
 int b200pc_group_points(const float *xyz, const float *new_xyz, const float *feat, const int64_t *idx, int B, int N,
                         int S, int K, int D, int xyz_first, float *out, b200pc_stream_t stream);
 /* grad_feat [B,N,D] must be zero-filled by the caller:
- * grad_feat[b, idx[b,s,k], d] += grad_out[b, (xyz_first ? 3 : 0) + d, k, s]                  */
+ * grad_feat[b, idx[b,s,k], d] += grad_out[b, (xyz_first ? 3 : 0) + d, k, s]
+ * Out-of-range slots (after one wrap) get no gradient.                                       */
 int b200pc_group_points_bwd(const float *grad_out, const int64_t *idx, int B, int N, int S, int K, int D,
                             int xyz_first, float *grad_feat, b200pc_stream_t stream);
 

@@ -277,7 +277,9 @@ def _group_setup(ctx, inputs, output):
 def _group_backward(ctx, gout):
     """differentiable in the features through the scatter kernel (what the reference's models train through); the
     coordinates get their gradient from the same three terms the unfused graph would produce, built with torch ops
-    on the three xyz channels."""
+    on the three xyz channels.  A slot whose index is still out of range after one wrap (the ball query's empty-ball
+    sentinel N, for one) was filled with zeros by the forward pass: it gives xyz no gradient, while new_xyz still gets
+    -gout there, because that output is 0 - centre."""
     (idx,) = ctx.saved_tensors
     N, D, xyz_first = ctx.N, ctx.D, ctx.xyz_first
     B, _, K, S = gout.shape
@@ -291,8 +293,9 @@ def _group_backward(ctx, gout):
             gnew = -gx.sum(dim=2).transpose(1, 2).contiguous()            # [B,S,3]
         if ctx.needs_input_grad[0]:
             rows = gx.permute(0, 3, 2, 1).reshape(B, S * K, 3)
-            flat = torch.where(idx < 0, idx + N, idx).reshape(B, S * K, 1).expand(-1, -1, 3)
-            gxyz = torch.zeros(B, N, 3, dtype=torch.float32, device=gout.device).scatter_add_(1, flat, rows)
+            flat = torch.where(idx < 0, idx + N, idx).reshape(B, S * K, 1)
+            flat = torch.where((flat >= 0) & (flat < N), flat, N).expand(-1, -1, 3)      # dropped slots land in spare row N
+            gxyz = torch.zeros(B, N + 1, 3, dtype=torch.float32, device=gout.device).scatter_add_(1, flat, rows)[:, :N]
     return gxyz, gnew, gfeat, None, None
 
 

@@ -264,6 +264,8 @@ __global__ void __launch_bounds__(256) interp_scalar_kernel(const float *__restr
 }
 
 // gradient: one warp per dense row.  gfeat[b,i_j,:] += gout*w_j ; gweight[b,n,j] = <gout, feat[i_j]>
+// A neighbour the forward pass dropped (index out of range after one wrap) contributed nothing: it gets no gfeat add and
+// gweight 0.
 __global__ void __launch_bounds__(256) interp_bwd_kernel(const float *__restrict__ gout, const float *__restrict__ feat,
                                                          const int64_t *__restrict__ idx, const float *__restrict__ w, int S,
                                                          int C, long N, long rows, float *__restrict__ gfeat,
@@ -275,13 +277,22 @@ __global__ void __launch_bounds__(256) interp_bwd_kernel(const float *__restrict
         const long b = row / N;
         long id[3];
         float ww[3], acc[3] = {0.f, 0.f, 0.f};
+        bool ok[3];                                      // warp-uniform: the whole warp works on one row
 #pragma unroll
-        for (int j = 0; j < 3; ++j) { id[j] = idx[row * 3 + j]; ww[j] = w[row * 3 + j]; clean_neighbour(id[j], ww[j], S); }
+        for (int j = 0; j < 3; ++j) {
+            long i = idx[row * 3 + j];
+            if (i < 0) i += S;
+            ok[j] = i >= 0 && i < S;
+            id[j] = ok[j] ? i : 0;
+            ww[j] = w[row * 3 + j];
+        }
         for (int c = lane; c < C; c += 32) {
             const float g = gout[row * C + c];
 #pragma unroll
             for (int j = 0; j < 3; ++j) {
+                if (!ok[j]) continue;
                 const long o = (b * S + id[j]) * C + c;
+                B200PC_DEV_ASSERT(id[j] >= 0 && id[j] < S);
                 atomicAdd(gfeat + o, g * ww[j]);
                 if (gweight) acc[j] += g * feat[o];
             }
@@ -292,7 +303,7 @@ __global__ void __launch_bounds__(256) interp_bwd_kernel(const float *__restrict
                 float a = acc[j];
 #pragma unroll
                 for (int o = 16; o > 0; o >>= 1) a += __shfl_xor_sync(0xffffffffu, a, o);
-                if (lane == 0) gweight[row * 3 + j] = a;
+                if (lane == 0) gweight[row * 3 + j] = ok[j] ? a : 0.0f;
             }
         }
     }

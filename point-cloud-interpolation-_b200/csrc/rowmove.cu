@@ -217,6 +217,7 @@ int group_bulk(const float *xyz, const float *new_xyz, const float *feat, const 
         while (ksplit < K && base_units * ksplit < 6 * warps_guess) ksplit <<= 1;
         if (ksplit > K) ksplit = K;
         kper = (K + ksplit - 1) / ksplit;
+        ksplit = (K + kper - 1) / kper;                                  // e.g. K = 10, 8 parts of 2 slots: only 5 hold any
         units = base_units * ksplit;
         const size_t idx_bytes = ((size_t)32 * (kper | 1) * 4 + 127) & ~(size_t)127;
         int w1 = (int)(RM_SMEM_BUDGET / (idx_bytes + tile)), w2 = (int)(RM_SMEM_BUDGET / (idx_bytes + 2 * tile));
@@ -225,6 +226,9 @@ int group_bulk(const float *xyz, const float *new_xyz, const float *feat, const 
         if (nwarps > GR_MAX_WARPS) nwarps = GR_MAX_WARPS;
         if (nwarps < 4 || (!force && nwarps < GR_MAX_WARPS)) return -100;
     }
+    // the kernel re-derives kper from ksplit; every part it numbers must start inside [0, K)
+    B200PC_REQUIRE((K + ksplit - 1) / ksplit == kper && (long)(ksplit - 1) * kper < K, "group_bulk: bad plan K=%d ksplit=%d kper=%d",
+                   K, ksplit, kper);
     const size_t idx_bytes = ((size_t)32 * (kper | 1) * 4 + 127) & ~(size_t)127;
     const int grid = (int)((units + nwarps - 1) / nwarps < sms ? (units + nwarps - 1) / nwarps : sms);
     const size_t smem = (size_t)nwarps * (idx_bytes + nst * tile);

@@ -80,6 +80,26 @@ for D in (0, 16, 20, 64, 128, 200):
     env()
 gi = P.knn_point(16, big[:1], big[:1, :4096].contiguous())
 env(BULK=1); P.group_points(big[:1], big[:1, :4096].contiguous(), torch.randn(1, 16384, 64, device=dev), gi, xyz_first=True); env()
+# asynchronous grouping with K cut into parts of several slots that do not divide K (default plan, then forced), with
+# sentinel and negative indices; feature gradients with D > 256 (the backward kernel loops over channel blocks)
+for B, S, K, D, bulk in ((16, 4096, 10, 16, None), (16, 4096, 12, 32, None), (16, 4096, 20, 64, None), (8, 4096, 20, 16, None),
+                         (8, 4096, 24, 32, None), (1, 16384, 48, 16, None), (1, 865, 256, 384, 1), (1, 4000, 256, 16, 1),
+                         (2, 777, 12, 392, 1), (2, 777, 12, 132, 1)):
+    env(**({} if bulk is None else dict(BULK=bulk)))
+    gi = torch.randint(-2048, 2049, (B, S, K), device=dev)                  # 2048 = the empty-ball sentinel
+    fe = torch.randn(B, 2048, D, device=dev)
+    for xf in (True, False):
+        P.group_points(big[:1, :2048].expand(B, -1, -1).contiguous(), big[:1, :S].expand(B, -1, -1).contiguous(), fe, gi, xyz_first=xf)
+env()
+for D in (257, 300, 520):
+    gi = torch.randint(-1000, 1001, (2, 777, 16), device=dev)
+    fe = torch.randn(2, 1000, D, device=dev, requires_grad=True)
+    for xf in (True, False):
+        P.group_points(ref[:, :1000].contiguous(), ref[:, :777].contiguous(), fe, gi, xyz_first=xf).sum().backward()
+# interpolation gradients with negative and dropped neighbours
+sf = torch.randn(2, 64, 12, device=dev, requires_grad=True)
+i3 = torch.randint(-70, 70, (2, 5000, 3), device=dev)
+P.three_interpolate(sf, i3, torch.rand(2, 5000, 3, device=dev, requires_grad=True)).sum().backward()
 P.square_distance(ref[:, :100], qry[:, :33])
 x = ref[:, :500].clone().requires_grad_(True); S3.chamfer_distance(x, qry)[0].backward()
 ff = torch.randn(2, 3000, 13, device=dev)
