@@ -372,7 +372,11 @@ extern "C" int b200pc_fps(const float *xyz, int B, int N, int npoint, const int6
     // C=8 0.62 / 0.68, C=16 0.63 / 0.94; one CTA 0.29 / 0.50.  The flat exchange wins exactly where the cluster is 4 CTAs
     // (batches of >= 10 clouds, e.g. C3: 3.05 -> 2.70 ms); everywhere else the two-level kernel stays.
     const int flat = tuning().fps_flat;
-    if (flat > 0 || (flat < 0 && C == 4)) {
+    const bool use_flat = flat > 0 || (flat < 0 && C == 4);
+    if (tuning().debug_plan)
+        fprintf(stderr, "b200pc fps plan: B=%d N=%d npoint=%d -> cluster %d, %d points/thread, exchange %s\n", B, N, npoint, C, P,
+                use_flat ? "flat" : "two-level");
+    if (use_flat) {
         switch (P) {
             case 1: return launch_fps_flat<1>(xyz, B, N, npoint, start, idx, C, st);
             case 2: return launch_fps_flat<2>(xyz, B, N, npoint, start, idx, C, st);

@@ -1300,7 +1300,13 @@ bool plan_search(int B, int N, int S, int k, int mode, SearchPlan *pl) {
     pl->n_tiles = pl->n_pad / TILE;
 
     const Tuning &tn = tuning();                      // tuning / debugging overrides (cached; not part of the ABI)
-    const int force_q = tn.force_q, force_w = tn.force_warps, force_split = tn.force_split;
+    const int force_q = tn.force_q, force_w = tn.force_warps > 0 ? tn.force_warps : 0;
+    // A forced split is evaluated as the only candidate (not filtered out of the 1, 2, 3, 4, 8, ... sequence below, which
+    // would leave no candidate for 5 or for a tile count outside it), clamped to the tile count and to the 32 lists one
+    // merge warp holds.
+    int force_split = tn.force_split > 0 ? tn.force_split : 0;
+    if (force_split > pl->n_tiles) force_split = pl->n_tiles;
+    if (force_split > MAX_SPLIT) force_split = MAX_SPLIT;
 
     double best_score = -1.0;
     int best_q = 1, best_w = 1, best_split = 1;
@@ -1310,21 +1316,35 @@ bool plan_search(int B, int N, int S, int k, int mode, SearchPlan *pl) {
         // after the other with half the resident warps: measured 20-40 % slower on every shape, so Q=2 is kept for
         // A/B measurements (B200PC_FORCE_Q=2) only.
         if (force_q ? q != force_q : q != 1) continue;
+        // A forced warp count is clamped once, to what one resident CTA can hold, and then only candidates that can run
+        // exactly that many warps compete: a smaller count at more CTAs per SM must not replace it unannounced.  One CTA
+        // per SM always passes the register check below.
+        int wforce = force_w;
+        if (wforce) {
+            const int cap = q == 1 ? MAX_WARPS_Q1 : MAX_WARPS;
+            const size_t budget1 = kMaxSmem - 1024;
+            const int fit1 = budget1 > kFixedSmem ? (int)((budget1 - kFixedSmem) / (32 * q * qb)) : 0;
+            if (wforce > cap) wforce = cap;
+            if (wforce > fit1) wforce = fit1 > 1 ? fit1 : 1;
+        }
         for (int c = 1; c <= 8; ++c) {                       // target CTAs per SM
             const size_t budget = kMaxSmem / c - 1024;          // ~1 KB per resident CTA is reserved by the system
             if (budget <= kFixedSmem + 32 * q * qb) continue;
             int wmax = (int)((budget - kFixedSmem) / (32 * q * qb));
             if (wmax > (q == 1 ? MAX_WARPS_Q1 : MAX_WARPS)) wmax = q == 1 ? MAX_WARPS_Q1 : MAX_WARPS;
             const long slots = (long)sms * c;
-            for (int split = 1; split <= MAX_SPLIT && split <= pl->n_tiles; split = split < 4 ? split + 1 : split * 2) {
-                if (force_split && split != (force_split > pl->n_tiles ? pl->n_tiles : force_split)) continue;
+            for (int split = force_split ? force_split : 1; split <= MAX_SPLIT && split <= pl->n_tiles;
+                 split = force_split ? MAX_SPLIT + 1 : split < 4 ? split + 1 : split * 2) {
                 // queries per CTA if the work items (query block x ref split) of each batch item fill the slots
                 long ipb = slots / ((long)B * split);           // query blocks per batch item, one wave
                 if (ipb < 1) ipb = 1;
                 int w = (int)((((long)S + ipb - 1) / ipb + 32 * q - 1) / (32 * q));
                 if (w < 1) w = 1;
                 if (w > wmax) w = wmax;
-                if (force_w) w = force_w > wmax ? wmax : force_w;
+                if (wforce) {
+                    if (wforce > wmax) continue;
+                    w = wforce;
+                }
                 // register file: 64K registers per SM, <= 128 (Q=2) / <= 72 (Q=1) per thread
                 if ((long)w * 32 * c * (q == 2 ? 128 : 72) > 65536) continue;
                 const long items = (long)B * (((long)S + 32L * q * w - 1) / (32L * q * w));
@@ -1350,6 +1370,9 @@ bool plan_search(int B, int N, int S, int k, int mode, SearchPlan *pl) {
             }
         }
     }
+    // No candidate: the one-warp plan below, which the check at the top allows -- unless Q = 2 was forced (or a Q that does
+    // not exist), which must not quietly run as Q = 1.
+    if (best_score < 0.0 && force_q > 1) return false;
     pl->q_per_thread = best_q;
     pl->consumer_warps = best_w;
     pl->q_per_block = best_q * best_w * 32;
@@ -1401,7 +1424,8 @@ static int run_search(const float *ref, const float *qry, int B, int N, int S, i
     }
     SearchPlan pl;
     if (!plan_search(B, N, S, k, mode, &pl)) {
-        set_error("search: list length k=%d does not fit in shared memory", k);
+        set_error("search: list length k=%d does not fit in shared memory%s", k,
+                  tuning().force_q > 1 ? " at the forced queries per thread (B200PC_FORCE_Q)" : "");
         return B200PC_EINVAL;
     }
     if (!ws || ws_bytes < pl.total_bytes) {
@@ -1409,10 +1433,6 @@ static int run_search(const float *ref, const float *qry, int B, int N, int S, i
         return B200PC_EWORKSPACE;
     }
     B200PC_REQUIRE((reinterpret_cast<uintptr_t>(ws) & 15) == 0, "search: workspace must be 16-byte aligned");
-    if (tuning().debug_plan)
-        fprintf(stderr, "b200pc plan: B=%d N=%d S=%d k=%d mode=%d -> %d warps/CTA, %d queries/CTA, ref split %d (%d tiles each), grid %s, %zu B smem\n", B, N, S,
-                k, mode, pl.consumer_warps, pl.q_per_block, pl.n_split, pl.tiles_per_split,
-                pl.grid_bytes ? (pl.grid_sorted ? "sorted" : "thresholds") : "off", pl.smem_bytes);
 
     char *w = static_cast<char *>(ws);
     float4 *packed = reinterpret_cast<float4 *>(w);
@@ -1476,6 +1496,11 @@ static int run_search(const float *ref, const float *qry, int B, int N, int S, i
         if (mode == MODE_TOPK) { a.part_d = reinterpret_cast<float *>(p); p += align_up(rows * k * 4, 256); }
         a.part_cnt = reinterpret_cast<int *>(p);
     }
+    if (tn.debug_plan)   // order: the ref order inside the tiles (strided: slot_to_ref; cell: sorted_slot)
+        fprintf(stderr, "b200pc plan: B=%d N=%d S=%d k=%d mode=%d -> %d warps/CTA, %d queries/CTA, ref split %d (%d tiles each), grid %s, "
+                "filter %s, order %s, %zu B smem\n", B, N, S, k, mode, pl.consumer_warps, pl.q_per_block, pl.n_split, pl.tiles_per_split,
+                pl.grid_bytes ? (pl.grid_sorted ? "sorted" : "thresholds") : "off", a.lane_filter ? "lane" : "broadcast",
+                pl.grid_sorted ? "cell" : strided_eff ? "strided" : "natural", pl.smem_bytes);
     int rc;
     if (mode == MODE_BALL) rc = launch_shape<B200PC_FORM_QRY_NORM_FIRST, MODE_BALL>(a, pl, B, st);
     else if (form == B200PC_FORM_REF_NORM_FIRST) rc = launch_shape<B200PC_FORM_REF_NORM_FIRST, MODE_TOPK>(a, pl, B, st);

@@ -11,6 +11,7 @@ import torch
 
 from b200pc import ops, synth
 from oracle import strict
+from test_gpu_plans import Knobs     # reads back the plan that ran (B200PC_DEBUG_PLAN)
 
 pytestmark = pytest.mark.gpu
 
@@ -78,10 +79,14 @@ def test_grid_variants_ties_and_duplicates(cuda_dev, monkeypatch, env):
 
 
 @pytest.mark.parametrize("env", VARIANTS, ids=IDS)
-def test_grid_variants_split_and_far_queries(cuda_dev, monkeypatch, env):
+def test_grid_variants_split_and_far_queries(cuda_dev, monkeypatch, capfd, env):
     _force(monkeypatch, env)
+    knobs = Knobs(monkeypatch, capfd)
+    knobs.set()
     a, b = synth.batch_pairs(3, 1, 16384)
-    _check(cuda_dev, a, b[:, :1024].copy(), 16, 2)      # few queries: the ref range is split over gridDim.z and merged
+    _, plans, _ = knobs.run(lambda: _check(cuda_dev, a, b[:, :1024].copy(), 16, 2))   # few queries: the ref range is split and merged
+    assert len(plans) == 1 and int(plans[0]["split"]) > 1, plans
+    assert plans[0]["grid"] == ("thresholds" if env["B200PC_GRID"] == "2" else "sorted"), plans
     _check(cuda_dev, a[:, :6000].copy(), (b[:, :300] + 500.0).astype(np.float32), 8, 0)     # queries outside the ref box
     sparse = a[:, :4000].copy()
     sparse[:, ::7] *= 40.0                              # a few refs far away: most cells empty, wide boxes

@@ -7,6 +7,7 @@ import torch
 
 from b200pc import ops, pointnet2_utils as P, pytorch3d_shim as S3, synth
 from oracle import strict
+from test_gpu_plans import Knobs, expect     # sets knobs and reads back the plan that ran (B200PC_DEBUG_PLAN)
 
 pytestmark = pytest.mark.gpu
 
@@ -66,12 +67,15 @@ def test_knn_tie_stress_lowest_index_wins(cuda_dev, form):
     np.testing.assert_array_equal(_bits(dist.cpu().numpy()), _bits(od))
 
 
-def test_knn_split_path_small_query_count(cuda_dev):
+def test_knn_split_path_small_query_count(cuda_dev, monkeypatch, capfd):
     # few queries against many refs -> the ref range is split over gridDim.z and merged
+    knobs = Knobs(monkeypatch, capfd)
+    knobs.set()
     a, b = synth.batch_pairs(3, 1, 16384)
     ref, qry = a, b[:, :1024].copy()
     for k, form in ((8, 0), (16, 2), (3, 1)):
-        idx, dist = ops.knn_search(_t(ref, cuda_dev), _t(qry, cuda_dev), k, form, want_dist=True)
+        (idx, dist), plans, _ = knobs.run(lambda: ops.knn_search(_t(ref, cuda_dev), _t(qry, cuda_dev), k, form, want_dist=True))
+        assert len(plans) == 1 and int(plans[0]["split"]) > 1, plans      # the planner still serves the split path here
         oi, od = strict.knn(ref, qry, k, form)
         np.testing.assert_array_equal(idx.cpu().numpy(), oi)
         np.testing.assert_array_equal(_bits(dist.cpu().numpy()), _bits(od))
@@ -217,14 +221,18 @@ def test_ball_query_exact_far_from_origin(cuda_dev):
 
 
 @pytest.mark.parametrize("form", [0, 1, 2])
-def test_broadcast_filter_fallback_matches(cuda_dev, monkeypatch, form):
+def test_broadcast_filter_fallback_matches(cuda_dev, monkeypatch, capfd, form):
     # B200PC_FILTER=0 keeps the queries in registers and broadcasts the refs (the warm-up filter, used for the whole
     # tile): same results by construction, kept under test because it is the A/B baseline of the lane filter
+    knobs = Knobs(monkeypatch, capfd)
+    knobs.set()
     a, b = synth.batch_pairs(23, 1, 5000)
     ref, qry = a[:, :5000].copy(), b[:, :1500].copy()
-    want = ops.knn_search(_t(ref, cuda_dev), _t(qry, cuda_dev), 16, form, want_dist=True)
-    monkeypatch.setenv("B200PC_FILTER", "0")
-    got = ops.knn_search(_t(ref, cuda_dev), _t(qry, cuda_dev), 16, form, want_dist=True)
+    want, plans, _ = knobs.run(lambda: ops.knn_search(_t(ref, cuda_dev), _t(qry, cuda_dev), 16, form, want_dist=True))
+    expect(plans, filter="lane")
+    knobs.set(FILTER=0)
+    got, plans, _ = knobs.run(lambda: ops.knn_search(_t(ref, cuda_dev), _t(qry, cuda_dev), 16, form, want_dist=True))
+    expect(plans, filter="broadcast")
     assert torch.equal(want[0], got[0]) and torch.equal(want[1], got[1])
     oi, od = strict.knn(ref, qry, 16, form)
     np.testing.assert_array_equal(got[0].cpu().numpy(), oi)
@@ -241,19 +249,23 @@ def test_randomised_shapes_scales_and_ties_fuzz(cuda_dev):
 
 
 @pytest.mark.parametrize("form", [0, 2])
-def test_knn_spatially_sorted_clouds_exact_and_not_pathological(cuda_dev, monkeypatch, form):
+def test_knn_spatially_sorted_clouds_exact_and_not_pathological(cuda_dev, monkeypatch, capfd, form):
     # a scan-ordered / spatially sorted cloud is the adversarial arrival order for a streaming k-best; the strided
     # tiles (search.cu slot_to_ref) make it behave like a shuffled one.  Results are identical either way.
+    knobs = Knobs(monkeypatch, capfd)
+    knobs.set()
     a, b = synth.batch_pairs(31, 2, 16384)
     order = lambda x: np.stack([c[np.lexsort((c[:, 2], c[:, 1], np.round(c[:, 0])))] for c in x])     # sorted along x, then y
     ref, qry = order(a), order(b)[:, ::8].copy()
     r, q = _t(ref, cuda_dev), _t(qry, cuda_dev)
-    idx, dist = ops.knn_search(r, q, 16, form, want_dist=True)
+    (idx, dist), plans, _ = knobs.run(lambda: ops.knn_search(r, q, 16, form, want_dist=True))
+    expect(plans, order="strided")
     oi, od = strict.knn(ref, qry, 16, form)
     np.testing.assert_array_equal(_bits(dist.cpu().numpy()), _bits(od))
     np.testing.assert_array_equal(idx.cpu().numpy(), oi)
-    monkeypatch.setenv("B200PC_NATURAL_ORDER", "1")                       # refs visited in index order: same answer
-    idx2, dist2 = ops.knn_search(r, q, 16, form, want_dist=True)
+    knobs.set(NATURAL_ORDER=1)                                            # refs visited in index order: same answer
+    (idx2, dist2), plans, _ = knobs.run(lambda: ops.knn_search(r, q, 16, form, want_dist=True))
+    expect(plans, order="natural")
     assert torch.equal(idx, idx2) and torch.equal(dist, dist2)
 
 

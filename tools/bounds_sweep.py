@@ -13,7 +13,8 @@ ops.TUNING_AUTORELOAD = True
 
 dev = torch.device("cuda:0")
 print("library:", os.path.basename(_lib.LIB_PATH), flush=True)
-ENV = ("B200PC_GRID", "B200PC_SEED", "B200PC_INTERLEAVE", "B200PC_SMALL_PATH", "B200PC_FORCE_SPLIT", "B200PC_BULK", "B200PC_FPS_FLAT", "B200PC_FPS_CLUSTER")
+ENV = ("B200PC_GRID", "B200PC_SEED", "B200PC_INTERLEAVE", "B200PC_SMALL_PATH", "B200PC_FORCE_SPLIT", "B200PC_BULK", "B200PC_FPS_FLAT", "B200PC_FPS_CLUSTER",
+       "B200PC_FORCE_WARPS", "B200PC_FORCE_Q", "B200PC_FILTER", "B200PC_NATURAL_ORDER")
 
 
 def env(**kw):
@@ -47,12 +48,41 @@ for kw in (dict(), dict(GRID=3, SMALL_PATH=0), dict(GRID=2, SMALL_PATH=0)):
 env()
 same = np.repeat(np.array([[[1.5, -2.0, 0.25]]], np.float32), 900, axis=1)
 env(GRID=3, SMALL_PATH=0); ops.knn_search(t(same), t(b[:1, :100]), 7, 0); env()
+# forced plans (tests/test_gpu_plans.py): every split a range count can come from, short and ragged ranges, k above the refs
+# of a range, warps per CTA with empty trailing warps, two queries per thread, the broadcast filter and the natural order
+for (B, N, S, k), splits in (((1, 513, 77, 300), (2,)), ((2, 2048, 333, 600), (3, 4)), ((1, 5000, 700, 16), (3, 4, 5, 7, 8)),
+                             ((1, 20000, 300, 64), (32, 40))):
+    a, b = synth.batch_pairs(12, B, max(N, S))
+    ref, qry = t(a[:, :N]), t(b[:, :S])
+    for split in splits:
+        for grid in (0, 2, 3):
+            env(SMALL_PATH=0, GRID=grid, FORCE_SPLIT=split)
+            for form in (0, 1, 2):
+                ops.knn_search(ref, qry, k, form, want_dist=True)
+            ops.knn_search_i32(ref, qry, k, 2)
+        env(FORCE_SPLIT=split)
+        P.query_ball_point(0.7, min(128, N), ref, qry); P.query_ball_point(100.0, 32, ref, qry)
+a, b = synth.batch_pairs(13, 1, 4100)
+for S in (33, 777, 4100):
+    ref, qry = t(a[:, :3000]), t(b[:, :S])
+    for q in (1, 2):
+        for w in (1, 2, 5, 14):
+            for kw in (dict(), dict(GRID=3, INTERLEAVE=1)):
+                env(SMALL_PATH=0, FORCE_Q=q, FORCE_WARPS=w, **kw)
+                ops.knn_search(ref, qry, 16, 0, want_dist=True); ops.knn_search_i32(ref, qry, 16, 2)
+            env(FORCE_Q=q, FORCE_WARPS=w); P.query_ball_point(1.0, 32, ref, qry)
+for kw in (dict(FILTER=0), dict(FILTER=0, FORCE_SPLIT=4), dict(NATURAL_ORDER=1), dict(NATURAL_ORDER=0, FORCE_SPLIT=4), dict(FORCE_Q=2, FORCE_SPLIT=4)):
+    env(SMALL_PATH=0, GRID=0, **kw)
+    for form in (0, 1, 2):
+        ops.knn_search(ref, qry, 16, form, want_dist=True)
+env()
 torch.cuda.synchronize(); print("searches ok", flush=True)
 
 # ---- FPS (single CTA, clusters, flat exchange), gather, group, interpolate, fusion, chamfer, polyfit, rebuild
 a, b = synth.batch_pairs(2, 2, 16384)
 big = t(a)
-for kw in (dict(), dict(FPS_FLAT=1), dict(FPS_FLAT=0), dict(FPS_CLUSTER=2), dict(FPS_CLUSTER=16)):
+for kw in (dict(), dict(FPS_FLAT=1), dict(FPS_FLAT=0), dict(FPS_CLUSTER=2), dict(FPS_CLUSTER=16), dict(FPS_CLUSTER=16, FPS_FLAT=1),
+           dict(FPS_CLUSTER=1, FPS_FLAT=1), dict(FPS_CLUSTER=8, FPS_FLAT=0)):
     env(**kw)
     for n, m in ((16384, 300), (12000, 64), (3000, 128), (40, 7)):
         ops.fps(big[:, :n].contiguous(), m, torch.tensor([1, n - 1], device=dev))
