@@ -20,6 +20,21 @@
  *    available from b200pc_last_error() (thread-local).  Nothing throws across this ABI.
  *  - there is NO CPU fallback: without a CUDA device every compute entry returns
  *    B200PC_ECUDA.
+ *
+ * Non-finite coordinates (NaN, +-inf: e.g. invalid LiDAR returns)
+ *  - Top-k (knn, knn_i32, three_nn, feature_propagation, fusion_group, chamfer, rebuild_pack): a (query, ref) pair is a
+ *    candidate only if its distance, in the call site's rounding, is finite.  Each row holds its candidates in ascending
+ *    (distance, index) order, then index -1 with distance +inf in the remaining slots -- on every kernel path and for both
+ *    index widths.  This departs from the reference's torch.topk, which ranks NaN distances last but still returns them.
+ *  - Domain: for finite coordinates with |c| < 2^62 every distance in every form is finite (|r|^2, |q|^2 <= 3*2^124,
+ *    |2q.r| <= 6*2^124, the expanded sum and |q-r|^2 <= 12*2^124 ~ 2.6e38 < FLT_MAX), so every finite pair is a candidate;
+ *    a pair with a NaN or +-inf coordinate always has a non-finite distance.  Finite coordinates beyond 2^62 are outside
+ *    the contract: indices stay in [-1, N) and nothing faults, but the results are not specified.
+ *  - Ball query: a NaN distance is never a hit (see b200pc_ball_query).
+ *  - Chamfer: a point without a candidate gets index -1 and minimum +inf, makes the loss +inf, and neither receives nor
+ *    gives gradient.
+ *  - FPS: a NaN or +inf distance never lowers a running minimum (the reference's `dist < distance` mask).
+ *  - Consumers of indices (gather, group_points, three_interpolate) wrap -1 once to the last row, as Python indexing does.
  */
 #ifndef B200PC_H
 #define B200PC_H
@@ -70,7 +85,8 @@ int b200pc_square_distance(const float *src, const float *dst, int B, int N, int
 /* form 0  -> Group.forward kNN branch, Utils/Layers.py:50-53 (exposed as knn_point)
  * form 2  -> pytorch3d.ops.knn_points(p1=qry, p2=ref, K=k) as called at Utils/Layers.py:220,
  *            311,393,430; PolyPCI/Models/Models_V1.py:113; PointINet20230424/models/layers.py:360
- * idx [B,S,k] int64 ascending by (distance, index); dist [B,S,k] may be NULL.
+ * idx [B,S,k] int64 ascending by (distance, index), -1 / +inf where fewer than k refs have a finite distance (see
+ * "Non-finite coordinates" above); dist [B,S,k] may be NULL.
  * k <= N (EINVAL otherwise, like torch.topk); the k-best lists live in shared memory: k up to ~780.  Empty work
  * (B == 0 or S == 0) returns OK without looking at the pointers.                                       */
 int b200pc_knn(const float *ref, const float *qry, int B, int N, int S, int k, int form, int64_t *idx,
@@ -199,7 +215,8 @@ int b200pc_poly_predict(const float *const *frames, const double *weights, int B
 /* ---- a9: chamfer_loss  Utils/Utils.py:39-48 -> pytorch3d.loss.chamfer_distance defaults --- */
 /* x [B,N,3], y [B,M,3].  Outputs: per-point nearest squared distance and index in both
  * directions (dx,ix: [B,N]; dy,iy: [B,M]) and the scalar loss[1] =
- * mean_b( mean_i dx + mean_j dy ).  loss is written (not accumulated).                       */
+ * mean_b( mean_i dx + mean_j dy ).  loss is written (not accumulated).  A point without a finite distance to the
+ * other cloud gets index -1 and minimum +inf (the loss is then +inf); chamfer_bwd gives it no gradient.        */
 int b200pc_chamfer_fwd(const float *x, const float *y, int B, int N, int M, float *dx, int64_t *ix, float *dy,
                        int64_t *iy, float *loss, void *workspace, size_t workspace_bytes,
                        b200pc_stream_t stream);

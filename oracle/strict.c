@@ -121,7 +121,8 @@ static inline float sqdist_direct(const float *a, const float *b)
 }
 
 /* ------------------------------------------------------------------------------------ */
-/* selection helper: the k smallest of row[0..n) under the total order (value, index).   */
+/* selection helper: the k smallest FINITE entries of row[0..n) under the total order     */
+/* (value, index), then -1 / +inf.                                                       */
 /* Done by value-threshold first (quickselect on a scratch copy), then an index-ordered  */
 /* sweep, then a tiny sort -- deliberately NOT the streaming insert the CUDA kernels use */
 /* ------------------------------------------------------------------------------------ */
@@ -145,24 +146,31 @@ static float kth_smallest(float *v, int n, int k) /* k is 0-based; v is clobbere
 
 static void select_k(const float *row, int n, int k, float *scratch, int64_t *idx_out, float *val_out)
 {
-    memcpy(scratch, row, (size_t)n * sizeof(float));
-    float tau = kth_smallest(scratch, n, k - 1);
+    /* only finite distances are candidates (include/b200pc.h, "Non-finite coordinates"): a NaN has no place in the order,
+     * and a +inf distance would tie with the padding below */
+    int nf = 0;
+    for (int i = 0; i < n; i++)
+        if (isfinite(row[i])) scratch[nf++] = row[i];
+    int kk = k < nf ? k : nf;
     int cnt = 0;
-    /* strictly below the threshold: all of them belong */
-    for (int i = 0; i < n && cnt < k; i++)   /* the bound only matters for NaN rows (no order): stay inside the buffers */
-        if (row[i] < tau) { idx_out[cnt] = i; val_out[cnt] = row[i]; cnt++; }
-    /* equal to the threshold: lowest indices first until k are collected */
-    for (int i = 0; i < n && cnt < k; i++)
-        if (row[i] == tau) { idx_out[cnt] = i; val_out[cnt] = row[i]; cnt++; }
-    for (; cnt < k; cnt++) { idx_out[cnt] = -1; val_out[cnt] = INFINITY; }   /* NaN rows only */
-    /* order the k survivors by (value, index) */
-    for (int a = 1; a < k; a++) {
+    if (kk > 0) {
+        float tau = kth_smallest(scratch, nf, kk - 1);
+        /* strictly below the threshold: all of them belong (a non-finite entry compares false) */
+        for (int i = 0; i < n && cnt < kk; i++)
+            if (row[i] < tau) { idx_out[cnt] = i; val_out[cnt] = row[i]; cnt++; }
+        /* equal to the threshold: lowest indices first until kk are collected */
+        for (int i = 0; i < n && cnt < kk; i++)
+            if (row[i] == tau) { idx_out[cnt] = i; val_out[cnt] = row[i]; cnt++; }
+    }
+    /* order the survivors by (value, index) */
+    for (int a = 1; a < cnt; a++) {
         float v = val_out[a]; int64_t id = idx_out[a]; int b = a - 1;
         while (b >= 0 && (val_out[b] > v || (val_out[b] == v && idx_out[b] > id))) {
             val_out[b + 1] = val_out[b]; idx_out[b + 1] = idx_out[b]; b--;
         }
         val_out[b + 1] = v; idx_out[b + 1] = id;
     }
+    for (; cnt < k; cnt++) { idx_out[cnt] = -1; val_out[cnt] = INFINITY; }   /* fewer than k candidates */
 }
 
 /* ------------------------------------------------------------------------------------ */
@@ -231,8 +239,10 @@ void orc_knn(const float *ref, const float *qry, int B, int N, int S, int k, int
 
 /* ------------------------------------------------------------------------------------ */
 /* a2: query_ball_point  Utils/Pointnet2Utils.py:88-108                                  */
-/* first `nsample` ref indices (ascending) with NOT(d > r2); pad with the first hit; a   */
+/* first `nsample` ref indices (ascending) with d <= r2; pad with the first hit; a       */
 /* query with no hit yields N in every slot.  d = square_distance(new_xyz, xyz).         */
+/* d <= r2 is the reference's NOT(d > r2) for every distance but NaN: a NaN distance     */
+/* (non-finite coordinates) is never a hit here, as in the kernels.                      */
 /* r2 is the fp32 rounding of the double radius**2 (computed by the caller).             */
 /* ------------------------------------------------------------------------------------ */
 typedef struct { float r2; int nsample; const float *xyz, *q; const float *rnorm; int B, N, S; int64_t *out; } ball_ctx;
@@ -248,7 +258,7 @@ static void ball_body(int64_t lo, int64_t hi, void *vc)
         for (int n = 0; n < c->N && cnt < c->nsample; n++) {
             const float *r = c->xyz + ((size_t)b * c->N + n) * 3;
             float d = sqdist_expanded(q, nq, r, c->rnorm[(size_t)b * c->N + n]);
-            if (!(d > c->r2)) o[cnt++] = n;
+            if (d <= c->r2) o[cnt++] = n;
         }
         int64_t first = cnt > 0 ? o[0] : (int64_t)c->N;
         for (int j = cnt; j < c->nsample; j++) o[j] = first;
@@ -352,14 +362,19 @@ static void interp_body(int64_t lo, int64_t hi, void *vc)
         int b = (int)(row / c->N);
         const int64_t *id = c->idx + (size_t)row * 3;
         const float *ww = c->w + (size_t)row * 3;
-        const float *f0 = c->feat + ((size_t)b * c->S + id[0]) * C;
-        const float *f1 = c->feat + ((size_t)b * c->S + id[1]) * C;
-        const float *f2 = c->feat + ((size_t)b * c->S + id[2]) * C;
+        int64_t i[3]; float wv[3];
+        for (int j = 0; j < 3; j++) {      /* the kernels' index rule: wrap once; still out of range -> row 0, weight 0 */
+            i[j] = id[j] < 0 ? id[j] + c->S : id[j]; wv[j] = ww[j];
+            if (i[j] < 0 || i[j] >= c->S) { i[j] = 0; wv[j] = 0.0f; }
+        }
+        const float *f0 = c->feat + ((size_t)b * c->S + i[0]) * C;
+        const float *f1 = c->feat + ((size_t)b * c->S + i[1]) * C;
+        const float *f2 = c->feat + ((size_t)b * c->S + i[2]) * C;
         float *o = c->out + (size_t)row * C;
         for (int ch = 0; ch < C; ch++) {
-            float a = f0[ch] * ww[0];
-            float bb = f1[ch] * ww[1];
-            float cc = f2[ch] * ww[2];
+            float a = f0[ch] * wv[0];
+            float bb = f1[ch] * wv[1];
+            float cc = f2[ch] * wv[2];
             float ab = a + bb;
             o[ch] = ab + cc;
         }
@@ -375,7 +390,8 @@ void orc_three_interpolate(const float *feat, const int64_t *idx, const float *w
 /* ------------------------------------------------------------------------------------ */
 /* a9: chamfer_loss -> pytorch3d.loss.chamfer_distance defaults (PARITY UNPINNED)        */
 /* Utils/Utils.py:39-48.  mean_b[ mean_i min_j d(x_i,y_j) + mean_j min_i d(x_i,y_j) ].   */
-/* One direction = for every a_i the nearest b_j (direct form, first minimum wins).      */
+/* One direction = for every a_i the nearest b_j (direct form, first minimum wins); a    */
+/* point without a finite distance gets -1 / +inf, which makes the loss +inf.            */
 /* The scalar is accumulated in double: its contract is 1e-5 relative, not bitwise.      */
 /* ------------------------------------------------------------------------------------ */
 typedef struct { const float *a, *b; int B, N, M; float *mn; int64_t *arg; } nn1_ctx;
@@ -386,7 +402,7 @@ static void nn1_body(int64_t lo, int64_t hi, void *vc)
         int b = (int)(row / c->N);
         const float *p = c->a + (size_t)row * 3;
         const float *o = c->b + (size_t)b * c->M * 3;
-        float best = INFINITY; int64_t bi = 0;
+        float best = INFINITY; int64_t bi = -1;     /* d < best: only a finite d is taken */
         for (int j = 0; j < c->M; j++) {
             float d = sqdist_direct(p, o + (size_t)j * 3);
             if (d < best) { best = d; bi = j; }

@@ -39,7 +39,7 @@ __global__ void __launch_bounds__(256) chamfer_bwd_kernel(const float *__restric
     if (r >= rows) return;
     const long b = r / Na;
     const long j = nn[r];
-    if (j < 0 || j >= Nb) return;          // a point with NaN coordinates has no nearest neighbour (-1): no gradient
+    if (j < 0 || j >= Nb) return;          // a point without a finite distance (non-finite coordinates) has index -1: no gradient
     const float s = 2.0f * scale * gloss[0];
     const float *pa = a + r * 3;
     const float *pb = bpts + (b * Nb + j) * 3;

@@ -30,7 +30,7 @@ __global__ void __launch_bounds__(256) fusion_features_kernel(const float *__res
     const long b = bs / S;
     const long plane = (long)S * K, o = e - b * plane;               // offset inside one [S,K] plane
     const long i = idx[e];
-    const bool ok = i >= 0 && i < N;                                 // -1: a NaN query ranks nothing -> NaN features, like gathering nothing
+    const bool ok = i >= 0 && i < N;                                 // -1: no candidate in this slot -> NaN features, like gathering nothing
     const float *q = qry + bs * 3;
     const float *r = ref + (b * N + (ok ? i : 0)) * 3;
     const float qn = __int_as_float(0x7fc00000);

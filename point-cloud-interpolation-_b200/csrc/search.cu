@@ -1044,7 +1044,11 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
                                 B200PC_DEV_ASSERT(off >= 0 && off < TILE && tile_ref0 + off < P.n_pad);
                                 cur &= cur - 1;
                                 const float d = ref_dist<FORM>(tp, off, ex, ey, ez, nq);
-                                if (d <= tau[j]) {
+                                // only a finite distance is a candidate: while the heap still holds its (+inf, 0xffffffff)
+                                // sentinels tau is +inf, and a +inf distance that the filter let through (a query such
+                                // as (+inf, 0, 0), whose filter value is -inf for refs with x > 0) would enter with a
+                                // real index.  NaN fails d <= tau, and no form yields -inf.
+                                if (d <= tau[j] && d < CUDART_INF_F) {
                                     // the refs are not visited in index order: an EQUAL distance still wins with a lower index
                                     // than the root's (rare; only then is the root read)
                                     const uint32_t ri = P.perm ? (uint32_t)__ldg(P.perm + (size_t)b * P.n_pad + tile_ref0 + off)
@@ -1161,7 +1165,7 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
                 float *dout = P.dist_out ? P.dist_out + row * k : nullptr;
                 for (int e = 0; e < k; ++e) {
                     const unsigned long long key = heap_all[e * QPB + slot];
-                    if (io) io[e] = (int64_t)(int32_t)(uint32_t)key;     // unfilled slot (a NaN query ranks nothing): -1, distance +inf
+                    if (io) io[e] = (int64_t)(int32_t)(uint32_t)key;     // unfilled slot (fewer than k candidates): -1, distance +inf
                     if (io32) io32[e] = (int32_t)(uint32_t)key;
                     if (dout) dout[e] = key_to_float((uint32_t)(key >> 32));
                 }

@@ -87,7 +87,8 @@ __global__ void __launch_bounds__(SMALL_WARPS * 32) small_search_kernel(const fl
             for (int i = 0; i < NI; ++i) {
                 const int r = i * 32 + lane;
                 const float d = dist_scalar<FORM>(sx[r], sy[r], sz[r], sn[r], qx, qy, qz, qn);
-                key[i] = r < N ? (((unsigned long long)okey(d) << 32) | (unsigned)r) : ~0ull;
+                // only a finite distance is a candidate (NaN and +inf get the empty key; no form yields -inf)
+                key[i] = r < N && d < CUDART_INF_F ? (((unsigned long long)okey(d) << 32) | (unsigned)r) : ~0ull;
             }
             unsigned long long best = ~0ull;
 #pragma unroll
@@ -96,9 +97,10 @@ __global__ void __launch_bounds__(SMALL_WARPS * 32) small_search_kernel(const fl
                 const unsigned hi = (unsigned)(best >> 32);
                 const unsigned whi = __reduce_min_sync(0xffffffffu, hi);
                 const unsigned wlo = __reduce_min_sync(0xffffffffu, hi == whi ? (unsigned)best : 0xffffffffu);
-                if (lane == 0) {
-                    if (idx_out) idx_out[row * k + e] = (int64_t)wlo;
-                    if (dist_out) dist_out[row * k + e] = okey_inv(whi);
+                if (lane == 0) {      // the empty key: fewer than k candidates, -1 with distance +inf
+                    const bool empty = whi == 0xffffffffu;
+                    if (idx_out) idx_out[row * k + e] = empty ? -1 : (int64_t)wlo;
+                    if (dist_out) dist_out[row * k + e] = empty ? CUDART_INF_F : okey_inv(whi);
                 }
                 if (hi == whi && (unsigned)best == wlo) {     // the winning lane retires that ref and rescans
                     unsigned long long nb = ~0ull;

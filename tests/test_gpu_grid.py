@@ -101,11 +101,9 @@ def test_grid_variants_non_finite_points(cuda_dev, monkeypatch, env):
     ref[0, 5] = np.nan; ref[0, 77, 1] = np.inf; ref[1, 100:110] = -np.inf
     qry[0, 3] = np.nan; qry[1, 9, 2] = np.inf
     # non-finite refs never enter the grid and go behind the finite ones in the cell order; a non-finite query starts from
-    # +inf.  The blind search is the yardstick here (it is pinned to the oracle on finite inputs by test_gpu_search.py).
-    idx, dist = ops.knn_search(_t(ref, cuda_dev), _t(qry, cuda_dev), 16, 0, want_dist=True)
-    monkeypatch.setenv("B200PC_GRID", "0"); ops.reload_tuning()
-    idx0, dist0 = ops.knn_search(_t(ref, cuda_dev), _t(qry, cuda_dev), 16, 0, want_dist=True)
-    assert torch.equal(idx, idx0) and torch.equal(dist.view(torch.int32), dist0.view(torch.int32))
+    # +inf and ranks nothing (-1, +inf)
+    for form in (0, 1, 2):
+        _check(cuda_dev, ref, qry, 16, form)
 
 
 def test_int32_output_and_three_nn_through_the_sorted_grid(cuda_dev, monkeypatch):

@@ -454,3 +454,175 @@ def test_knn_points_and_chamfer_against_an_independent_kd_tree():
         ta, tb = cKDTree(a[bi].astype(np.float64)), cKDTree(b[bi].astype(np.float64))
         want += (tb.query(a[bi].astype(np.float64))[0] ** 2).mean() + (ta.query(b[bi].astype(np.float64))[0] ** 2).mean()
     assert abs(loss - want / 2) <= 1e-5 * abs(want / 2)
+
+
+# ---------------------------------------------------------------- non-finite coordinates (include/b200pc.h, "Non-finite")
+# The rule every search follows: a (query, ref) pair is a candidate only if its distance is finite.  A row holds its
+# candidates in ascending (distance, index) order, then -1 with distance +inf.  The restatements below compute the same
+# distances as the oracle's forms with numpy and apply that rule with a plain lexsort.
+def _dense_form(ref, qry, form):
+    """[B,S,N] distances in the oracle's rounding: forms 0 / 1 from square_distance, form 2 emulated (direct, FMA)"""
+    if form == 0:
+        return strict.square_distance(ref, qry).transpose(0, 2, 1)
+    if form == 1:
+        return strict.square_distance(qry, ref)
+    f32 = np.float32
+    with np.errstate(invalid="ignore", over="ignore"):
+        d = (qry[:, :, None, :] - ref[:, None, :, :]).astype(f32)          # q - r: squared, so the sign is irrelevant
+        acc = (d[..., 0] * d[..., 0]).astype(f32)
+        acc = _fma32(d[..., 1], d[..., 1], acc)
+        return _fma32(d[..., 2], d[..., 2], acc)
+
+
+def _topk_finite(dist, k):
+    """the k smallest finite entries of every row of dist [..., N] by (value, index), padded with (-1, +inf)"""
+    flat = dist.reshape(-1, dist.shape[-1])
+    idx = np.full((flat.shape[0], k), -1, np.int64)
+    val = np.full((flat.shape[0], k), np.inf, np.float32)
+    for r, row in enumerate(flat):
+        cand = np.flatnonzero(np.isfinite(row))
+        order = cand[np.lexsort((cand, row[cand]))][:k]
+        idx[r, :len(order)] = order
+        val[r, :len(order)] = row[order]
+    return idx.reshape(dist.shape[:-1] + (k,)), val.reshape(dist.shape[:-1] + (k,))
+
+
+def _non_finite_cloud(seed, B, N, S):
+    """refs and queries with NaN, +inf and -inf in one or all three coordinates, mixed-sign finite coordinates, a
+    (+inf, 0, 0) query, and -- for B > 1 -- a last batch item whose refs are all non-finite"""
+    rng = np.random.default_rng(seed)
+    ref = rng.normal(size=(B, N, 3)).astype(np.float32) * 4
+    qry = rng.normal(size=(B, S, 3)).astype(np.float32) * 4
+    bad = [np.nan, np.inf, -np.inf]
+    for b in range(B):
+        for j, n in enumerate(rng.choice(N, size=N // 5, replace=False)):
+            if j % 3 == 0:
+                ref[b, n] = bad[j % 9 // 3]
+            else:
+                ref[b, n, j % 3] = bad[j % 2]
+    qry[:, 0] = [np.inf, 0.0, 0.0]
+    qry[:, 1] = [np.nan, 1.0, 1.0]
+    qry[:, 2] = -np.inf
+    qry[:, 3] = [0.5, np.inf, -np.inf]
+    if B > 1:
+        ref[-1, :, rng.integers(0, 3)] = np.nan
+        ref[-1, ::2] = np.inf
+    return ref, qry
+
+
+def test_non_finite_knn_keeps_only_finite_candidates_in_the_issue_case():
+    # 40 refs: refs 3 and 20..25 are NaN and ref 10 has y = +inf, so 32 refs are finite; the queries are finite
+    rng = np.random.default_rng(1)
+    ref = rng.normal(size=(1, 40, 3)).astype(np.float32)
+    ref[0, [3, 20, 21, 22, 23, 24, 25]] = np.nan
+    ref[0, 10, 1] = np.inf
+    qry = rng.normal(size=(1, 6, 3)).astype(np.float32)
+    finite = np.setdiff1d(np.arange(40), [3, 10, 20, 21, 22, 23, 24, 25])
+    for form in (0, 1, 2):
+        full = _dense_form(ref, qry, form)
+        for k in (4, 32, 33, 40):
+            idx, dist = strict.knn(ref, qry, k, form)
+            want_i, want_d = _topk_finite(full, k)
+            np.testing.assert_array_equal(idx, want_i)
+            np.testing.assert_array_equal(bits(dist), bits(want_d))
+            n = min(k, 32)
+            assert np.isin(idx[..., :n], finite).all() and (idx[..., n:] == -1).all() and np.isinf(dist[..., n:]).all()
+            assert (np.diff(dist[..., :n], axis=-1) >= 0).all()
+
+
+@pytest.mark.parametrize("form", [0, 1, 2])
+@pytest.mark.parametrize("k", [1, 8, 30, 50])             # below, at and above the 40 finite refs of the first item
+def test_non_finite_knn_matches_restatement(form, k):
+    ref, qry = _non_finite_cloud(2, 3, 50, 12)
+    idx, dist = strict.knn(ref, qry, k, form)
+    want_i, want_d = _topk_finite(_dense_form(ref, qry, form), k)
+    np.testing.assert_array_equal(idx, want_i)
+    np.testing.assert_array_equal(bits(dist), bits(want_d))
+    assert (idx[-1] == -1).all()                           # the item without a finite ref ranks nothing
+    assert (idx[:, 0:4] == -1).all()                       # nor do the non-finite queries
+    assert (idx[:2, 4:, :min(k, 40)] >= 0).all()           # a finite query ranks every finite ref
+
+
+def test_non_finite_knn_ties_by_index():
+    # grid-snapped points: exact arithmetic and many equal distances, with NaN refs between them
+    ref = synth.grid_snapped(3, 1, 300, span=3).copy()
+    ref[0, 7::11] = np.nan
+    qry = synth.grid_snapped(4, 1, 40, span=3)
+    for form in (0, 1, 2):
+        full = _dense_form(ref, qry, form)
+        idx, dist = strict.knn(ref, qry, 16, form)
+        want_i, want_d = _topk_finite(full, 16)
+        assert (np.diff(want_d, axis=-1) == 0).any(-1).mean() > 0.5
+        np.testing.assert_array_equal(idx, want_i)
+        np.testing.assert_array_equal(bits(dist), bits(want_d))
+
+
+def test_non_finite_nearest_and_chamfer():
+    x, y = _non_finite_cloud(5, 2, 60, 30)
+    for a, b in ((x, y), (y, x)):
+        mn, arg = strict.nearest(a, b)
+        want_i, want_d = _topk_finite(_dense_form(b, a, 2), 1)
+        np.testing.assert_array_equal(arg, want_i[..., 0])
+        np.testing.assert_array_equal(bits(mn), bits(want_d[..., 0]))
+    loss, dx, ix, dy, iy = strict.chamfer(x, y)
+    assert loss == np.inf and (ix[1] == -1).all() and (dy[1] == np.inf).all()
+    # finite clouds: the loss stays finite and matches the float64 formula
+    xf, yf = x[:1, 4:].copy(), y[:1].copy()
+    xf[~np.isfinite(xf).all(-1)] = 0.25
+    yf[~np.isfinite(yf).all(-1)] = -0.5
+    loss = strict.chamfer(xf, yf)[0]
+    d64 = ((xf[:, :, None].astype(np.float64) - yf[:, None].astype(np.float64)) ** 2).sum(-1)
+    want = (d64.min(2).mean(1) + d64.min(1).mean(1)).mean()
+    assert abs(loss - want) <= 1e-5 * want
+
+
+def test_non_finite_ball_query_never_hits():
+    ref, qry = _non_finite_cloud(6, 2, 80, 20)
+    for radius, ns in ((1.0, 8), (3.0, 32), (1e3, 80)):
+        got = strict.query_ball_point(radius, ns, ref, qry)
+        d = _dense_form(ref, qry, 1)
+        hit = d <= strict.radius_sq(radius)                # NaN compares false: never a hit
+        want = np.full(got.shape, 80, np.int64)
+        for b, s in np.ndindex(2, 20):
+            h = np.flatnonzero(hit[b, s])[:ns]
+            if len(h):
+                want[b, s] = h[0]
+                want[b, s, :len(h)] = h
+        np.testing.assert_array_equal(got, want)
+        assert (got[1] == 80).all() and (got[:, :4] == 80).all()
+
+
+def test_three_interpolate_applies_the_kernels_index_rule():
+    # -1 (an unfilled three-NN slot) wraps once to the last row, like Python indexing; anything still out of range reads
+    # row 0 with weight 0 -- the kernels' clean_neighbour
+    rng = np.random.default_rng(7)
+    feat = rng.normal(size=(2, 5, 4)).astype(np.float32)
+    feat[1, 0, 2] = np.inf
+    idx = np.array([[[0, 1, -1], [-5, 4, 2], [6, -6, 3], [-1, -1, -1]]] * 2, np.int64)
+    w = rng.uniform(0.1, 1, size=(2, 4, 3)).astype(np.float32)
+    got = strict.three_interpolate(feat, idx, w)
+    want = np.empty_like(got)
+    for b, n in np.ndindex(2, 4):
+        terms = []
+        for j in range(3):
+            i, ww = idx[b, n, j], w[b, n, j]
+            i = i + 5 if i < 0 else i
+            if not 0 <= i < 5:
+                i, ww = 0, np.float32(0)
+            with np.errstate(invalid="ignore"):
+                terms.append((feat[b, i] * ww).astype(np.float32))
+        want[b, n] = ((terms[0] + terms[1]).astype(np.float32) + terms[2]).astype(np.float32)
+    np.testing.assert_array_equal(bits(got), bits(want))
+    assert np.isnan(got[1, 2, 2])                          # 0 * inf of a dropped neighbour, as on the device
+
+
+@pytest.mark.parametrize("start", [0, 3, 5, 9])
+def test_non_finite_fps_matches_the_reference_loop(start):
+    # NaN and +inf distances never lower a running minimum (the reference's `dist < distance` mask); 1e30 points square to
+    # +inf; a non-finite start leaves every minimum at 1e10
+    a, _ = synth.batch_pairs(8, 2, 300)
+    a = a.copy()
+    a[:, 3] = np.nan; a[:, 5, 1] = np.inf; a[:, 9, 0] = -np.inf; a[:, 40] = 1e30; a[:, 41, 2] = -1e30; a[1, 100:110, 2] = np.nan
+    st = np.array([start, start])
+    want = ref_torch.fps(torch.from_numpy(a), 64, torch.from_numpy(st)).numpy()
+    np.testing.assert_array_equal(strict.farthest_point_sample(a, 64, st), want)

@@ -45,6 +45,16 @@ bad_r, bad_q = a[:, :N].copy(), b[:, :S].copy()
 bad_r[0, 7] = np.nan; bad_r[0, 99, 2] = np.inf; bad_q[0, 3] = np.nan
 for kw in (dict(), dict(GRID=3, SMALL_PATH=0), dict(GRID=2, SMALL_PATH=0)):
     env(**kw); ops.knn_search(t(bad_r), t(bad_q), 16, 0, want_dist=True); P.query_ball_point(1.0, 16, t(bad_r), t(bad_q))
+# k above the finite count on the small path (rows end in -1), and a split range (tile 1 of the strided order, 2 tiles)
+# holding only non-finite refs; (+inf, 0, 0) is the query whose filter value is -inf for refs with x > 0
+few = bad_r[:1, :900].copy(); few[0, 8:] = np.nan
+half = bad_r[:1, :1000].copy(); half[0, 1::2] = np.inf
+bq = bad_q[:1, :64].copy(); bq[0, 5] = [np.inf, 0.0, 0.0]
+for kw, cloud in ((dict(SMALL_PATH=1), few), (dict(SMALL_PATH=0, GRID=0, FORCE_SPLIT=2), half), (dict(SMALL_PATH=0, GRID=3), half)):
+    env(**kw)
+    for form in (0, 1, 2):
+        ops.knn_search(t(cloud), t(bq), 16, form, want_dist=True); ops.knn_search_i32(t(cloud), t(bq), 16, form)
+    ops.chamfer(t(cloud), t(bq)); ops.fusion_group(t(bq), t(cloud), 16, t(cloud))
 env()
 same = np.repeat(np.array([[[1.5, -2.0, 0.25]]], np.float32), 900, axis=1)
 env(GRID=3, SMALL_PATH=0); ops.knn_search(t(same), t(b[:1, :100]), 7, 0); env()
