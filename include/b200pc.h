@@ -14,8 +14,11 @@
  *  - indices are int64 (torch.long), exactly as the reference produces/consumes them;
  *  - `stream` is a cudaStream_t passed as void* (NULL = legacy default stream); all work is
  *    stream-ordered, nothing synchronises, no global mutable state, re-entrant;
- *  - `workspace` is caller-owned device scratch of at least *_workspace_bytes(); it may be
- *    reused by the next call on the same stream;
+ *  - `workspace` is caller-owned device scratch of at least *_workspace_bytes(), 16-byte aligned (a search that needs
+ *    it returns B200PC_EINVAL otherwise); its contents on entry do not matter, and it may be reused by the next call on the same
+ *    stream;
+ *  - every other buffer needs only its element's natural alignment (4 bytes for fp32 / int32, 8 for int64) unless its
+ *    entry says otherwise; kernels that move 16-byte vectors check the alignment and take a scalar path without it;
  *  - return value: 0 on success, a negative B200PC_E* code on failure; the message is
  *    available from b200pc_last_error() (thread-local).  Nothing throws across this ABI.
  *  - there is NO CPU fallback: without a CUDA device every compute entry returns
@@ -196,7 +199,9 @@ int b200pc_channel_max(const float *x, int64_t rows, int C, float *out, b200pc_s
  *   peer memory); this rank's slab [s_offset, s_offset+S_local) is written into every one of them by the same kernel,
  *   so the all-gather of the shard outputs needs no separate collective -- the ranks meet at a barrier afterwards.
  * With n_peers == 0 the records stay local (single GPU, or an NCCL all_gather of local_out by the caller).
- * peer_out is a HOST array of device pointers.  workspace: b200pc_rebuild_pack_workspace_bytes().                    */
+ * peer_out is a HOST array of device pointers.  The records are stored 16 bytes at a time: local_out and every peer_out[p]
+ * must be 16-byte aligned (B200PC_EINVAL before anything is launched otherwise).
+ * workspace: b200pc_rebuild_pack_workspace_bytes().                                                                  */
 size_t b200pc_rebuild_pack_workspace_bytes(int B, int N, int S_local);
 int b200pc_rebuild_pack(const float *ref, const float *qry, int B, int N, int S_local, int s_offset, float *local_out,
                         void *const *peer_out, int n_peers, void *workspace, size_t workspace_bytes,

@@ -676,7 +676,18 @@ def chamfer(x, y):
 
 def poly_predict(frames, weights):
     """frames: list of F [B,...] fp32 CUDA tensors, weights [B,F] float64 on the device -> sum_f w[b,f] * frames[f][b]"""
-    return _O.poly_predict([_prep(f, "frame") for f in frames], weights.contiguous())
+    frames = [_prep(f, "frame") for f in frames]
+    if not frames:
+        raise ValueError("poly_predict: no frames")
+    shape, dev = frames[0].shape, frames[0].device
+    if any(f.shape != shape or f.device != dev for f in frames):
+        raise ValueError("poly_predict: all frames must share shape and device")
+    # the kernel reads B*F doubles from `weights`: anything else would read past the buffer or reinterpret its bits
+    if not isinstance(weights, torch.Tensor) or weights.dtype != torch.float64 or weights.device != dev:
+        raise ValueError("poly_predict: weights must be a float64 tensor on %s" % dev)
+    if tuple(weights.shape) != (shape[0], len(frames)):
+        raise ValueError("poly_predict: weights must be [B, F] = [%d, %d], got %s" % (shape[0], len(frames), tuple(weights.shape)))
+    return _O.poly_predict(frames, weights.contiguous())
 
 
 def reload_tuning():

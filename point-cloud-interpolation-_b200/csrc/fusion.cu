@@ -135,6 +135,11 @@ extern "C" int b200pc_rebuild_pack(const float *ref, const float *qry, int B, in
     if (B == 0 || S_local == 0) return B200PC_OK;
     B200PC_REQUIRE(ref && qry && (local_out || n_peers > 0), "rebuild_pack: null pointer");
     B200PC_REQUIRE(n_peers == 0 || peer_out, "rebuild_pack: n_peers=%d but no pointer array", n_peers);
+    // the records are stored as float4: every destination must be 16-byte aligned (checked before anything is launched)
+    B200PC_REQUIRE((reinterpret_cast<uintptr_t>(local_out) & 15) == 0, "rebuild_pack: local_out must be 16-byte aligned");
+    for (int p = 0; p < n_peers; ++p)
+        B200PC_REQUIRE(peer_out[p] && (reinterpret_cast<uintptr_t>(peer_out[p]) & 15) == 0,
+                       "rebuild_pack: peer_out[%d] must be a non-null, 16-byte aligned pointer", p);
     if (!workspace || workspace_bytes < b200pc_rebuild_pack_workspace_bytes(B, N, S_local)) {
         set_error("rebuild_pack: workspace too small (%zu < %zu bytes)", workspace_bytes, b200pc_rebuild_pack_workspace_bytes(B, N, S_local));
         return B200PC_EWORKSPACE;

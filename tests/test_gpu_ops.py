@@ -274,6 +274,22 @@ def test_poly_fit_rejects_cpu_and_bad_counts(cuda_dev):
         polypci.fit_and_predict(g, [[0.0, -1.0]], [0.5], 1)
 
 
+def test_poly_predict_rejects_weights_and_frames_it_cannot_read(cuda_dev):
+    """the kernel reads B*F doubles from `weights` and F frames of one shape: anything else is refused before the call"""
+    from b200pc import ops
+    f = [torch.zeros(2, 3, 8, device=cuda_dev) for _ in range(3)]
+    w = torch.zeros(2, 3, dtype=torch.float64, device=cuda_dev)
+    assert ops.poly_predict(f, w).shape == (2, 3, 8)
+    bad = {"float32 weights": (f, w.float()), "[B, F-1] weights": (f, w[:, :2].contiguous()),
+           "[F, B] weights": (f, torch.zeros(3, 2, dtype=torch.float64, device=cuda_dev)), "[B*F] weights": (f, w.reshape(-1)),
+           "weights on the host": (f, w.cpu()), "frames of two shapes": (f[:2] + [torch.zeros(2, 3, 9, device=cuda_dev)], w),
+           "no frames": ([], w[:, :0])}
+    for what, (frames, weights) in bad.items():
+        with pytest.raises(ValueError):
+            ops.poly_predict(frames, weights)
+        torch.cuda.synchronize()
+
+
 def test_sample_points_is_fps_plus_gather(cuda_dev):
     # Sample.forward (Utils/Layers.py:23-27): the FPS kernel also writes the picks' coordinates
     a, _ = synth.batch_pairs(60, 3, 16384)

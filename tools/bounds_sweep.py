@@ -149,4 +149,91 @@ ops.unpack_rebuild(ops.rebuild_pack(ref, qry))
 from b200pc import polypci
 frames = [torch.randn(2, 3, 2000, device=dev) for _ in range(5)]
 polypci.fit_and_predict(frames, [[0.0, 1.0, -1.0, 2.0, -2.0]] * 2, [0.5, -0.25], 3)
+torch.cuda.synchronize(); print("row movers ok", flush=True)
+
+# ---- the C entries at the smallest offsets the contract allows (tests/test_gpu_buffer_hygiene.py): fp32 / int32 buffers 4 bytes
+# and int64 buffers 8 bytes past a 256-byte boundary, the search workspace and the 16-byte records 16 bytes past one, and the
+# kernels that accumulate into a non-zero base
+import ctypes as C
+lib = _lib.load()
+
+
+def off(a, align):
+    """a device copy of `a` whose data starts `align` bytes past a 256-byte boundary"""
+    a = torch.as_tensor(np.ascontiguousarray(a)) if isinstance(a, np.ndarray) else a
+    n = a.numel() * a.element_size()
+    raw = torch.empty(n + 512, dtype=torch.uint8, device=dev)
+    s = (align - raw.data_ptr()) % 256
+    v = raw[s:s + n].view(a.dtype).view(a.shape)
+    v.copy_(a)
+    return v
+
+
+def f32(*shape):
+    return off(torch.randn(*shape), 4)
+
+
+def i64(a):
+    return off(torch.as_tensor(np.asarray(a, np.int64)), 8)
+
+
+def ok(rc):
+    assert rc == 0, lib.b200pc_last_error()
+
+
+def p(x):
+    return x.data_ptr() if x is not None else None
+
+
+st = C.c_void_p(torch.cuda.current_stream().cuda_stream)
+for (B, N, S, k), kw in (((2, 513, 77, 300), dict(SMALL_PATH=0, GRID=0, FORCE_SPLIT=2)), ((2, 5000, 700, 16), dict(SMALL_PATH=0, GRID=3, FORCE_SPLIT=3)),
+                         ((2, 700, 333, 16), dict(SMALL_PATH=1)), ((2, 3000, 333, 16), dict(SMALL_PATH=0, FORCE_Q=2, GRID=0))):
+    env(**kw); ops.reload_tuning()
+    a, b = synth.batch_pairs(14, B, max(N, S))
+    a[B - 1, 2:] = np.nan
+    ref, qry = off(a[:, :N].copy(), 4), off(b[:, :S].copy(), 4)
+    nws = lib.b200pc_search_workspace_bytes(B, N, S, k)
+    ws = off(torch.empty(nws, dtype=torch.uint8), 16)
+    ok(lib.b200pc_knn(p(ref), p(qry), B, N, S, k, 0, p(i64(np.zeros((B, S, k)))), p(f32(B, S, k)), p(ws), nws, st))
+    ok(lib.b200pc_knn_i32(p(ref), p(qry), B, N, S, k, 2, p(off(torch.zeros(B, S, k, dtype=torch.int32), 4)), p(f32(B, S, k)), p(ws), nws, st))
+    ok(lib.b200pc_ball_query(p(ref), p(qry), B, N, S, C.c_float(1.0), min(k, 64), p(i64(np.zeros((B, S, min(k, 64))))), p(ws), nws, st))
+    nws3 = lib.b200pc_search_workspace_bytes(B, N, S, 3)
+    ws3 = off(torch.empty(nws3, dtype=torch.uint8), 16)
+    ok(lib.b200pc_three_nn(p(qry), p(ref), B, S, N, 0, p(f32(B, S, 3)), p(i64(np.zeros((B, S, 3)))), p(f32(B, S, 3)), p(ws3), nws3, st))
+env(); ops.reload_tuning()
+B, N, S, R = 2, 900, 123, 777
+pts, new = f32(B, N, 64), f32(B, S, 3)
+gidx = np.random.default_rng(5).integers(-N, N, size=(B, R)); gidx[:, ::37] = N
+ok(lib.b200pc_gather(p(pts), p(i64(gidx)), B, N, 64, R, p(f32(B, R, 64)), p(off(torch.zeros(1, dtype=torch.int32), 4)), st))
+ok(lib.b200pc_gather_bwd(p(f32(B, R, 64)), p(i64(gidx)), B, N, 64, R, p(f32(B, N, 64)), st))
+i3 = np.random.default_rng(6).integers(-1, S, size=(B, N, 3))
+ok(lib.b200pc_three_interpolate(p(f32(B, S, 12)), p(i64(i3)), p(f32(B, N, 3)), B, S, N, 12, p(f32(B, N, 12)), st))
+ok(lib.b200pc_three_interpolate_bwd(p(f32(B, N, 12)), p(f32(B, S, 12)), p(i64(i3)), p(f32(B, N, 3)), B, S, N, 12, p(f32(B, S, 12)), p(f32(B, N, 3)), st))
+gk = np.random.default_rng(7).integers(-N, N + 1, size=(B, S, 16))
+for bulk in (0, 1):
+    env(BULK=bulk); ops.reload_tuning()
+    for xf in (0, 1):
+        ok(lib.b200pc_group_points(p(pts[..., :3].contiguous()), p(new), p(pts), p(i64(gk)), B, N, S, 16, 64, xf, p(f32(B, 67, 16, S)), st))
+        ok(lib.b200pc_group_points_bwd(p(f32(B, 67, 16, S)), p(i64(gk)), B, N, S, 16, 64, xf, p(f32(B, N, 64)), st))
+env(); ops.reload_tuning()
+ok(lib.b200pc_square_distance(p(f32(B, 77, 3)), p(f32(B, 1004, 3)), B, 77, 1004, p(f32(B, 77, 1004)), st))
+ok(lib.b200pc_channel_max(p(off(torch.randn(1001, 4), 16)), 1001, 4, p(f32(1001)), st))
+fr = [f32(3, 999) for _ in range(16)]
+ok(lib.b200pc_poly_predict((C.c_void_p * 16)(*[p(f) for f in fr]), p(off(torch.randn(3, 16, dtype=torch.float64), 8)), 3, 16, 999, p(f32(3, 999)), st))
+a, b = synth.batch_pairs(15, 2, 1200)
+ref, qry = off(a, 4), off(b[:, :333].copy(), 4)
+nws = lib.b200pc_search_workspace_bytes(2, 1200, 333, 16)
+ws = off(torch.empty(nws, dtype=torch.uint8), 16)
+ok(lib.b200pc_fusion_group(p(qry), p(ref), p(f32(2, 1200, 13)), 2, 1200, 333, 16, 13, p(f32(2, 4, 333, 16)), p(f32(2, 3, 333, 16)),
+                           p(f32(2, 13, 333, 16)), p(i64(np.zeros((2, 333, 16)))), p(ws), nws, st))
+ix, iy = i64(np.zeros((2, 333))), i64(np.zeros((2, 1200)))
+nws = max(lib.b200pc_search_workspace_bytes(2, 1200, 333, 1), lib.b200pc_search_workspace_bytes(2, 333, 1200, 1))
+ws = off(torch.empty(nws, dtype=torch.uint8), 16)
+ok(lib.b200pc_chamfer_fwd(p(qry), p(ref), 2, 333, 1200, p(f32(2, 333)), p(ix), p(f32(2, 1200)), p(iy), p(f32(1)), p(ws), nws, st))
+ok(lib.b200pc_chamfer_bwd(p(qry), p(ref), p(ix), p(iy), p(f32(1)), 2, 333, 1200, p(f32(2, 333, 3)), p(f32(2, 1200, 3)), st))
+nws = lib.b200pc_rebuild_pack_workspace_bytes(2, 1200, 333)
+ws = off(torch.empty(nws, dtype=torch.uint8), 16)
+peers = [off(torch.randn(1500, 2, 4), 16) for _ in range(8)]
+ok(lib.b200pc_rebuild_pack(p(ref), p(qry), 2, 1200, 333, 700, p(off(torch.zeros(333, 2, 4), 16)), (C.c_void_p * 8)(*[p(q) for q in peers]), 8,
+                           p(ws), nws, st))
 torch.cuda.synchronize(); print("bounds sweep ok", flush=True)
