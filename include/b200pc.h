@@ -95,6 +95,21 @@ int b200pc_square_distance(const float *src, const float *dst, int B, int N, int
 int b200pc_knn(const float *ref, const float *qry, int B, int N, int S, int k, int form, int64_t *idx,
                float *dist, void *workspace, size_t workspace_bytes, b200pc_stream_t stream);
 
+/* Ragged batches: pytorch3d.ops.knn_points(p1=qry, p2=ref, lengths1=qry_len, lengths2=ref_len, K=k) for clouds of
+ * different sizes padded to [B,N,3] / [B,S,3] (LiDAR sweeps: the number of valid returns changes from frame to frame).
+ * ref_len, qry_len: DEVICE int64 [B] (torch.long, as in pytorch3d); either may be NULL = every item full.  With
+ * n_b = clamp(ref_len[b], 0, N) and s_b = clamp(qry_len[b], 0, S) -- clamped on the device, nothing is read back:
+ *   rows q <  s_b: bit-identical (indices and distances) to b200pc_knn of qry[b,q] against ref[b, :n_b] -- same form, same
+ *                  (distance, index) order, same non-finite rule; k > n_b (n_b == 0 included) ends the row in -1 / +inf;
+ *   rows q >= s_b: every slot -1 / +inf.
+ * No output depends on the contents of the padded rows (ref[b, n_b:], qry[b, s_b:]).  The work follows the lengths: an
+ * item's refs fill ceil(n_b / 512) tiles, padded queries are not searched.  k <= N (EINVAL otherwise, like b200pc_knn);
+ * workspace: b200pc_search_workspace_bytes(B, N, S, k) of the padded shape.  pytorch3d's zero padding of the empty slots
+ * is the facade's business (b200pc.pytorch3d_shim); this entry keeps -1 / +inf.                                     */
+int b200pc_knn_ragged(const float *ref, const float *qry, const int64_t *ref_len, const int64_t *qry_len, int B, int N,
+                      int S, int k, int form, int64_t *idx, float *dist, void *workspace, size_t workspace_bytes,
+                      b200pc_stream_t stream);
+
 /* The same search with 32-bit indices (N < 2^31 always holds): for host-buffer callers that read the result back over
  * PCIe -- half the bytes of the int64 form the reference's tensors use.  Same order, same ties, -1 for unfilled slots. */
 int b200pc_knn_i32(const float *ref, const float *qry, int B, int N, int S, int k, int form, int32_t *idx, float *dist,
@@ -228,6 +243,24 @@ int b200pc_chamfer_fwd(const float *x, const float *y, int B, int N, int M, floa
 /* gx [B,N,3], gy [B,M,3] are written (zero-filled internally); gloss is a device scalar.     */
 int b200pc_chamfer_bwd(const float *x, const float *y, const int64_t *ix, const int64_t *iy, const float *gloss,
                        int B, int N, int M, float *gx, float *gy, b200pc_stream_t stream);
+
+/* Ragged Chamfer: pytorch3d.loss.chamfer_distance(x, y, x_lengths=x_len, y_lengths=y_len) with any point / batch reduction,
+ * e.g. per-sample scores (batch_reduction=None) of interpolated frames against full-resolution sweeps of other sizes.
+ * x [B,N,3], y [B,M,3] padded; x_len, y_len: DEVICE int64 [B] or NULL (full), clamped to [0,N] / [0,M] on the device.
+ * Per point, as b200pc_chamfer_fwd against the other cloud's valid points (the two searches of b200pc_knn_ragged, K = 1,
+ * form 2); padded points get index -1 and minimum +inf.  sums [B,2] fp32 = { sum of dx[b,i] over i < x_len[b],
+ * sum of dy[b,j] over j < y_len[b] }, accumulated in double in a fixed order (the same bits on every run).  The reductions
+ * ("mean": divide by max(len, 1); "sum"; batch "mean" / "sum" / none) are left to the caller.  An empty item sums to 0.
+ * workspace: max(b200pc_search_workspace_bytes(B, M, N, 1), b200pc_search_workspace_bytes(B, N, M, 1)).            */
+int b200pc_chamfer_ragged_fwd(const float *x, const float *y, const int64_t *x_len, const int64_t *y_len, int B, int N,
+                              int M, float *dx, int64_t *ix, float *dy, int64_t *iy, float *sums, void *workspace,
+                              size_t workspace_bytes, b200pc_stream_t stream);
+/* gsums [B,2] (device) = d loss / d sums.  gx [B,N,3], gy [B,M,3] are written (zero-filled internally):
+ * 2 gsums[b,0] (x_i - y_ix) into x_i and its negative into y_ix, likewise for y with gsums[b,1].  A padded point, or one
+ * with index -1, gives and receives no gradient.                                                                     */
+int b200pc_chamfer_ragged_bwd(const float *x, const float *y, const int64_t *ix, const int64_t *iy, const int64_t *x_len,
+                              const int64_t *y_len, const float *gsums, int B, int N, int M, float *gx, float *gy,
+                              b200pc_stream_t stream);
 
 /* ---- measurement helper: sustained FP32 FMA throughput of the current device ------------- */
 /* runs a register-resident FFMA2 chain kernel for `iters` iterations; *tflops receives the

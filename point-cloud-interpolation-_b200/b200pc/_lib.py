@@ -30,6 +30,7 @@ SIGNATURES = {
     "b200pc_fps_workspace_bytes": (_z, [_i, _i]),
     "b200pc_square_distance": (_i, [_p, _p, _i, _i, _i, _p, _p]),
     "b200pc_knn": (_i, [_p, _p, _i, _i, _i, _i, _i, _p, _p, _p, _z, _p]),
+    "b200pc_knn_ragged": (_i, [_p, _p, _p, _p, _i, _i, _i, _i, _i, _p, _p, _p, _z, _p]),
     "b200pc_knn_i32": (_i, [_p, _p, _i, _i, _i, _i, _i, _p, _p, _p, _z, _p]),
     "b200pc_ball_query": (_i, [_p, _p, _i, _i, _i, _f, _i, _p, _p, _z, _p]),
     "b200pc_three_nn": (_i, [_p, _p, _i, _i, _i, _i, _p, _p, _p, _p, _z, _p]),
@@ -50,6 +51,8 @@ SIGNATURES = {
     "b200pc_group_points_bwd": (_i, [_p, _p, _i, _i, _i, _i, _i, _i, _p, _p]),
     "b200pc_chamfer_fwd": (_i, [_p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _z, _p]),
     "b200pc_chamfer_bwd": (_i, [_p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p]),
+    "b200pc_chamfer_ragged_fwd": (_i, [_p, _p, _p, _p, _i, _i, _i, _p, _p, _p, _p, _p, _p, _z, _p]),
+    "b200pc_chamfer_ragged_bwd": (_i, [_p, _p, _p, _p, _p, _p, _p, _i, _i, _i, _p, _p, _p]),
     "b200pc_fma_peak": (_i, [_i, C.POINTER(C.c_double), C.POINTER(C.c_double), _p]),
     "b200pc_knn_host": (_i, [_p, _p, _i, _i, _i, _i, _i, _p, _p]),
     "b200pc_ball_query_host": (_i, [_p, _p, _i, _i, _i, _f, _i, _p]),

@@ -93,6 +93,7 @@ OP_SCHEMAS = {
     # op name == C entry point without the b200pc_ prefix (tests/test_abi.py keeps the two lists in step)
     "square_distance": "(Tensor src, Tensor dst) -> Tensor",
     "knn": "(Tensor ref, Tensor qry, int k, int form, bool want_dist) -> (Tensor, Tensor)",
+    "knn_ragged": "(Tensor ref, Tensor qry, Tensor? ref_len, Tensor? qry_len, int k, int form, bool want_dist) -> (Tensor, Tensor)",
     "knn_i32": "(Tensor ref, Tensor qry, int k, int form) -> Tensor",
     "ball_query": "(Tensor xyz, Tensor new_xyz, float r2, int nsample) -> Tensor",
     "fps": "(Tensor xyz, int npoint, Tensor start) -> Tensor",
@@ -110,6 +111,8 @@ OP_SCHEMAS = {
     "rebuild_pack": "(Tensor ref, Tensor qry, int s_offset, int[] peer_ptrs) -> Tensor",
     "chamfer_fwd": "(Tensor x, Tensor y) -> (Tensor, Tensor, Tensor, Tensor, Tensor)",
     "chamfer_bwd": "(Tensor x, Tensor y, Tensor ix, Tensor iy, Tensor gloss) -> (Tensor, Tensor)",
+    "chamfer_ragged_fwd": "(Tensor x, Tensor y, Tensor? x_len, Tensor? y_len) -> (Tensor, Tensor, Tensor, Tensor, Tensor)",
+    "chamfer_ragged_bwd": "(Tensor x, Tensor y, Tensor ix, Tensor iy, Tensor? x_len, Tensor? y_len, Tensor gsums) -> (Tensor, Tensor)",
     "poly_predict": "(Tensor[] frames, Tensor weights) -> Tensor",
 }
 for _name, _schema in OP_SCHEMAS.items():
@@ -157,6 +160,20 @@ def _knn(ref, qry, k, form, want_dist):
     nws = _search_ws(lib, B, N, S, k)
     ws = _workspace(nws, dev)
     _call(dev, lib.b200pc_knn, _ptr(ref), _ptr(qry), B, N, S, k, int(form), _ptr(idx), _ptr(dist), _ptr(ws), nws, _stream(dev))
+    return idx, (dist if want_dist else _f32(B, S, 0, like=ref))
+
+
+@_register("knn_ragged", lambda ref, qry, ref_len, qry_len, k, form, want_dist: _knn_fake(ref, qry, k, form, want_dist))
+def _knn_ragged(ref, qry, ref_len, qry_len, k, form, want_dist):
+    B, N, _ = ref.shape; S = qry.shape[1]
+    dev = ref.device
+    idx = _i64(B, S, k, like=ref)
+    dist = _f32(B, S, k, like=ref) if want_dist else None
+    lib = _lib.load()
+    nws = _search_ws(lib, B, N, S, k)
+    ws = _workspace(nws, dev)
+    _call(dev, lib.b200pc_knn_ragged, _ptr(ref), _ptr(qry), _ptr(ref_len), _ptr(qry_len), B, N, S, k, int(form), _ptr(idx), _ptr(dist),
+          _ptr(ws), nws, _stream(dev))
     return idx, (dist if want_dist else _f32(B, S, 0, like=ref))
 
 
@@ -492,6 +509,50 @@ def _chamfer_backward(ctx, gloss, *_):
 torch.library.register_autograd("b200pc::chamfer_fwd", _chamfer_backward, setup_context=_chamfer_setup, lib=_L)
 
 
+def _chamfer_ragged_fake(x, y, x_len, y_len):
+    B, N, M = x.shape[0], x.shape[1], y.shape[1]
+    return _f32(B, 2, like=x), _f32(B, N, like=x), _i64(B, N, like=x), _f32(B, M, like=x), _i64(B, M, like=x)
+
+
+@_register("chamfer_ragged_fwd", _chamfer_ragged_fake)
+def _chamfer_ragged_fwd(x, y, x_len, y_len):
+    B, N, _ = x.shape; M = y.shape[1]
+    dev = x.device
+    dx = _f32(B, N, like=x); ix = _i64(B, N, like=x)
+    dy = _f32(B, M, like=x); iy = _i64(B, M, like=x)
+    sums = _f32(B, 2, like=x)
+    lib = _lib.load()
+    nws = max(_search_ws(lib, B, M, N, 1), _search_ws(lib, B, N, M, 1))
+    ws = _workspace(nws, dev)
+    _call(dev, lib.b200pc_chamfer_ragged_fwd, _ptr(x), _ptr(y), _ptr(x_len), _ptr(y_len), B, N, M, _ptr(dx), _ptr(ix), _ptr(dy), _ptr(iy),
+          _ptr(sums), _ptr(ws), nws, _stream(dev))
+    return sums, dx, ix, dy, iy
+
+
+@_register("chamfer_ragged_bwd", lambda x, y, ix, iy, x_len, y_len, gsums: (torch.empty_like(x), torch.empty_like(y)))
+def _chamfer_ragged_bwd(x, y, ix, iy, x_len, y_len, gsums):
+    B, N, _ = x.shape; M = y.shape[1]
+    gx = torch.empty_like(x); gy = torch.empty_like(y)
+    _call(x.device, _lib.load().b200pc_chamfer_ragged_bwd, _ptr(x), _ptr(y), _ptr(ix), _ptr(iy), _ptr(x_len), _ptr(y_len), _ptr(gsums),
+          B, N, M, _ptr(gx), _ptr(gy), _stream(x.device))
+    return gx, gy
+
+
+def _chamfer_ragged_setup(ctx, inputs, output):
+    x, y, x_len, y_len = inputs
+    _, _, ix, _, iy = output
+    ctx.save_for_backward(x, y, ix, iy, x_len, y_len)
+
+
+def _chamfer_ragged_backward(ctx, gsums, *_):
+    x, y, ix, iy, x_len, y_len = ctx.saved_tensors
+    gx, gy = torch.ops.b200pc.chamfer_ragged_bwd(x, y, ix, iy, x_len, y_len, gsums.contiguous().float())
+    return gx, gy, None, None
+
+
+torch.library.register_autograd("b200pc::chamfer_ragged_fwd", _chamfer_ragged_backward, setup_context=_chamfer_ragged_setup, lib=_L)
+
+
 # ---- f4 ----------------------------------------------------------------------------------
 @_register("poly_predict", lambda frames, weights: torch.empty_like(frames[0]))
 def _poly_predict(frames, weights):
@@ -523,6 +584,36 @@ def knn_search(ref, qry, k, form, want_dist=False):
     if k > ref.shape[1]:   # torch.topk raises RuntimeError("selected index k out of range")
         raise RuntimeError("selected index k out of range (k=%d > %d reference points)" % (k, ref.shape[1]))
     idx, dist = _O.knn(ref.detach(), qry.detach(), k, int(form), bool(want_dist))      # indices / raw distances carry no gradient
+    return (idx, dist) if want_dist else idx
+
+
+def _lengths(lengths, B, dev, name):
+    """per-item lengths of a ragged batch: None (every item full) or int64 [B] on `dev`.  The values are NOT checked on
+    the host (that would cost a device->host sync): the kernels clamp them to [0, padded size]."""
+    if lengths is None:
+        return None
+    if not isinstance(lengths, torch.Tensor):
+        raise TypeError("%s must be a torch.Tensor or None" % name)
+    if lengths.dtype.is_floating_point or lengths.dtype.is_complex or lengths.dtype == torch.bool:
+        raise TypeError("%s must be an integer tensor, got %s" % (name, lengths.dtype))
+    if tuple(lengths.shape) != (B,):
+        raise ValueError("%s must have shape [%d], got %s" % (name, B, tuple(lengths.shape)))
+    return _idx64(lengths, dev)
+
+
+def knn_ragged(ref, qry, k, form, ref_len=None, qry_len=None, want_dist=False):
+    """knn_search on a ragged batch: item b has ref_len[b] valid refs and qry_len[b] valid queries (int [B] tensors or None
+    = full; clamped to [0, N] / [0, S] on the device).  Valid rows equal knn_search of qry[b, :s_b] against ref[b, :n_b] bit
+    for bit; slots without a valid ref and padded rows are -1 / +inf.  k <= N; k > ref_len[b] is allowed."""
+    ref = _prep(ref, "ref"); qry = _prep(qry, "qry")
+    k = int(k)
+    if k > ref.shape[1]:
+        raise RuntimeError("selected index k out of range (k=%d > %d reference points)" % (k, ref.shape[1]))
+    if ref.shape[0] != qry.shape[0]:
+        raise ValueError("knn_ragged: ref and qry must have the same batch size")
+    B = ref.shape[0]
+    rl = _lengths(ref_len, B, ref.device, "ref_len"); ql = _lengths(qry_len, B, ref.device, "qry_len")
+    idx, dist = _O.knn_ragged(ref.detach(), qry.detach(), rl, ql, k, int(form), bool(want_dist))
     return (idx, dist) if want_dist else idx
 
 
@@ -672,6 +763,42 @@ def unpack_rebuild(records):
 def chamfer(x, y):
     """x [B,N,3], y [B,M,3] -> (loss scalar, dx [B,N], ix [B,N], dy [B,M], iy [B,M]); loss is differentiable."""
     return _O.chamfer_fwd(_prep(x, "x"), _prep(y, "y"))
+
+
+def chamfer_ragged(x, y, x_len=None, y_len=None):
+    """Chamfer terms of a ragged batch: x [B,N,3], y [B,M,3] padded, x_len / y_len int [B] tensors or None (full).
+    -> (sums [B,2] = per-item sums of the valid points' minima in each direction, differentiable in x and y;
+        dx [B,N], ix [B,N], dy [B,M], iy [B,M] with -1 / +inf for padded points).  The point / batch reductions are torch
+    arithmetic on `sums` (chamfer_reduce)."""
+    x = _prep(x, "x"); y = _prep(y, "y")
+    if x.shape[0] != y.shape[0]:
+        raise ValueError("chamfer_ragged: x and y must have the same batch size")
+    B = x.shape[0]
+    return _O.chamfer_ragged_fwd(x, y, _lengths(x_len, B, x.device, "x_len"), _lengths(y_len, B, x.device, "y_len"))
+
+
+def chamfer_reduce(sums, x_len, y_len, N, M, point_reduction="mean", batch_reduction="mean"):
+    """pytorch3d.loss.chamfer_distance's reductions of the per-item sums [B,2]: point_reduction "mean" divides each sum
+    by max(length, 1) (the padded size when the lengths are None), "sum" keeps it; batch_reduction "mean" / "sum" / None
+    (-> [B])."""
+    if point_reduction not in ("mean", "sum"):
+        raise ValueError('point_reduction must be "mean" or "sum", got %r' % (point_reduction,))
+    if batch_reduction not in ("mean", "sum", None):
+        raise ValueError('batch_reduction must be "mean", "sum" or None, got %r' % (batch_reduction,))
+    B = sums.shape[0]
+    cx, cy = sums[:, 0], sums[:, 1]
+    if point_reduction == "mean":
+        def div(lengths, full):
+            if lengths is None:
+                return torch.full((B,), float(max(full, 1)), dtype=sums.dtype, device=sums.device)
+            return lengths.to(sums.device).clamp(0, full).clamp(min=1).to(sums.dtype)
+        cx = cx / div(x_len, N)
+        cy = cy / div(y_len, M)
+    def batch(c):                  # per direction, then added, in pytorch3d's order
+        if batch_reduction is None:
+            return c
+        return c.sum() / max(B, 1) if batch_reduction == "mean" else c.sum()
+    return batch(cx) + batch(cy)
 
 
 def poly_predict(frames, weights):

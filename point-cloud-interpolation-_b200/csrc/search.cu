@@ -78,21 +78,27 @@ __device__ __forceinline__ int slot_to_ref(int s, int strided, int n_tiles) {
 }
 static_assert(TILE == 512, "slot_to_ref assumes 512-slot tiles");
 
+// Ragged batches (item_len, search.cuh): an item's refs are dealt into its OWN ceil(n_b / 512) tiles (slot_to_ref with n_tiles = this count): the slots of those
+// tiles past n_b are padding records, the tiles behind them are never packed or visited.  Dense calls: n_b = N, so this is
+// the padded tile count and nothing changes.
+__device__ __forceinline__ int item_tiles(int n_b) { return (n_b + TILE - 1) / TILE; }
+
 struct GridDesc;
 __device__ __forceinline__ void grid_count_ref(const GridDesc *desc, unsigned *counts, int b, float x, float y, float z);
 
 // grid != null: also count the ref into the occupancy grid (section 1b, the variant without sorting)
-__global__ void pack_refs_kernel(const float *__restrict__ ref, int N, int n_pad, int strided, float4 *__restrict__ packed,
-                                 const GridDesc *__restrict__ grid, unsigned *__restrict__ counts) {
+__global__ void pack_refs_kernel(const float *__restrict__ ref, const int64_t *__restrict__ ref_len, int N, int n_pad, int strided,
+                                 float4 *__restrict__ packed, const GridDesc *__restrict__ grid, unsigned *__restrict__ counts) {
     const int p = blockIdx.x * blockDim.x + threadIdx.x;  // pair index
-    if (p >= n_pad / 2) return;
     const int b = blockIdx.y;
+    const int n_b = item_len(ref_len, b, N), nt_b = item_tiles(n_b);
+    if (p >= nt_b * (TILE / 2)) return;
     const float *r = ref + (size_t)b * N * 3;
     float x[2], y[2], z[2], w[2];
 #pragma unroll
     for (int h = 0; h < 2; ++h) {
-        const int i = slot_to_ref(2 * p + h, strided, n_pad / TILE);
-        if (i < N) {
+        const int i = slot_to_ref(2 * p + h, strided, nt_b);
+        if (i < n_b) {
             x[h] = r[i * 3 + 0]; y[h] = r[i * 3 + 1]; z[h] = r[i * 3 + 2];
             w[h] = filter_norm(torch_sq_norm(x[h], y[h], z[h]));
             if (grid) grid_count_ref(grid, counts, b, x[h], y[h], z[h]);
@@ -191,17 +197,21 @@ __device__ __forceinline__ int grid_cell_index(const GridDesc &g, float x, float
     return (cz * g.dim[0][1] + cy) * g.dim[0][0] + cx;
 }
 
-__global__ void __launch_bounds__(1024) grid_bbox_kernel(const float *__restrict__ ref, int N, GridDesc *__restrict__ desc) {
+// only the item's valid refs (i < n_b) enter the box and n_finite: an item with fewer than k of them starts from +inf, and
+// one with none has an empty box (lo = +inf, hi = -inf, one cell)
+__global__ void __launch_bounds__(1024) grid_bbox_kernel(const float *__restrict__ ref, const int64_t *__restrict__ ref_len, int N,
+                                                         GridDesc *__restrict__ desc) {
     const int b = blockIdx.x;
+    const int n_b = item_len(ref_len, b, N);
     const float *r = ref + (size_t)b * N * 3;
     float lo[3] = {CUDART_INF_F, CUDART_INF_F, CUDART_INF_F}, hi[3] = {-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F};
     int nf = 0;
-    for (int i0 = threadIdx.x; i0 < N; i0 += 4 * blockDim.x) {          // four points per thread in flight
+    for (int i0 = threadIdx.x; i0 < n_b; i0 += 4 * blockDim.x) {        // four points per thread in flight
         float x[4], y[4], z[4];
 #pragma unroll
         for (int u = 0; u < 4; ++u) {
             const int i = i0 + u * blockDim.x;
-            const bool in = i < N;
+            const bool in = i < n_b;
             x[u] = in ? r[i * 3] : CUDART_NAN_F; y[u] = in ? r[i * 3 + 1] : 0.f; z[u] = in ? r[i * 3 + 2] : 0.f;
         }
 #pragma unroll
@@ -279,12 +289,15 @@ __device__ __forceinline__ void grid_count_ref(const GridDesc *desc, unsigned *c
     if (isfinite(x) && isfinite(y) && isfinite(z)) atomicAdd(counts + (size_t)b * GRID_STRIDE + grid_cell_index(desc[b], x, y, z), 1u);
 }
 
-// one atomic per point: refs (finite ones) into counts, queries (clamped into the border cells; NaN -> cell 0) into qcend
-__global__ void __launch_bounds__(256) grid_count_kernel(const float *__restrict__ ref, int N, const float *__restrict__ qry, int S,
+// one atomic per point: refs (finite ones) into counts, queries (clamped into the border cells; NaN -> cell 0) into qcend.
+// Padded refs and queries of a ragged item are not counted.
+__global__ void __launch_bounds__(256) grid_count_kernel(const float *__restrict__ ref, const int64_t *__restrict__ ref_len, int N,
+                                                         const float *__restrict__ qry, const int64_t *__restrict__ qry_len, int S,
                                                          const GridDesc *__restrict__ desc, unsigned *__restrict__ counts,
                                                          unsigned *__restrict__ qcend) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
     if (i >= N + S) return;
+    if (i < N ? i >= item_len(ref_len, b, N) : i - N >= item_len(qry_len, b, S)) return;
     const GridDesc &g = desc[b];
     const float *p = i < N ? ref + ((size_t)b * N + i) * 3 : qry + ((size_t)b * S + (i - N)) * 3;
     const float x = p[0], y = p[1], z = p[2];
@@ -469,34 +482,39 @@ __device__ __forceinline__ unsigned sorted_slot(unsigned p, int n_tiles, int tps
     return s * span + (r - q * t) * TILE + q;
 }
 
-__global__ void __launch_bounds__(256) grid_scatter_kernel(const float *__restrict__ ref, int N, int n_pad, int tps, const float *__restrict__ qry,
-                                                           int S, const GridDesc *__restrict__ desc, GridBufs gb, float4 *__restrict__ packed, int k_seed) {
+// Ragged items: positions n_b .. 512 * item_tiles(n_b) - 1 are the padding of the item's own tiles, the slots behind them
+// are left alone (never visited), and only the s_b valid queries enter the sorted copy (positions 0 .. s_b - 1).
+__global__ void __launch_bounds__(256) grid_scatter_kernel(const float *__restrict__ ref, const int64_t *__restrict__ ref_len, int N, int n_pad,
+                                                           int tps, const float *__restrict__ qry, const int64_t *__restrict__ qry_len, int S,
+                                                           const GridDesc *__restrict__ desc, GridBufs gb, float4 *__restrict__ packed, int k_seed) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.y;
     const GridDesc &g = desc[b];
     if (i < n_pad) {
+        const int n_b = item_len(ref_len, b, N), nt_b = item_tiles(n_b);
+        if (i >= nt_b * TILE) return;
         float x = CUDART_INF_F, y = 0.0f, z = 0.0f, w = CUDART_INF_F;    // padding (see pack_refs_kernel)
         unsigned pos = (unsigned)i;
-        if (i < N) {
+        if (i < n_b) {
             const float *r = ref + ((size_t)b * N + i) * 3;
             x = r[0]; y = r[1]; z = r[2];
             w = filter_norm(torch_sq_norm(x, y, z));
             if (isfinite(x) && isfinite(y) && isfinite(z)) pos = atomicAdd(gb.cend + (size_t)b * GRID_MAX_CELLS + grid_cell_index(g, x, y, z), 1u);
             else pos = (unsigned)g.n_finite + atomicAdd(gb.tail + b, 1u);
-            B200PC_DEV_ASSERT(pos < (unsigned)N);
+            B200PC_DEV_ASSERT(pos < (unsigned)n_b);
             if (k_seed == 0) gb.sorted[(size_t)b * N + pos] = make_float4(x, y, z, __int_as_float(i));   // only grid_seed_kernel reads it
         }
-        const unsigned sl = sorted_slot(pos, n_pad / TILE, tps);
-        B200PC_DEV_ASSERT(sl < (unsigned)n_pad);
+        const unsigned sl = sorted_slot(pos, nt_b, tps);
+        B200PC_DEV_ASSERT(sl < (unsigned)(nt_b * TILE));
         gb.perm[(size_t)b * n_pad + sl] = i;
         const unsigned chunk = sl >> 3, slot = ((sl >> 1) & 3u) ^ (chunk & 3u);
         float *o = reinterpret_cast<float *>(packed + ((size_t)b * (n_pad / 2) + (size_t)chunk * 4 + slot) * 2) + (sl & 1u);
         o[0] = x; o[2] = y; o[4] = z; o[6] = w;
-    } else if (i - n_pad < S) {
+    } else if (i - n_pad < item_len(qry_len, b, S)) {
         const int j = i - n_pad;
         const float *qp = qry + ((size_t)b * S + j) * 3;
         const float x = qp[0], y = qp[1], z = qp[2];
         const unsigned pos = atomicAdd(gb.qcend + (size_t)b * GRID_MAX_CELLS + grid_cell_index(g, x, y, z), 1u);
-        B200PC_DEV_ASSERT(pos < (unsigned)S);
+        B200PC_DEV_ASSERT(pos < (unsigned)item_len(qry_len, b, S));
         gb.qsorted[(size_t)b * S + pos] = make_float4(x, y, z, __int_as_float(j));
         if (k_seed > 0) {                                  // the query's starting threshold, here rather than in a launch of its own
             const float q[3] = {x, y, z};
@@ -522,7 +540,8 @@ __global__ void __launch_bounds__(256) grid_scatter_kernel(const float *__restri
 // Queries with no such box take the corner bound of the whole bounding box; non-finite queries and clouds with fewer than
 // k finite refs start from +inf.  Boxes of level >= `exact` are not looked into: their queries take the box's corner bound.
 constexpr int SEED_THREADS = 128, SEED_BINS = 64, SEED_SHIFT = 21, SEED_MAX_REFS = 192;
-__global__ void __launch_bounds__(SEED_THREADS) grid_seed_kernel(const float4 *__restrict__ qsorted, const float *__restrict__ qraw, int S, int N, int k,
+__global__ void __launch_bounds__(SEED_THREADS) grid_seed_kernel(const float4 *__restrict__ qsorted, const float *__restrict__ qraw,
+                                                                 const int64_t *__restrict__ qry_len, int S, int N, int k,
                                                                  const GridDesc *__restrict__ desc, const unsigned *__restrict__ counts,
                                                                  const unsigned *__restrict__ cend, const float4 *__restrict__ sorted,
                                                                  float *__restrict__ seed, int exact) {
@@ -536,7 +555,7 @@ __global__ void __launch_bounds__(SEED_THREADS) grid_seed_kernel(const float4 *_
         for (int i = threadIdx.x; i < SEED_BINS * SEED_THREADS / 8; i += SEED_THREADS) hz[i] = make_uint4(0u, 0u, 0u, 0u);
     }
     __syncthreads();
-    if (qi >= S) return;
+    if (qi >= item_len(qry_len, b, S)) return;          // padded queries: the search reads no threshold for them
     float q[3];
     if (qsorted) {
         const float4 qv = __ldg(qsorted + (size_t)b * S + qi);
@@ -720,6 +739,7 @@ __device__ __forceinline__ f32x2 chunk_pair_dist(const float4 *cb, int chunk, in
 struct SearchArgs {
     const float4 *packed;  // [B][n_pad/2][2]
     const float *qry;      // [B][S][3]
+    const int64_t *ref_len, *qry_len;   // [B] valid refs / queries per item (ragged batches), or null: all valid
     int N, n_pad, S, k;
     int strided;           // 1: tile t holds refs t, t + n_tiles, ... (top-k); 0: natural order (ball query)
     float r2;              // ball radius^2 (fp32)
@@ -829,6 +849,7 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
     const float4 *tiles = reinterpret_cast<const float4 *>(smem);
     const uint32_t bar_base = smem_u32(smem + STAGES * TILE_BYTES);   // full[s] at +8s, empty[s] at +8(STAGES+s)
     int *issued = reinterpret_cast<int *>(smem + STAGES * TILE_BYTES + 8 * 2 * STAGES);   // tiles issued so far
+    int *item_nt = issued + 1;                    // tiles of this batch item (slot_to_ref in the drain; kept out of the registers)
     // query records [QPB] float4 {-2qx, -2qy, -2qz, filter threshold} (read by the lane filter), then
     // top-k: heap [k+1][QPB] u64 and candidate buffer [CAND_CAP][QPB] u16.   ball: list [k][QPB] u32
     float4 *qrec = reinterpret_cast<float4 *>(smem + STAGES * TILE_BYTES + BAR_BYTES);
@@ -838,9 +859,17 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
 
     const int lane = threadIdx.x & 31;
     const int b = blockIdx.y, split = blockIdx.z;
+    // Ragged items: the tile loop stops at the item's own tiles, and a CTA that holds no valid query (its lowest query,
+    // blockIdx.x * QPB or, dealt warp by warp, 32 * blockIdx.x, is past s_b) visits none.  A range without tiles of the
+    // item still writes its partial list of every row: all sentinel keys, which the merge turns into -1 / +inf.
     const int tile0 = split * P.tiles_per_split;
-    const int tile1 = min(tile0 + P.tiles_per_split, P.n_pad / TILE);
-    const int ntiles = tile1 - tile0;
+    int ntiles, s_b = item_len(P.qry_len, b, P.S);
+    {
+        const int nt_b = item_tiles(item_len(P.ref_len, b, P.N));
+        const int first_q = P.qsorted && P.interleave ? (int)blockIdx.x * 32 : (int)blockIdx.x * QPB;
+        ntiles = min(tile0 + P.tiles_per_split, first_q < s_b ? nt_b : 0) - tile0;     // <= 0: no tile
+        if (threadIdx.x == 0) *item_nt = nt_b;
+    }
     const int k = P.k;
     const char *src = reinterpret_cast<const char *>(P.packed) + ((size_t)b * P.n_pad + (size_t)tile0 * TILE) * 16;
 
@@ -869,13 +898,18 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
     };
     // Per-query state that stays in registers across the filter: tau (exact threshold) and the ball count.  Everything
     // else about a query is rebuilt from its 16-byte shared-memory record at the start of a drain.
+    // A padded query of a ragged item (qi >= s_b) is not loaded and starts from tau = -inf: nothing ever hits, its row is
+    // written from the sentinel heap (-1 / +inf), and a warp with no valid query skips the filters altogether.
     float tau[Q];
     int cnt[Q];
+    bool live_any = false;
 #pragma unroll
     for (int j = 0; j < Q; ++j) {
         const int qi = query_of(j);
+        const bool live = qi < s_b;
+        live_any = live_any || live;
         float x = 0.f, y = 0.f, z = 0.f;
-        if (qi < P.S) {
+        if (live) {
             if (P.qsorted) {
                 const float4 qv = __ldg(P.qsorted + (size_t)b * P.S + qi);
                 x = qv.x; y = qv.y; z = qv.z;
@@ -886,9 +920,9 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
         }
         cnt[j] = 0;
         if (MODE == MODE_TOPK) {
-            tau[j] = P.debug_nodrain ? -CUDART_INF_F : CUDART_INF_F;
+            tau[j] = P.debug_nodrain || !live ? -CUDART_INF_F : CUDART_INF_F;
             // warm start: an upper bound of the k-th distance from grid_seed_kernel
-            if (P.seed && !P.debug_nodrain && qi < P.S) tau[j] = __ldg(P.seed + (size_t)b * P.S + qi);
+            if (P.seed && !P.debug_nodrain && live) tau[j] = __ldg(P.seed + (size_t)b * P.S + qi);
             for (int e = 0; e < k; ++e) heap_all[e * QPB + j * NCT + ct] = HEAP_SENTINEL;
             heap_all[k * QPB + j * NCT + ct] = 0ull;   // pad: the smallest key, never selected as a child
         } else {
@@ -904,6 +938,7 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
         for (int j = 0; j < Q; ++j) cold = cold || tau[j] == CUDART_INF_F;
         warp_cold = __any_sync(FULL, cold);
     }
+    const bool warp_live = MODE == MODE_BALL || __any_sync(FULL, live_any);
     for (int t = 0; t < ntiles; ++t) {
         const int s = t % STAGES;
         mbar_wait(bar_base + 8 * s, (t / STAGES) & 1);
@@ -1052,7 +1087,7 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
                                     // the refs are not visited in index order: an EQUAL distance still wins with a lower index
                                     // than the root's (rare; only then is the root read)
                                     const uint32_t ri = P.perm ? (uint32_t)__ldg(P.perm + (size_t)b * P.n_pad + tile_ref0 + off)
-                                                               : (uint32_t)slot_to_ref(tile_ref0 + off, P.strided, P.n_pad / TILE);
+                                                               : (uint32_t)slot_to_ref(tile_ref0 + off, P.strided, *item_nt);
                                     B200PC_DEV_ASSERT(ri < (uint32_t)P.n_pad);
                                     if (d < tau[j] || ri < (uint32_t)lds_u64(hb)) {
                                         heap_sift_root<true>(hb, SB, (uint32_t)k * SB, ((unsigned long long)order_key(d) << 32) | ri);
@@ -1102,7 +1137,7 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
         uint32_t mask[Q][2];
         // the warm-up schedule of the first tile is only needed by warps that hold a query starting from tau = +inf
         const bool warm = MODE == MODE_TOPK && t == 0 && warp_cold;
-        int c = 0;
+        int c = warp_live ? 0 : CHUNKS_PER_TILE;         // a warp without a valid query only releases the stages
         if (MODE == MODE_BALL) {
             // a ball is "the first nsample refs by index": once every query of the warp has its nsample refs, no later ref
             // can change anything -- the warp only keeps releasing stages so that the other warps' tiles keep coming
@@ -1140,6 +1175,7 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
     }
 
     // ---------------- results ----------------
+    s_b = item_len(P.qry_len, b, P.S);
 #pragma unroll
     for (int j = 0; j < Q; ++j) {
         const int qi = query_of(j);
@@ -1155,8 +1191,9 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
             }
         }
         if (qi >= P.S) continue;
-        // cell-ordered queries: the result goes to the caller's row
-        const size_t row = (size_t)b * P.S + (P.qsorted ? __float_as_int(__ldg(&P.qsorted[(size_t)b * P.S + qi].w)) : qi);
+        // cell-ordered queries: the result goes to the caller's row.  Only the s_b valid queries are in the sorted copy, so
+        // the sorted positions s_b .. S-1 are free and take the padded rows s_b .. S-1 one to one.
+        const size_t row = (size_t)b * P.S + (P.qsorted && qi < s_b ? __float_as_int(__ldg(&P.qsorted[(size_t)b * P.S + qi].w)) : qi);
         B200PC_DEV_ASSERT(row >= (size_t)b * P.S && row < (size_t)(b + 1) * P.S);
         if (P.n_split == 1) {
             int64_t *io = P.idx_out ? P.idx_out + row * k : nullptr;
@@ -1416,14 +1453,16 @@ static int launch_shape(const SearchArgs &a, const SearchPlan &pl, int B, cudaSt
     return launch_one<FORM, MODE, 1>(a, pl, B, st);
 }
 
-static int run_search(const float *ref, const float *qry, int B, int N, int S, int k, int form, int mode, float r2,
-                      int64_t *idx, int32_t *idx32, float *dist, void *ws, size_t ws_bytes, cudaStream_t st) {
+// ref_len / qry_len: [B] device lengths of a ragged batch (top-k only), or null.  The plan and the workspace are those of
+// the padded shape.
+static int run_search(const float *ref, const float *qry, const int64_t *ref_len, const int64_t *qry_len, int B, int N, int S, int k,
+                      int form, int mode, float r2, int64_t *idx, int32_t *idx32, float *dist, void *ws, size_t ws_bytes, cudaStream_t st) {
     B200PC_REQUIRE(B >= 0 && N >= 1 && S >= 0 && k >= 1, "search: bad sizes B=%d N=%d S=%d k=%d", B, N, S, k);
     if (B == 0 || S == 0) return B200PC_OK;             // empty work: nothing to validate, empty tensors have null pointers
     B200PC_REQUIRE(ref && qry, "search: null input pointer");
     B200PC_REQUIRE(idx || idx32 || dist, "search: no output requested");
     if (!idx32) {   // small reference sets: warp-per-query kernel, one launch, no workspace (small_search.cu)
-        const int rc_small = run_small(ref, qry, B, N, S, k, form, mode, r2, idx, dist, st);
+        const int rc_small = run_small(ref, qry, ref_len, qry_len, B, N, S, k, form, mode, r2, idx, dist, st);
         if (rc_small != -100) return rc_small;
     }
     SearchPlan pl;
@@ -1452,34 +1491,34 @@ static int run_search(const float *ref, const float *qry, int B, int N, int S, i
         const size_t zero_bytes = pl.grid_sorted ? reinterpret_cast<char *>(gb.cend) - reinterpret_cast<char *>(gb.counts)
                                                  : (size_t)B * GRID_STRIDE * sizeof(unsigned);
         B200PC_CUDA(cudaMemsetAsync(gb.counts, 0, zero_bytes, st));
-        grid_bbox_kernel<<<B, 1024, 0, st>>>(ref, N, gb.desc);
+        grid_bbox_kernel<<<B, 1024, 0, st>>>(ref, ref_len, N, gb.desc);
         B200PC_LAUNCH_CHECK();
     }
     if (pl.grid_bytes && pl.grid_sorted) {
         // count -> pyramid + segment sums -> scan -> scatter (sorted copies, packed tiles, slot table) -> starting thresholds
-        grid_count_kernel<<<dim3((N + S + 255) / 256, B), 256, 0, st>>>(ref, N, qry, S, gb.desc, gb.counts, gb.qcend);
+        grid_count_kernel<<<dim3((N + S + 255) / 256, B), 256, 0, st>>>(ref, ref_len, N, qry, qry_len, S, gb.desc, gb.counts, gb.qcend);
         B200PC_LAUNCH_CHECK();
         grid_pyramid_kernel<<<dim3(GRID_SEGS, B, 2), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.qcend, gb.qseg);
         B200PC_LAUNCH_CHECK();
         grid_scan_kernel<<<dim3(GRID_SEGS, B, 2), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.cend, gb.qcend, gb.qseg);
         B200PC_LAUNCH_CHECK();
-        grid_scatter_kernel<<<dim3((pl.n_pad + S + 255) / 256, B), 256, 0, st>>>(ref, N, pl.n_pad, pl.tiles_per_split, qry, S, gb.desc, gb, packed,
-                                                                                  tn.seed > 0 ? 0 : k);
+        grid_scatter_kernel<<<dim3((pl.n_pad + S + 255) / 256, B), 256, 0, st>>>(ref, ref_len, N, pl.n_pad, pl.tiles_per_split, qry, qry_len, S,
+                                                                                  gb.desc, gb, packed, tn.seed > 0 ? 0 : k);
         B200PC_LAUNCH_CHECK();
         if (tn.seed > 0) {                               // thresholds from the refs inside the boxes (A/B: B200PC_SEED=n); else the scatter wrote them
-            grid_seed_kernel<<<dim3((S + SEED_THREADS - 1) / SEED_THREADS, B), SEED_THREADS, 0, st>>>(gb.qsorted, nullptr, S, N, k, gb.desc, gb.counts,
+            grid_seed_kernel<<<dim3((S + SEED_THREADS - 1) / SEED_THREADS, B), SEED_THREADS, 0, st>>>(gb.qsorted, nullptr, qry_len, S, N, k, gb.desc, gb.counts,
                                                                                                 gb.cend, gb.sorted, gb.seed, tn.seed);
             B200PC_LAUNCH_CHECK();
         }
         strided_eff = 0;                                  // the slot order is sorted_slot's
     } else {
         dim3 grid((pl.n_pad / 2 + 255) / 256, B);
-        pack_refs_kernel<<<grid, 256, 0, st>>>(ref, N, pl.n_pad, strided, packed, pl.grid_bytes ? gb.desc : nullptr, gb.counts);
+        pack_refs_kernel<<<grid, 256, 0, st>>>(ref, ref_len, N, pl.n_pad, strided, packed, pl.grid_bytes ? gb.desc : nullptr, gb.counts);
         B200PC_LAUNCH_CHECK();
         if (pl.grid_bytes) {                              // thresholds only: the caller's order of refs and queries stays
             grid_pyramid_kernel<<<dim3(GRID_SEGS, B, 1), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.qcend, gb.qseg);
             B200PC_LAUNCH_CHECK();
-            grid_seed_kernel<<<dim3((S + SEED_THREADS - 1) / SEED_THREADS, B), SEED_THREADS, 0, st>>>(nullptr, qry, S, N, k, gb.desc, gb.counts, gb.cend,
+            grid_seed_kernel<<<dim3((S + SEED_THREADS - 1) / SEED_THREADS, B), SEED_THREADS, 0, st>>>(nullptr, qry, qry_len, S, N, k, gb.desc, gb.counts, gb.cend,
                                                                                                 gb.sorted, gb.seed, 0);
             B200PC_LAUNCH_CHECK();
             gb.qsorted = nullptr; gb.perm = nullptr;
@@ -1487,7 +1526,7 @@ static int run_search(const float *ref, const float *qry, int B, int N, int S, i
     }
 
     SearchArgs a;
-    a.packed = packed; a.strided = strided_eff; a.qry = qry; a.N = N; a.n_pad = pl.n_pad; a.S = S; a.k = k; a.r2 = r2;
+    a.packed = packed; a.strided = strided_eff; a.qry = qry; a.ref_len = ref_len; a.qry_len = qry_len; a.N = N; a.n_pad = pl.n_pad; a.S = S; a.k = k; a.r2 = r2;
     a.n_split = pl.n_split; a.tiles_per_split = pl.tiles_per_split;
     a.debug_nodrain = tn.nodrain;
     a.lane_filter = tn.filter >= 0 ? tn.filter != 0 : 1;                          // 0: A/B measurement only
@@ -1524,23 +1563,23 @@ static int run_search(const float *ref, const float *qry, int B, int N, int S, i
 }
 
 int run_topk(const float *ref, const float *qry, int B, int N, int S, int k, int form, int64_t *idx, float *dist,
-             void *ws, size_t ws_bytes, cudaStream_t st) {
+             void *ws, size_t ws_bytes, cudaStream_t st, const int64_t *ref_len, const int64_t *qry_len) {
     B200PC_REQUIRE(form >= 0 && form <= 2, "knn: unknown distance form %d", form);
     B200PC_REQUIRE(k <= N, "knn: k=%d exceeds the number of reference points N=%d", k, N);
-    return run_search(ref, qry, B, N, S, k, form, MODE_TOPK, 0.f, idx, nullptr, dist, ws, ws_bytes, st);
+    return run_search(ref, qry, ref_len, qry_len, B, N, S, k, form, MODE_TOPK, 0.f, idx, nullptr, dist, ws, ws_bytes, st);
 }
 
 int run_topk_i32(const float *ref, const float *qry, int B, int N, int S, int k, int form, int32_t *idx32, float *dist,
                  void *ws, size_t ws_bytes, cudaStream_t st) {
     B200PC_REQUIRE(form >= 0 && form <= 2, "knn: unknown distance form %d", form);
     B200PC_REQUIRE(k <= N, "knn: k=%d exceeds the number of reference points N=%d", k, N);
-    return run_search(ref, qry, B, N, S, k, form, MODE_TOPK, 0.f, nullptr, idx32, dist, ws, ws_bytes, st);
+    return run_search(ref, qry, nullptr, nullptr, B, N, S, k, form, MODE_TOPK, 0.f, nullptr, idx32, dist, ws, ws_bytes, st);
 }
 
 int run_ball(const float *ref, const float *qry, int B, int N, int S, float r2, int nsample, int64_t *idx,
              void *ws, size_t ws_bytes, cudaStream_t st) {
     B200PC_REQUIRE(idx || B == 0 || S == 0, "ball_query: null output pointer");
-    return run_search(ref, qry, B, N, S, nsample, B200PC_FORM_QRY_NORM_FIRST, MODE_BALL, r2, idx, nullptr, nullptr, ws,
+    return run_search(ref, qry, nullptr, nullptr, B, N, S, nsample, B200PC_FORM_QRY_NORM_FIRST, MODE_BALL, r2, idx, nullptr, nullptr, ws,
                       ws_bytes, st);
 }
 
@@ -1563,6 +1602,12 @@ extern "C" size_t b200pc_search_workspace_bytes(int B, int N, int S, int k) {
 extern "C" int b200pc_knn(const float *ref, const float *qry, int B, int N, int S, int k, int form, int64_t *idx,
                           float *dist, void *workspace, size_t workspace_bytes, b200pc_stream_t stream) {
     return run_topk(ref, qry, B, N, S, k, form, idx, dist, workspace, workspace_bytes, as_stream(stream));
+}
+
+extern "C" int b200pc_knn_ragged(const float *ref, const float *qry, const int64_t *ref_len, const int64_t *qry_len, int B, int N,
+                                 int S, int k, int form, int64_t *idx, float *dist, void *workspace, size_t workspace_bytes,
+                                 b200pc_stream_t stream) {
+    return run_topk(ref, qry, B, N, S, k, form, idx, dist, workspace, workspace_bytes, as_stream(stream), ref_len, qry_len);
 }
 
 extern "C" int b200pc_knn_i32(const float *ref, const float *qry, int B, int N, int S, int k, int form, int32_t *idx,

@@ -6,6 +6,14 @@ namespace b200pc {
 
 enum SearchMode { MODE_TOPK = 0, MODE_BALL = 1 };
 
+// Ragged batches (b200pc_knn_ragged, b200pc_chamfer_ragged_*): item b has clamp(len[b], 0, full) valid points; a null
+// length array means every item is full.  The clamp happens here, on the device: nothing is read back to the host.
+__device__ __forceinline__ int item_len(const int64_t *len, int b, int full) {
+    if (!len) return full;
+    const int64_t v = __ldg(len + b);
+    return v < 0 ? 0 : (v > (int64_t)full ? full : (int)v);
+}
+
 // Geometry of one search launch, derived deterministically from the problem size so that the
 // workspace-size query and the launcher always agree.
 struct SearchPlan {
@@ -27,15 +35,16 @@ struct SearchPlan {
 // k: list length (k for top-k, nsample for ball).  Returns false if k cannot be served.
 bool plan_search(int B, int N, int S, int k, int mode, SearchPlan *plan);
 
-// Top-k search: idx [B,S,k] int64 and/or dist [B,S,k] (either may be null, not both).
+// Top-k search: idx [B,S,k] int64 and/or dist [B,S,k] (either may be null, not both).  ref_len / qry_len: [B] device
+// lengths of a ragged batch (b200pc_knn_ragged), null = every item full.
 int run_topk(const float *ref, const float *qry, int B, int N, int S, int k, int form, int64_t *idx, float *dist,
-             void *ws, size_t ws_bytes, cudaStream_t st);
+             void *ws, size_t ws_bytes, cudaStream_t st, const int64_t *ref_len = nullptr, const int64_t *qry_len = nullptr);
 
 int run_ball(const float *ref, const float *qry, int B, int N, int S, float r2, int nsample, int64_t *idx,
              void *ws, size_t ws_bytes, cudaStream_t st);
 
 // warp-per-query path for N <= 1024 (small_search.cu); returns -100 when it declines the problem
-int run_small(const float *ref, const float *qry, int B, int N, int S, int k, int form, int mode, float r2, int64_t *idx,
-              float *dist, cudaStream_t st);
+int run_small(const float *ref, const float *qry, const int64_t *ref_len, const int64_t *qry_len, int B, int N, int S, int k, int form,
+              int mode, float r2, int64_t *idx, float *dist, cudaStream_t st);
 
 }  // namespace b200pc

@@ -43,22 +43,34 @@ __device__ __forceinline__ float dist_scalar(float rx, float ry, float rz, float
 }
 
 // NI = refs per lane (N <= 32*NI)
+// ref_len / qry_len (top-k only): ragged batch lengths or null.  Refs i >= n_b are never read and never candidates; rows
+// q >= s_b are written as -1 / +inf without a search.
 template <int FORM, int MODE, int NI>
 __global__ void __launch_bounds__(SMALL_WARPS * 32) small_search_kernel(const float *__restrict__ ref, const float *__restrict__ qry,
+                                                                        const int64_t *__restrict__ ref_len, const int64_t *__restrict__ qry_len,
                                                                         int N, int S, int k, float r2, int64_t *__restrict__ idx_out,
                                                                         float *__restrict__ dist_out) {
     __shared__ float sx[SMALL_MAX_N], sy[SMALL_MAX_N], sz[SMALL_MAX_N], sn[SMALL_MAX_N];
     const int b = blockIdx.y;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int n_b = item_len(ref_len, b, N), s_b = item_len(qry_len, b, S);
     const float *rb = ref + (size_t)b * N * 3;
     for (int i = threadIdx.x; i < 32 * NI; i += blockDim.x) {
         float x = 0.f, y = 0.f, z = 0.f;
-        if (i < N) { x = rb[i * 3]; y = rb[i * 3 + 1]; z = rb[i * 3 + 2]; }
+        if (i < n_b) { x = rb[i * 3]; y = rb[i * 3 + 1]; z = rb[i * 3 + 2]; }
         sx[i] = x; sy[i] = y; sz[i] = z;
         sn[i] = FORM == B200PC_FORM_DIRECT ? 0.f : sq_norm_torch(x, y, z);
     }
     __syncthreads();
     for (int q = blockIdx.x * SMALL_WARPS + warp; q < S; q += gridDim.x * SMALL_WARPS) {
+        if (MODE == MODE_TOPK && q >= s_b) {
+            const size_t row = (size_t)b * S + q;
+            for (int e = lane; e < k; e += 32) {
+                if (idx_out) idx_out[row * k + e] = -1;
+                if (dist_out) dist_out[row * k + e] = CUDART_INF_F;
+            }
+            continue;
+        }
         const float *qp = qry + ((size_t)b * S + q) * 3;
         const float qx = qp[0], qy = qp[1], qz = qp[2];
         const float qn = FORM == B200PC_FORM_DIRECT ? 0.f : sq_norm_torch(qx, qy, qz);
@@ -88,7 +100,7 @@ __global__ void __launch_bounds__(SMALL_WARPS * 32) small_search_kernel(const fl
                 const int r = i * 32 + lane;
                 const float d = dist_scalar<FORM>(sx[r], sy[r], sz[r], sn[r], qx, qy, qz, qn);
                 // only a finite distance is a candidate (NaN and +inf get the empty key; no form yields -inf)
-                key[i] = r < N && d < CUDART_INF_F ? (((unsigned long long)okey(d) << 32) | (unsigned)r) : ~0ull;
+                key[i] = r < n_b && d < CUDART_INF_F ? (((unsigned long long)okey(d) << 32) | (unsigned)r) : ~0ull;
             }
             unsigned long long best = ~0ull;
 #pragma unroll
@@ -117,14 +129,14 @@ __global__ void __launch_bounds__(SMALL_WARPS * 32) small_search_kernel(const fl
 }
 
 template <int FORM, int MODE>
-static int launch_small(const float *ref, const float *qry, int B, int N, int S, int k, float r2, int64_t *idx, float *dist,
-                        cudaStream_t st) {
+static int launch_small(const float *ref, const float *qry, const int64_t *ref_len, const int64_t *qry_len, int B, int N, int S, int k,
+                        float r2, int64_t *idx, float *dist, cudaStream_t st) {
     const int ni = (N + 31) / 32;
     int blocks = (S + SMALL_WARPS - 1) / SMALL_WARPS;
     const int cap = sm_count() * 8;
     if (blocks > cap) blocks = cap;
     dim3 grid(blocks, B);
-#define B200PC_SMALL(NI_) small_search_kernel<FORM, MODE, NI_><<<grid, SMALL_WARPS * 32, 0, st>>>(ref, qry, N, S, k, r2, idx, dist)
+#define B200PC_SMALL(NI_) small_search_kernel<FORM, MODE, NI_><<<grid, SMALL_WARPS * 32, 0, st>>>(ref, qry, ref_len, qry_len, N, S, k, r2, idx, dist)
     if (ni <= 1) B200PC_SMALL(1);
     else if (ni <= 2) B200PC_SMALL(2);
     else if (ni <= 4) B200PC_SMALL(4);
@@ -137,8 +149,8 @@ static int launch_small(const float *ref, const float *qry, int B, int N, int S,
 }
 
 // decides whether the warp-per-query path serves this problem; returns -100 if not (caller streams instead)
-int run_small(const float *ref, const float *qry, int B, int N, int S, int k, int form, int mode, float r2, int64_t *idx,
-              float *dist, cudaStream_t st) {
+int run_small(const float *ref, const float *qry, const int64_t *ref_len, const int64_t *qry_len, int B, int N, int S, int k, int form,
+              int mode, float r2, int64_t *idx, float *dist, cudaStream_t st) {
     if (N > SMALL_MAX_N) return -100;
     const int forced = tuning().small_path;             // cached knob (-1: decide by size)
     if (forced >= 0) { if (forced == 0) return -100; }
@@ -148,10 +160,12 @@ int run_small(const float *ref, const float *qry, int B, int N, int S, int k, in
         const long queries = (long)B * S;
         if (!(queries <= 4096 || (mode == MODE_TOPK && k * 4 >= N))) return -100;
     }
-    if (mode == MODE_BALL) return launch_small<B200PC_FORM_QRY_NORM_FIRST, MODE_BALL>(ref, qry, B, N, S, k, r2, idx, nullptr, st);
-    if (form == B200PC_FORM_REF_NORM_FIRST) return launch_small<B200PC_FORM_REF_NORM_FIRST, MODE_TOPK>(ref, qry, B, N, S, k, 0.f, idx, dist, st);
-    if (form == B200PC_FORM_QRY_NORM_FIRST) return launch_small<B200PC_FORM_QRY_NORM_FIRST, MODE_TOPK>(ref, qry, B, N, S, k, 0.f, idx, dist, st);
-    return launch_small<B200PC_FORM_DIRECT, MODE_TOPK>(ref, qry, B, N, S, k, 0.f, idx, dist, st);
+    if (mode == MODE_BALL) return launch_small<B200PC_FORM_QRY_NORM_FIRST, MODE_BALL>(ref, qry, nullptr, nullptr, B, N, S, k, r2, idx, nullptr, st);
+    if (form == B200PC_FORM_REF_NORM_FIRST)
+        return launch_small<B200PC_FORM_REF_NORM_FIRST, MODE_TOPK>(ref, qry, ref_len, qry_len, B, N, S, k, 0.f, idx, dist, st);
+    if (form == B200PC_FORM_QRY_NORM_FIRST)
+        return launch_small<B200PC_FORM_QRY_NORM_FIRST, MODE_TOPK>(ref, qry, ref_len, qry_len, B, N, S, k, 0.f, idx, dist, st);
+    return launch_small<B200PC_FORM_DIRECT, MODE_TOPK>(ref, qry, ref_len, qry_len, B, N, S, k, 0.f, idx, dist, st);
 }
 
 }  // namespace b200pc
