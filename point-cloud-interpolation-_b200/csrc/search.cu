@@ -159,13 +159,15 @@ struct GridBufs {
     GridDesc *desc;          // [B]
     unsigned *counts;        // [B][GRID_STRIDE]     refs per cell, all levels
     unsigned *qcend;         // [B][GRID_MAX_CELLS]  queries per level-0 cell, then (in place) the running end of each cell's range
-    unsigned *tail;          // [B]                  non-finite refs placed so far (they go behind the finite ones)
+    unsigned *tail;          // [B + 1]              non-finite refs placed so far (they go behind the finite ones); then the
+                             //                      work counter of the pruned search (query groups dealt so far)
     unsigned *cend;          // [B][GRID_MAX_CELLS]  refs: start, then end of each level-0 cell's range in the sorted order
     unsigned *seg, *qseg;    // [B][GRID_SEGS]       counts per 1024-cell segment (refs, queries)
     float4 *sorted;          // [B][N]   refs in cell order {x, y, z, index}
     float4 *qsorted;         // [B][S]   queries in cell order {x, y, z, index}
     int *perm;               // [B][n_pad]  sorted slot -> ref index
     float *seed;             // [B][S]   starting thresholds, in the sorted query order
+    float4 *blocks;          // [B][n_pad / 64][2]  pruned search: {lo, max |r|^2}, {hi, 0} of every 64-ref block (grid_block_kernel)
 };
 static size_t grid_layout(int B, int N, int S, int n_pad, char *base, GridBufs *g) {
     size_t o = 0;
@@ -173,7 +175,7 @@ static size_t grid_layout(int B, int N, int S, int n_pad, char *base, GridBufs *
     GridDesc *desc = reinterpret_cast<GridDesc *>(take((size_t)B * sizeof(GridDesc)));
     unsigned *counts = reinterpret_cast<unsigned *>(take((size_t)B * GRID_STRIDE * sizeof(unsigned)));
     unsigned *qcend = reinterpret_cast<unsigned *>(take((size_t)B * GRID_MAX_CELLS * sizeof(unsigned)));
-    unsigned *tail = reinterpret_cast<unsigned *>(take((size_t)B * sizeof(unsigned)));
+    unsigned *tail = reinterpret_cast<unsigned *>(take((size_t)(B + 1) * sizeof(unsigned)));
     unsigned *cend = reinterpret_cast<unsigned *>(take((size_t)B * GRID_MAX_CELLS * sizeof(unsigned)));
     unsigned *seg = reinterpret_cast<unsigned *>(take((size_t)B * GRID_SEGS * sizeof(unsigned)));
     unsigned *qseg = reinterpret_cast<unsigned *>(take((size_t)B * GRID_SEGS * sizeof(unsigned)));
@@ -181,7 +183,8 @@ static size_t grid_layout(int B, int N, int S, int n_pad, char *base, GridBufs *
     float4 *qsorted = reinterpret_cast<float4 *>(take((size_t)B * S * sizeof(float4)));
     int *perm = reinterpret_cast<int *>(take((size_t)B * n_pad * sizeof(int)));
     float *seed = reinterpret_cast<float *>(take((size_t)B * S * sizeof(float)));
-    if (g) *g = GridBufs{desc, counts, qcend, tail, cend, seg, qseg, sorted, qsorted, perm, seed};
+    float4 *blocks = reinterpret_cast<float4 *>(take((size_t)B * (n_pad / 64) * 2 * sizeof(float4)));
+    if (g) *g = GridBufs{desc, counts, qcend, tail, cend, seg, qseg, sorted, qsorted, perm, seed, blocks};
     return o;
 }
 
@@ -289,6 +292,29 @@ __device__ __forceinline__ void grid_count_ref(const GridDesc *desc, unsigned *c
     if (isfinite(x) && isfinite(y) && isfinite(z)) atomicAdd(counts + (size_t)b * GRID_STRIDE + grid_cell_index(desc[b], x, y, z), 1u);
 }
 
+// Brick order of the level-0 cells (the pruned search, grid_mode 3): the grid is cut into 4 x 4 x 4-cell bricks (the last
+// brick along an axis may be thinner), bricks in raster order, cells in raster order inside their brick.  Rank r of that
+// order -> raster cell index; a bijection of [0, cells), so the counters stay indexed by raster cell.  64 consecutive
+// refs of this order sit in a few neighbouring bricks: compact boxes, which is what the block table of the pruned search
+// needs (raster order cuts a 64-ref run into thin slabs of one x-row; host simulation, tools/prune_sim.py).
+constexpr int BRICK = 4;
+__device__ __forceinline__ int brick_cell(const GridDesc &g, int r) {
+    const int gx = g.dim[0][0], gy = g.dim[0][1], gz = g.dim[0][2];
+    const int bz = r / (BRICK * gx * gy);
+    r -= bz * BRICK * gx * gy;
+    const int d = min(BRICK, gz - BRICK * bz);          // depth of this slab of bricks
+    const int by = r / (BRICK * gx * d);
+    r -= by * BRICK * gx * d;
+    const int h = min(BRICK, gy - BRICK * by);          // height of this row of bricks
+    const int bx = r / (BRICK * h * d);
+    r -= bx * BRICK * h * d;
+    const int w = min(BRICK, gx - BRICK * bx);          // width of this brick
+    const int lz = r / (h * w);
+    r -= lz * h * w;
+    const int ly = r / w, lx = r - ly * w;
+    return ((BRICK * bz + lz) * gy + BRICK * by + ly) * gx + BRICK * bx + lx;
+}
+
 // one atomic per point: refs (finite ones) into counts, queries (clamped into the border cells; NaN -> cell 0) into qcend.
 // Padded refs and queries of a ragged item are not counted.
 __global__ void __launch_bounds__(256) grid_count_kernel(const float *__restrict__ ref, const int64_t *__restrict__ ref_len, int N,
@@ -311,10 +337,11 @@ __global__ void __launch_bounds__(256) grid_count_kernel(const float *__restrict
 // blockIdx.z = 0: the coarser levels of the ref counts -- every occupied level-0 cell adds its count to its ancestors (a
 // few thousand atomics per cloud; counting all five levels per ref tripled the counting kernel's time: the coarse cells
 // contend).  Block x owns the cells [1024 x, 1024 x + 1024) and leaves their total in seg[b][x] for grid_scan_kernel.
-// blockIdx.z = 1: only the segment totals, of the query counts.
+// blockIdx.z = 1: only the segment totals, of the query counts.  brick = 1: the segments are 1024 consecutive ranks of the
+// brick order (brick_cell), the order grid_scan_kernel then scans in.
 __global__ void __launch_bounds__(256) grid_pyramid_kernel(const GridDesc *__restrict__ desc, unsigned *__restrict__ counts,
                                                            unsigned *__restrict__ seg, const unsigned *__restrict__ qcend,
-                                                           unsigned *__restrict__ qseg) {
+                                                           unsigned *__restrict__ qseg, int brick) {
     const int b = blockIdx.y;
     const bool refs = blockIdx.z == 0;
     const GridDesc &g = desc[b];
@@ -324,8 +351,10 @@ __global__ void __launch_bounds__(256) grid_pyramid_kernel(const GridDesc *__res
     unsigned sum = 0;
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-        const int c = blockIdx.x * 1024 + i * 256 + threadIdx.x;
-        const unsigned n = c < cells ? src[c] : 0u;
+        const int r = blockIdx.x * 1024 + i * 256 + threadIdx.x;
+        const int c = brick && r < cells ? brick_cell(g, r) : r;
+        B200PC_DEV_ASSERT(r >= cells || (c >= 0 && c < cells));
+        const unsigned n = r < cells ? src[c] : 0u;
         sum += n;
         if (n == 0 || !refs) continue;
         const int cx = c % g.dim[0][0], cy = (c / g.dim[0][0]) % g.dim[0][1], cz = c / (g.dim[0][0] * g.dim[0][1]);
@@ -349,9 +378,10 @@ __global__ void __launch_bounds__(256) grid_pyramid_kernel(const GridDesc *__res
 
 // counts -> start offsets (exclusive scan in the linear cell order): cend[c] = points in cells < c.  The scatter below then
 // advances cend[c] to the END of cell c (= start of cell c + 1).  z = 0: refs (counts -> cend), z = 1: queries (in place).
+// brick = 1: the scan runs over the ranks of the brick order instead (cend[c] = points in the cells that precede c in it).
 __global__ void __launch_bounds__(256) grid_scan_kernel(const GridDesc *__restrict__ desc, const unsigned *__restrict__ counts,
                                                         const unsigned *__restrict__ seg, unsigned *__restrict__ cend,
-                                                        unsigned *__restrict__ qcend, const unsigned *__restrict__ qseg) {
+                                                        unsigned *__restrict__ qcend, const unsigned *__restrict__ qseg, int brick) {
     const int b = blockIdx.y, x = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const bool refs = blockIdx.z == 0;
     const GridDesc &g = desc[b];
@@ -368,11 +398,20 @@ __global__ void __launch_bounds__(256) grid_scan_kernel(const GridDesc *__restri
         if (lane == 0) sh[8] = v;
     }
     const int c0 = x * 1024 + 4 * threadIdx.x;
-    uint4 v = *reinterpret_cast<const uint4 *>(in + c0);    // refs: may run into level 1, masked below
-    if (c0 + 0 >= cells) v.x = 0;
-    if (c0 + 1 >= cells) v.y = 0;
-    if (c0 + 2 >= cells) v.z = 0;
-    if (c0 + 3 >= cells) v.w = 0;
+    uint4 v;
+    int bc[4];                                             // brick order: the raster cells of ranks c0 .. c0 + 3
+    if (brick) {
+#pragma unroll
+        for (int u = 0; u < 4; ++u) bc[u] = c0 + u < cells ? brick_cell(g, c0 + u) : -1;
+        v.x = bc[0] >= 0 ? in[bc[0]] : 0u; v.y = bc[1] >= 0 ? in[bc[1]] : 0u;
+        v.z = bc[2] >= 0 ? in[bc[2]] : 0u; v.w = bc[3] >= 0 ? in[bc[3]] : 0u;
+    } else {
+        v = *reinterpret_cast<const uint4 *>(in + c0);     // refs: may run into level 1, masked below
+        if (c0 + 0 >= cells) v.x = 0;
+        if (c0 + 1 >= cells) v.y = 0;
+        if (c0 + 2 >= cells) v.z = 0;
+        if (c0 + 3 >= cells) v.w = 0;
+    }
     const unsigned mine = v.x + v.y + v.z + v.w;
     unsigned inc = mine;                                   // inclusive scan over the warp, then over the 8 warps
 #pragma unroll
@@ -387,7 +426,14 @@ __global__ void __launch_bounds__(256) grid_scan_kernel(const GridDesc *__restri
     uint4 o4;
     o4.x = start; o4.y = o4.x + v.x; o4.z = o4.y + v.y; o4.w = o4.z + v.z;
     B200PC_DEV_ASSERT(c0 + 3 < GRID_MAX_CELLS);
-    *reinterpret_cast<uint4 *>(out + c0) = o4;
+    if (brick) {       // every cell belongs to one thread, so the in-place query scan reads all its cells before any write
+        if (bc[0] >= 0) out[bc[0]] = o4.x;
+        if (bc[1] >= 0) out[bc[1]] = o4.y;
+        if (bc[2] >= 0) out[bc[2]] = o4.z;
+        if (bc[3] >= 0) out[bc[3]] = o4.w;
+    } else {
+        *reinterpret_cast<uint4 *>(out + c0) = o4;
+    }
 }
 
 // Move every point to its cell's range.  Refs: the sorted copy {x, y, z, index} for the seeds, the packed tile records of
@@ -520,6 +566,44 @@ __global__ void __launch_bounds__(256) grid_scatter_kernel(const float *__restri
             const float q[3] = {x, y, z};
             gb.seed[(size_t)b * S + pos] = grid_corner_seed(g, gb.counts + (size_t)b * GRID_STRIDE, q, k_seed);
         }
+    }
+}
+
+// Block table of the pruned search: one warp per block of PRUNE_BLOCK consecutive sorted refs (= packed slots, the slot order
+// is the sorted order there), lane l reads the l-th record pair.  The box is the min / max of the block's finite coordinates
+// (exact: no rounding), the fourth word of the first record the largest fl|r|^2 (torch_sq_norm) of them.  Only blocks below
+// n_finite are ever visited, and each of those holds at least one finite ref; the others are left alone.
+constexpr int PRUNE_BLOCK = 64;            // refs per block: 8 chunks
+__global__ void __launch_bounds__(256) grid_block_kernel(const float4 *__restrict__ packed, int n_pad, const GridDesc *__restrict__ desc,
+                                                         float4 *__restrict__ blocks) {
+    const int lane = threadIdx.x & 31, blk = (int)((blockIdx.x * blockDim.x + threadIdx.x) >> 5), b = blockIdx.y;
+    if (blk >= (desc[b].n_finite + PRUNE_BLOCK - 1) / PRUNE_BLOCK) return;
+    const float4 *rec = packed + (size_t)b * n_pad + (size_t)blk * PRUNE_BLOCK + 2 * lane;
+    const float4 A = rec[0], Bv = rec[1];      // {x0, x1, y0, y1}, {z0, z1, w0, w1}
+    float lo[3] = {CUDART_INF_F, CUDART_INF_F, CUDART_INF_F}, hi[3] = {-CUDART_INF_F, -CUDART_INF_F, -CUDART_INF_F}, mw = 0.0f;
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const float x = h ? A.y : A.x, y = h ? A.w : A.z, z = h ? Bv.y : Bv.x;
+        if (isfinite(x) && isfinite(y) && isfinite(z)) {
+            lo[0] = fminf(lo[0], x); hi[0] = fmaxf(hi[0], x);
+            lo[1] = fminf(lo[1], y); hi[1] = fmaxf(hi[1], y);
+            lo[2] = fminf(lo[2], z); hi[2] = fmaxf(hi[2], z);
+            mw = fmaxf(mw, torch_sq_norm(x, y, z));
+        }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int a = 0; a < 3; ++a) {
+            lo[a] = fminf(lo[a], __shfl_xor_sync(0xffffffffu, lo[a], o));
+            hi[a] = fmaxf(hi[a], __shfl_xor_sync(0xffffffffu, hi[a], o));
+        }
+        mw = fmaxf(mw, __shfl_xor_sync(0xffffffffu, mw, o));
+    }
+    if (lane == 0) {
+        float4 *t = blocks + ((size_t)b * (n_pad / PRUNE_BLOCK) + blk) * 2;
+        t[0] = make_float4(lo[0], lo[1], lo[2], mw);
+        t[1] = make_float4(hi[0], hi[1], hi[2], 0.0f);
     }
 }
 
@@ -751,6 +835,13 @@ struct SearchArgs {
     const float *seed;     // [B][S]
     const int *perm;       // [B][n_pad]
     int interleave;        // cell-ordered queries dealt to the CTAs warp by warp (1) or in contiguous blocks (0)
+    // pruned search (section 3b): block table, grid descriptors, cell ends of the sorted refs, work counter, smem per warp
+    int B;
+    const float4 *blocks;
+    const GridDesc *desc;
+    const unsigned *cend;
+    unsigned *work;
+    int warp_bytes;
     int64_t *idx_out;      // [B][S][k]   (n_split == 1)
     int32_t *idx32_out;    // same rows as 32-bit indices (host-buffer callers: halves the read-back); either may be null
     float *dist_out;       // [B][S][k] or null
@@ -1233,6 +1324,282 @@ __global__ void __launch_bounds__(Q == 1 ? MAX_WARPS_Q1 * 32 : MAX_WARPS * 32, Q
 }
 
 // ---------------------------------------------------------------------------------------------
+// 3b. the pruned search (grid_mode 3): per warp, only the ref blocks that can hold a neighbour
+// ---------------------------------------------------------------------------------------------
+// Refs and queries are sorted in brick order (brick_cell), and every run of 64 sorted refs is a block with a box and a norm
+// bound (grid_block_kernel).  A warp owns 32 consecutive sorted queries -- a compact patch of space -- and walks the blocks of
+// its item outwards from the block that holds its own cell (home, home + 1, home - 1, home + 2, ...: near blocks first, so
+// that tau tightens early).  Blocks are tested 32 at a time when the walk enters their window (lane = block, the warp's
+// queries broadcast), and each block that passed is tested again when it is reached, against the lanes' CURRENT thresholds;
+// a block that some lane may need joins the batch, and every PRUNE_BATCH blocks (32 chunks, 4 KB) are copied into the warp's own
+// shared-memory buffer and go through the same lane filter and drain as a tile of search_kernel.  The visiting order and
+// the pruning change which refs are looked at, never the keys: results are bit-identical to the brute-force search.
+//
+// The bound.  Claim: if dist_ref(q, r) <= tau for some ref r of the block (dist_ref: the reference's rounded distance in any
+// of the three forms), then LB <= tau, where
+//     LB = fl(fl(G (1 - 2^-19)) - fl(1.2e-6 fl(nq + W) + 1e-37)),  G = fl(gz^2 + fl(gy^2 + fl(gx^2)))  (two FMAs),
+//     g_a = max(fl(lo_a - q_a), fl(q_a - hi_a), 0),  W = the block's largest fl|r|^2,  nq = fl|q|^2,  eps = 2^-24.
+//   * [lo, hi] holds every finite coordinate of the block exactly, so the real box distance B = sum (max(lo - q, q - hi, 0))^2
+//     is <= D = |q - r|^2 (real).  Each rounding above raises a positive value by at most a factor (1 + eps), so
+//     G <= B (1 + eps)^5 <= D (1 + 5.01 eps) (plus < 1e-44 from products that underflow).
+//   * direct form: 5 roundings of positive terms, dist_ref >= D (1 - 5.01 eps).
+//   * expanded forms: filter_threshold bounds |dist_ref - (U + nq)| by 5.01 eps (M + nq) with M <= |q|^2 + 2.01 |r|^2, and
+//     U + nq differs from D by the roundings of the two norms, <= 3.01 eps (|q|^2 + |r|^2): |dist_ref - D| <= 13.1 eps
+//     (|q|^2 + |r|^2) <= 13.2 eps (nq + W).
+//   so dist_ref >= G (1 - 10.03 eps) - 13.2 eps (nq + W) - 1e-44 for every finite ref of the block, in every form.
+//   * computed: fl(G (1 - 32 eps)) <= G (1 - 31 eps); the subtrahend is >= 20.1 eps (1 - eps)^2 (nq + W) + 1e-37; the final
+//     subtraction adds at most eps (G + subtrahend).  LB <= G (1 - 30 eps) - 19.9 eps (nq + W) - 1e-37 < that lower bound.
+//   A block is visited iff !(LB > tau): a NaN or infinite LB or tau (huge coordinates, W or nq = inf, tau = +inf before k
+//   refs are known) visits it.  G >= 2^126 visits too: the analysis above assumes no overflow.  tau only decreases, so a
+//   block skipped now holds no ref that could enter later; and tau never drops below the k-th smallest key's distance, so
+//   an equal distance with a lower index is still visited (the test is <=).  An item with fewer than k finite refs keeps
+//   tau = +inf and visits every block: the brute-force search.  A non-finite query has no finite distance to anything (its
+//   row is -1 / +inf) and visits nothing; neither do padded queries of a ragged item.
+constexpr int PRUNE_BATCH = 4;                 // blocks per visit: 32 chunks, one per lane of the lane filter
+constexpr int PRUNED_MAX_WARPS = 16;
+
+__device__ __forceinline__ float prune_lb(float4 lo, float4 hi, float x, float y, float z, float nq) {
+    const float gx = fmaxf(fmaxf(__fsub_rn(lo.x, x), __fsub_rn(x, hi.x)), 0.0f);
+    const float gy = fmaxf(fmaxf(__fsub_rn(lo.y, y), __fsub_rn(y, hi.y)), 0.0f);
+    const float gz = fmaxf(fmaxf(__fsub_rn(lo.z, z), __fsub_rn(z, hi.z)), 0.0f);
+    const float G = __fmaf_rn(gz, gz, __fmaf_rn(gy, gy, __fmul_rn(gx, gx)));
+    if (!(G < 0x1p126f)) return -CUDART_INF_F;
+    return __fsub_rn(__fmul_rn(G, 1.0f - 0x1p-19f), __fmaf_rn(1.2e-6f, __fadd_rn(nq, lo.w), 1e-37f));
+}
+
+// per-warp shared memory: query records [32] float4, staged chunks [32][REC] float4, their ref indices [32 * CHUNK] int,
+// query positions {x, y, z, |q|^2} [32] float4 and thresholds [32] float, heap [k+1][32] u64, candidate buffer
+// [CAND_CAP][32] u16, block list [PRUNE_BATCH] int; a multiple of 128 bytes (the drain's pair un-swizzle XORs addresses)
+static size_t pruned_warp_bytes(int k) {
+    return align_up(32 * 16 + 32 * REC * 16 + 32 * CHUNK * 4 + 32 * 16 + 32 * 4 + (size_t)(k + 1) * 32 * 8 + CAND_CAP * 32 * 2 +
+                    PRUNE_BATCH * 4, 128);
+}
+
+template <int FORM>
+__global__ void __launch_bounds__(PRUNED_MAX_WARPS * 32, 1) pruned_search_kernel(const SearchArgs P) {
+    constexpr unsigned FULL = 0xffffffffu;
+    extern __shared__ __align__(128) unsigned char smem[];
+    const int lane = threadIdx.x & 31, k = P.k;
+    unsigned char *wb = smem + (size_t)(threadIdx.x >> 5) * P.warp_bytes;
+    float4 *qrec = reinterpret_cast<float4 *>(wb);
+    float4 *buf = qrec + 32;
+    int *bidx = reinterpret_cast<int *>(buf + 32 * REC);      // ref index of every staged slot
+    float4 *qpos = reinterpret_cast<float4 *>(bidx + 32 * CHUNK);
+    float *qtau = reinterpret_cast<float *>(qpos + 32);
+    unsigned long long *heap = reinterpret_cast<unsigned long long *>(qtau + 32);
+    unsigned short *cand = reinterpret_cast<unsigned short *>(heap + (size_t)(k + 1) * 32) + lane;
+    int *blist = reinterpret_cast<int *>(cand - lane + CAND_CAP * 32);
+    const uint32_t hb = smem_u32(heap + lane), SB = 32u * 8u;
+    const int gpi = (P.S + 31) >> 5;                   // query groups per item
+    const int nbt = P.n_pad / PRUNE_BLOCK;             // block-table rows per item
+
+    int g = 0;
+    if (lane == 0) g = (int)atomicAdd(P.work, 1u);
+    g = __shfl_sync(FULL, g, 0);
+    while (g < P.B * gpi) {
+        const int b = g / gpi, q0 = (g - b * gpi) * 32, qi = q0 + lane;
+        const int s_b = item_len(P.qry_len, b, P.S);
+        float x = 0.0f, y = 0.0f, z = 0.0f, tau = -CUDART_INF_F;      // dead lane: wants no block, never hits
+        if (qi < s_b) {
+            const float4 qv = __ldg(P.qsorted + (size_t)b * P.S + qi);
+            if (isfinite(qv.x) && isfinite(qv.y) && isfinite(qv.z)) {
+                x = qv.x; y = qv.y; z = qv.z;
+                tau = __ldg(P.seed + (size_t)b * P.S + qi);
+            }
+        }
+        const float nq = torch_sq_norm(x, y, z);
+        qrec[lane] = make_float4(-2.0f * x, -2.0f * y, -2.0f * z, filter_threshold(tau, nq));
+        qpos[lane] = make_float4(x, y, z, nq);
+        qtau[lane] = tau;
+        for (int e = 0; e < k; ++e) heap[e * 32 + lane] = HEAP_SENTINEL;
+        heap[k * 32 + lane] = 0ull;                    // pad: the smallest key, never selected as a child
+        __syncwarp();
+
+        const GridDesc &gd = P.desc[b];
+        const int nblk = (gd.n_finite + PRUNE_BLOCK - 1) / PRUNE_BLOCK;
+        int hi = 0;                                    // home block: where the refs of the cell of the group's middle query end
+        {
+            const int qm = min(q0 + 16, s_b - 1);
+            if (qm >= q0 && nblk > 0) {
+                const float4 qv = __ldg(P.qsorted + (size_t)b * P.S + qm);
+                const unsigned e = __ldg(P.cend + (size_t)b * GRID_MAX_CELLS + grid_cell_index(gd, qv.x, qv.y, qv.z));
+                hi = min((int)(e / PRUNE_BLOCK), nblk - 1);
+            }
+        }
+        int lo = hi - 1;
+        bool up = true;
+        const float4 *table = P.blocks + (size_t)b * nbt * 2;
+        // Window test: lane j takes block 32 w + j and tests it against the 32 queries of the warp (their positions and
+        // current thresholds broadcast from shared memory) -- 32 blocks in flight instead of one.  Bit j of the result: some
+        // lane may need the block.  Thresholds only decrease, so a clear bit stays right; a set bit is tested again, against
+        // the thresholds of the moment, when the walk reaches the block.
+        auto window = [&](const int w) {
+            const int blk = w * 32 + lane;
+            bool want = false;
+            if (blk < nblk) {
+                const float4 blo = __ldg(table + 2 * blk), bhi = __ldg(table + 2 * blk + 1);
+#pragma unroll 8
+                for (int l = 0; l < 32; ++l) {
+                    const float4 qp = qpos[l];
+                    want |= !(prune_lb(blo, bhi, qp.x, qp.y, qp.z, qp.w) > qtau[l]);
+                }
+            }
+            return __ballot_sync(FULL, want);
+        };
+        int wu = -1, wd = -1;                          // windows of the upward and downward cursor, and their bits
+        uint32_t mu = 0u, md = 0u;
+        auto next_block = [&]() {                      // home, home + 1, home - 1, home + 2, ... that passed their window; -1 at the end
+            while (true) {
+                int r = -1;
+                if (hi < nblk && (lo < 0 || up)) {
+                    r = hi++; up = false;
+                    if (r >> 5 != wu) { wu = r >> 5; mu = wu == wd ? md : window(wu); }
+                    if ((mu >> (r & 31)) & 1u) return r;
+                } else if (lo >= 0) {
+                    r = lo--; up = true;
+                    if (r >> 5 != wd) { wd = r >> 5; md = wd == wu ? mu : window(wd); }
+                    if ((md >> (r & 31)) & 1u) return r;
+                } else {
+                    return -1;
+                }
+            }
+        };
+        const float4 *src = P.packed + (size_t)b * P.n_pad;
+
+        // stage the nb listed blocks, filter them against the warp's 32 queries and drain the hits
+        auto visit = [&](const int nb) {
+            __syncwarp();                              // blist is written; the previous drain is done with buf
+            float4 v[8];
+            int ri[8];
+#pragma unroll
+            for (int p = 0; p < 8; ++p) {              // float4 f = 32 p + lane of the batch: block f / 64 = p / 2; slot f too
+                const int f = p * 32 + lane;
+                B200PC_DEV_ASSERT(p / 2 >= nb || (blist[p / 2] >= 0 && blist[p / 2] < nbt));
+                if (p / 2 < nb) {
+                    v[p] = __ldg(src + (size_t)blist[p / 2] * PRUNE_BLOCK + (f & 63));
+                    ri[p] = __ldg(P.perm + (size_t)b * P.n_pad + blist[p / 2] * PRUNE_BLOCK + (f & 63));
+                }
+            }
+#pragma unroll
+            for (int p = 0; p < 8; ++p)
+                if (p / 2 < nb) { buf[p * 32 + lane] = v[p]; bidx[p * 32 + lane] = ri[p]; }
+            __syncwarp();
+            // lane filter (as filter_lanes): lane l keeps chunk l, the ballot of query i is lane i's 32-chunk hit mask
+            float4 R[REC];
+            {
+                const float4 *cb = buf + lane * REC;
+                const int rot = (lane & 3) << 1;
+#pragma unroll
+                for (int p = 0; p < REC; ++p) R[p] = cb[p ^ rot];
+            }
+            uint32_t mine = 0u;
+#pragma unroll FILTER_UNROLL
+            for (int l = 0; l < 32; ++l) {
+                const float4 qv = qrec[l];
+                const float m = chunk_umin(R, splat2(qv.x), splat2(qv.y), splat2(qv.z));
+                if (m < qv.w) mine |= 1u << l;
+            }
+            uint32_t m0 = warp_transpose32(mine, lane) & (nb == PRUNE_BATCH ? FULL : (1u << (nb * 8)) - 1u);
+            // drain (as search_kernel's): phase 1 re-tests the hit chunks ref by ref, phase 2 inserts the survivors
+            const float4 qv = qrec[lane];
+            const float ex = FORM == B200PC_FORM_DIRECT ? 0.5f * qv.x : qv.x, ey = FORM == B200PC_FORM_DIRECT ? 0.5f * qv.y : qv.y,
+                        ez = FORM == B200PC_FORM_DIRECT ? 0.5f * qv.z : qv.z;
+            const f32x2 b0 = splat2(qv.x), b1 = splat2(qv.y), b2 = splat2(qv.z);
+            float thr = qv.w;
+            while (__any_sync(FULL, m0 != 0u)) {
+                int nc = 0;
+                while (__any_sync(FULL, m0 != 0u && nc < CAND_CAP)) {
+                    if (m0 != 0u && nc < CAND_CAP) {
+                        const int cc = __ffs(m0) - 1;
+                        m0 &= m0 - 1;
+                        const float4 *dq = buf + cc * REC + 2 * (cc & 3);
+                        float u[8];
+#pragma unroll
+                        for (int p = 0; p < 4; ++p) {
+                            const float4 *pp = reinterpret_cast<const float4 *>(reinterpret_cast<uintptr_t>(dq) ^ (uintptr_t)(p * 32));
+                            unpack2(pair_u(pp[0], pp[1], b0, b1, b2), u[2 * p], u[2 * p + 1]);
+                        }
+                        uint32_t cm = 0u;
+#pragma unroll
+                        for (int i = 0; i < 8; ++i) cm |= (u[i] < thr) ? (1u << i) : 0u;
+                        if (cm != 0u) { cand[nc * 32] = (unsigned short)((cc << 8) | cm); ++nc; }
+                    }
+                }
+                uint32_t cur = 0u;
+                int e = 0, base = 0;
+                while (true) {
+                    if (cur == 0u && e < nc) {
+                        const uint32_t v = cand[e * 32];
+                        ++e;
+                        cur = v & 0xffu;
+                        base = (int)(v >> 8) * CHUNK;
+                    }
+                    if (!__any_sync(FULL, cur != 0u)) break;
+                    if (cur != 0u) {
+                        const int off = base + __ffs(cur) - 1;
+                        cur &= cur - 1;
+                        const float d = ref_dist<FORM>(buf, off, ex, ey, ez, nq);
+                        if (d <= tau && d < CUDART_INF_F) {      // only finite distances are candidates (see search_kernel)
+                            B200PC_DEV_ASSERT(off >= 0 && off < 32 * CHUNK);
+                            const uint32_t ri = (uint32_t)bidx[off];
+                            B200PC_DEV_ASSERT(ri < (uint32_t)P.N);
+                            if (d < tau || ri < (uint32_t)lds_u64(hb)) {
+                                heap_sift_root<true>(hb, SB, (uint32_t)k * SB, ((unsigned long long)order_key(d) << 32) | ri);
+                                tau = fminf(tau, key_to_float((uint32_t)(lds_u64(hb) >> 32)));
+                            }
+                        }
+                    }
+                }
+                thr = filter_threshold(tau, nq);
+            }
+            reinterpret_cast<float *>(qrec + lane)[3] = filter_threshold(tau, nq);
+            qtau[lane] = tau;
+            __syncwarp();
+        };
+
+        int nb = 0;
+        int cur = next_block();
+        float4 clo = make_float4(0.f, 0.f, 0.f, 0.f), chi = clo;
+        if (cur >= 0) { clo = __ldg(table + 2 * cur); chi = __ldg(table + 2 * cur + 1); }
+        while (cur >= 0) {
+            const int nx = next_block();
+            float4 nlo = clo, nhi = chi;
+            if (nx >= 0) { nlo = __ldg(table + 2 * nx); nhi = __ldg(table + 2 * nx + 1); }   // one block ahead
+            if (__any_sync(FULL, !(prune_lb(clo, chi, x, y, z, nq) > tau))) {
+                if (lane == 0) blist[nb] = cur;
+                ++nb;
+            }
+            if (nb == PRUNE_BATCH || (nx < 0 && nb > 0)) { visit(nb); nb = 0; }
+            cur = nx; clo = nlo; chi = nhi;
+        }
+
+        // results: heapsort, rows of the caller's order (padded rows s_b .. S-1 one to one, as in search_kernel)
+        for (int n = k; n > 1; --n) {
+            const unsigned long long top = lds_u64(hb);
+            const unsigned long long last = lds_u64(hb + (uint32_t)(n - 1) * SB);
+            heap_sift_root<false>(hb, SB, (uint32_t)(n - 1) * SB, last);
+            sts_u64(hb + (uint32_t)(n - 1) * SB, top);
+        }
+        if (qi < P.S) {
+            const size_t row = (size_t)b * P.S + (qi < s_b ? __float_as_int(__ldg(&P.qsorted[(size_t)b * P.S + qi].w)) : qi);
+            B200PC_DEV_ASSERT(row >= (size_t)b * P.S && row < (size_t)(b + 1) * P.S);
+            int64_t *io = P.idx_out ? P.idx_out + row * k : nullptr;
+            int32_t *io32 = P.idx32_out ? P.idx32_out + row * k : nullptr;
+            float *dout = P.dist_out ? P.dist_out + row * k : nullptr;
+            for (int e = 0; e < k; ++e) {
+                const unsigned long long key = heap[e * 32 + lane];
+                if (io) io[e] = (int64_t)(int32_t)(uint32_t)key;
+                if (io32) io32[e] = (int32_t)(uint32_t)key;
+                if (dout) dout[e] = key_to_float((uint32_t)(key >> 32));
+            }
+        }
+        __syncwarp();
+        if (lane == 0) g = (int)atomicAdd(P.work, 1u);
+        g = __shfl_sync(FULL, g, 0);
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
 // 4. merge of partial lists (only when the ref range was split)
 // ---------------------------------------------------------------------------------------------
 // One WARP per query row: lane s holds the head of partial list s (n_split <= 32) as a 64-bit key (order(d) << 32 | index),
@@ -1321,16 +1688,31 @@ static const size_t kFixedSmem = (size_t)STAGES * TILE_BYTES + BAR_BYTES;
 // slots = SMs * CTAs-per-SM.  Among the candidates the one with the best wave efficiency wins;
 // ties go to more resident warps.
 // warm start only where it pays: the grid costs a memset, a bounding-box kernel and one atomic per ref
-// 0: no grid; 1: counts + starting thresholds only (4 small launches); 2: refs and queries sorted by cell as well (7 launches)
+// 0: no grid; 1: counts + starting thresholds only (4 small launches); 2: refs and queries sorted by cell as well (7 launches);
+// 3: sorted in brick order with a block table, pruned per warp (section 3b; 8 launches)
+static bool pruned_fits(int k) { return pruned_warp_bytes(k) <= kMaxSmem - 1024; }
+// the knobs that only mean something to search_kernel: a forced ref split, two queries per thread, exact-box seeds (they
+// walk x-rows of the raster order), the broadcast filter, the no-drain measurement
+static const char *pruned_conflict(const Tuning &tn) {
+    if (tn.force_split > 0) return "B200PC_FORCE_SPLIT";
+    if (tn.force_q > 1) return "B200PC_FORCE_Q";
+    if (tn.seed > 0) return "B200PC_SEED";
+    if (tn.filter == 0) return "B200PC_FILTER=0";
+    if (tn.nodrain) return "B200PC_DEBUG_NODRAIN";
+    return nullptr;
+}
 static int grid_mode(int B, int N, int S, int k) {
     const int g = tuning().grid;
     if (g <= 0) return 0;
-    if (g == 2 || g == 3) return g - 1;                        // forced: 2 = thresholds only, 3 = sorted
+    if (g >= 2 && g <= 4) return g - 1;                        // forced: 2 = thresholds only, 3 = sorted, 4 = pruned
     // measured (tools/grid_probe.py): a nearest-neighbour search (k = 1) inserts too little to pay for any of it; the sorted
     // variant wins where the drain is a large part of a long search (C2: -12 %, k = 64: -28 %) and loses its three extra
     // launches on the short ones (fusion search of one frame pair, three-NN)
     if (k < 3 || N < 2048 || (long)B * N * S < GRID_MIN_PAIRS) return 0;
-    return k >= 8 && (long)B * N * S >= GRID_SORT_MIN_PAIRS ? 2 : 1;
+    if (k < 8 || (long)B * N * S < GRID_SORT_MIN_PAIRS) return 1;
+    // the pruned search visits ~6 % of the pairs at C2 (measured, B200: C2 0.63 -> 0.45 ms of search, 2 x 16384^2 -10 %,
+    // 32 x 8192^2 -31 %, k = 64 -10 %); a knob that forces a search_kernel plan keeps the brute-force order
+    return pruned_fits(k) && !pruned_conflict(tuning()) ? 3 : 2;
 }
 
 bool plan_search(int B, int N, int S, int k, int mode, SearchPlan *pl) {
@@ -1429,9 +1811,26 @@ bool plan_search(int B, int N, int S, int k, int mode, SearchPlan *pl) {
     // grid path of a top-k search (section 1b): counters, cell-sorted copies of refs and queries, one starting threshold per query
     pl->grid_bytes = 0;
     pl->grid_sorted = 0;
-    if (mode == MODE_TOPK && grid_mode(B, N, S, k)) {
+    pl->grid_pruned = 0;
+    const int gm = mode == MODE_TOPK ? grid_mode(B, N, S, k) : 0;
+    if (gm) {
         pl->grid_bytes = grid_layout(B, N, S, pl->n_pad, nullptr, nullptr);
-        pl->grid_sorted = grid_mode(B, N, S, k) == 2;
+        pl->grid_sorted = gm >= 2;
+        pl->grid_pruned = gm == 3;
+    }
+    if (pl->grid_pruned) {
+        // persistent warps of 32 queries each, as many per CTA as the shared memory takes (16 at k = 16); no ref split
+        if (!pruned_fits(k)) return false;
+        int w = (int)((kMaxSmem - 1024) / pruned_warp_bytes(k));
+        if (w > PRUNED_MAX_WARPS) w = PRUNED_MAX_WARPS;
+        if (force_w > 0 && force_w < w) w = force_w;
+        pl->q_per_thread = 1;
+        pl->consumer_warps = w;
+        pl->q_per_block = 32 * w;
+        pl->tiles_per_split = pl->n_tiles;
+        pl->n_split = 1;
+        pl->smem_bytes = (size_t)w * pruned_warp_bytes(k);
+        pl->part_bytes = 0;
     }
     pl->total_bytes = pl->packed_bytes + pl->part_bytes + pl->grid_bytes;
     return true;
@@ -1453,6 +1852,22 @@ static int launch_shape(const SearchArgs &a, const SearchPlan &pl, int B, cudaSt
     return launch_one<FORM, MODE, 1>(a, pl, B, st);
 }
 
+// persistent: as many CTAs as are resident at once (never more than there are query groups); warps take groups off a counter
+template <int FORM>
+static int launch_pruned(const SearchArgs &a, const SearchPlan &pl, int B, cudaStream_t st) {
+    auto kern = pruned_search_kernel<FORM>;
+    B200PC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pl.smem_bytes));
+    int per_sm = 0;
+    B200PC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, pl.consumer_warps * 32, pl.smem_bytes));
+    const long groups = (long)B * ((a.S + 31) / 32);
+    long ctas = (long)sm_count() * (per_sm > 1 ? per_sm : 1);
+    const long need = (groups + pl.consumer_warps - 1) / pl.consumer_warps;
+    if (ctas > need) ctas = need;
+    kern<<<(unsigned)ctas, pl.consumer_warps * 32, pl.smem_bytes, st>>>(a);
+    B200PC_LAUNCH_CHECK();
+    return B200PC_OK;
+}
+
 // ref_len / qry_len: [B] device lengths of a ragged batch (top-k only), or null.  The plan and the workspace are those of
 // the padded shape.
 static int run_search(const float *ref, const float *qry, const int64_t *ref_len, const int64_t *qry_len, int B, int N, int S, int k,
@@ -1464,6 +1879,12 @@ static int run_search(const float *ref, const float *qry, const int64_t *ref_len
     if (!idx32) {   // small reference sets: warp-per-query kernel, one launch, no workspace (small_search.cu)
         const int rc_small = run_small(ref, qry, ref_len, qry_len, B, N, S, k, form, mode, r2, idx, dist, st);
         if (rc_small != -100) return rc_small;
+    }
+    const Tuning &tn = tuning();
+    if (mode == MODE_TOPK && tn.grid == 4 && pruned_conflict(tn)) {
+        set_error("search: the pruned search (B200PC_GRID=4) runs one query per lane over its own block list and cannot honour %s",
+                  pruned_conflict(tn));
+        return B200PC_EINVAL;
     }
     SearchPlan pl;
     if (!plan_search(B, N, S, k, mode, &pl)) {
@@ -1482,7 +1903,6 @@ static int run_search(const float *ref, const float *qry, const int64_t *ref_len
     // top-k: refs dealt out to the tiles in a strided order (see slot_to_ref).  Not for form 1: its only caller is three-NN
     // feature propagation, whose reference points are FPS picks -- an order that is already ideal for a running k-best
     // (every prefix is a well-spread sample; measured 0.32 ms natural vs 0.36 ms strided on C3).
-    const Tuning &tn = tuning();
     const int strided = mode == MODE_TOPK && (tn.natural_order >= 0 ? tn.natural_order == 0 : form != B200PC_FORM_QRY_NORM_FIRST);
     GridBufs gb{};
     int strided_eff = strided;
@@ -1498,13 +1918,18 @@ static int run_search(const float *ref, const float *qry, const int64_t *ref_len
         // count -> pyramid + segment sums -> scan -> scatter (sorted copies, packed tiles, slot table) -> starting thresholds
         grid_count_kernel<<<dim3((N + S + 255) / 256, B), 256, 0, st>>>(ref, ref_len, N, qry, qry_len, S, gb.desc, gb.counts, gb.qcend);
         B200PC_LAUNCH_CHECK();
-        grid_pyramid_kernel<<<dim3(GRID_SEGS, B, 2), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.qcend, gb.qseg);
+        grid_pyramid_kernel<<<dim3(GRID_SEGS, B, 2), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.qcend, gb.qseg, pl.grid_pruned);
         B200PC_LAUNCH_CHECK();
-        grid_scan_kernel<<<dim3(GRID_SEGS, B, 2), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.cend, gb.qcend, gb.qseg);
+        grid_scan_kernel<<<dim3(GRID_SEGS, B, 2), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.cend, gb.qcend, gb.qseg, pl.grid_pruned);
         B200PC_LAUNCH_CHECK();
-        grid_scatter_kernel<<<dim3((pl.n_pad + S + 255) / 256, B), 256, 0, st>>>(ref, ref_len, N, pl.n_pad, pl.tiles_per_split, qry, qry_len, S,
-                                                                                  gb.desc, gb, packed, tn.seed > 0 ? 0 : k);
+        // pruned: one tile per "split" makes sorted_slot the identity, so that 64 consecutive slots are 64 consecutive sorted refs
+        grid_scatter_kernel<<<dim3((pl.n_pad + S + 255) / 256, B), 256, 0, st>>>(ref, ref_len, N, pl.n_pad, pl.grid_pruned ? 1 : pl.tiles_per_split,
+                                                                                  qry, qry_len, S, gb.desc, gb, packed, tn.seed > 0 ? 0 : k);
         B200PC_LAUNCH_CHECK();
+        if (pl.grid_pruned) {
+            grid_block_kernel<<<dim3((pl.n_pad / PRUNE_BLOCK * 32 + 255) / 256, B), 256, 0, st>>>(packed, pl.n_pad, gb.desc, gb.blocks);
+            B200PC_LAUNCH_CHECK();
+        }
         if (tn.seed > 0) {                               // thresholds from the refs inside the boxes (A/B: B200PC_SEED=n); else the scatter wrote them
             grid_seed_kernel<<<dim3((S + SEED_THREADS - 1) / SEED_THREADS, B), SEED_THREADS, 0, st>>>(gb.qsorted, nullptr, qry_len, S, N, k, gb.desc, gb.counts,
                                                                                                 gb.cend, gb.sorted, gb.seed, tn.seed);
@@ -1516,7 +1941,7 @@ static int run_search(const float *ref, const float *qry, const int64_t *ref_len
         pack_refs_kernel<<<grid, 256, 0, st>>>(ref, ref_len, N, pl.n_pad, strided, packed, pl.grid_bytes ? gb.desc : nullptr, gb.counts);
         B200PC_LAUNCH_CHECK();
         if (pl.grid_bytes) {                              // thresholds only: the caller's order of refs and queries stays
-            grid_pyramid_kernel<<<dim3(GRID_SEGS, B, 1), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.qcend, gb.qseg);
+            grid_pyramid_kernel<<<dim3(GRID_SEGS, B, 1), 256, 0, st>>>(gb.desc, gb.counts, gb.seg, gb.qcend, gb.qseg, 0);
             B200PC_LAUNCH_CHECK();
             grid_seed_kernel<<<dim3((S + SEED_THREADS - 1) / SEED_THREADS, B), SEED_THREADS, 0, st>>>(nullptr, qry, qry_len, S, N, k, gb.desc, gb.counts, gb.cend,
                                                                                                 gb.sorted, gb.seed, 0);
@@ -1531,6 +1956,8 @@ static int run_search(const float *ref, const float *qry, const int64_t *ref_len
     a.debug_nodrain = tn.nodrain;
     a.lane_filter = tn.filter >= 0 ? tn.filter != 0 : 1;                          // 0: A/B measurement only
     a.qsorted = gb.qsorted; a.seed = gb.seed; a.perm = gb.perm; a.interleave = tn.interleave == 1;
+    a.B = B; a.blocks = gb.blocks; a.desc = gb.desc; a.cend = gb.cend; a.work = gb.tail ? gb.tail + B : nullptr;
+    a.warp_bytes = (int)pruned_warp_bytes(k);
     a.idx_out = idx; a.idx32_out = idx32; a.dist_out = dist; a.part_d = nullptr; a.part_i = nullptr; a.part_cnt = nullptr;
     if (pl.n_split > 1) {
         const size_t rows = (size_t)B * S * pl.n_split;
@@ -1542,10 +1969,14 @@ static int run_search(const float *ref, const float *qry, const int64_t *ref_len
     if (tn.debug_plan)   // order: the ref order inside the tiles (strided: slot_to_ref; cell: sorted_slot)
         fprintf(stderr, "b200pc plan: B=%d N=%d S=%d k=%d mode=%d -> %d warps/CTA, %d queries/CTA, ref split %d (%d tiles each), grid %s, "
                 "filter %s, order %s, %zu B smem\n", B, N, S, k, mode, pl.consumer_warps, pl.q_per_block, pl.n_split, pl.tiles_per_split,
-                pl.grid_bytes ? (pl.grid_sorted ? "sorted" : "thresholds") : "off", a.lane_filter ? "lane" : "broadcast",
+                pl.grid_bytes ? (pl.grid_pruned ? "pruned" : pl.grid_sorted ? "sorted" : "thresholds") : "off", a.lane_filter ? "lane" : "broadcast",
                 pl.grid_sorted ? "cell" : strided_eff ? "strided" : "natural", pl.smem_bytes);
     int rc;
-    if (mode == MODE_BALL) rc = launch_shape<B200PC_FORM_QRY_NORM_FIRST, MODE_BALL>(a, pl, B, st);
+    if (pl.grid_pruned) {
+        if (form == B200PC_FORM_REF_NORM_FIRST) rc = launch_pruned<B200PC_FORM_REF_NORM_FIRST>(a, pl, B, st);
+        else if (form == B200PC_FORM_QRY_NORM_FIRST) rc = launch_pruned<B200PC_FORM_QRY_NORM_FIRST>(a, pl, B, st);
+        else rc = launch_pruned<B200PC_FORM_DIRECT>(a, pl, B, st);
+    } else if (mode == MODE_BALL) rc = launch_shape<B200PC_FORM_QRY_NORM_FIRST, MODE_BALL>(a, pl, B, st);
     else if (form == B200PC_FORM_REF_NORM_FIRST) rc = launch_shape<B200PC_FORM_REF_NORM_FIRST, MODE_TOPK>(a, pl, B, st);
     else if (form == B200PC_FORM_QRY_NORM_FIRST) rc = launch_shape<B200PC_FORM_QRY_NORM_FIRST, MODE_TOPK>(a, pl, B, st);
     else rc = launch_shape<B200PC_FORM_DIRECT, MODE_TOPK>(a, pl, B, st);

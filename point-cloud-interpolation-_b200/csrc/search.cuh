@@ -29,6 +29,7 @@ struct SearchPlan {
     size_t part_bytes;    // workspace: partial lists (n_split > 1)
     size_t grid_bytes;    // workspace: occupancy grid (counters, sorted copies, starting thresholds) of a warm-started top-k search, else 0
     int grid_sorted;      // 1: refs and queries are visited in cell order (search.cu section 1b)
+    int grid_pruned;      // 1: ... in brick order, each warp visiting only the ref blocks that can hold a neighbour (section 3b)
     size_t total_bytes;
 };
 

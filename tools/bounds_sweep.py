@@ -34,7 +34,7 @@ for B, N, S, k in ((2, 3000, 700, 16), (1, 513, 31, 3), (3, 1000, 777, 1), (1, 5
     a, b = synth.batch_pairs(11, B, max(N, S))
     ref, qry = t(a[:, :N]), t(b[:, :S])
     for kw in (dict(), dict(GRID=0, SMALL_PATH=0), dict(GRID=2, SMALL_PATH=0), dict(GRID=3, SMALL_PATH=0), dict(GRID=3, SMALL_PATH=0, INTERLEAVE=1, SEED=5),
-               dict(GRID=3, SMALL_PATH=0, SEED=2, FORCE_SPLIT=3), dict(SMALL_PATH=1)):
+               dict(GRID=3, SMALL_PATH=0, SEED=2, FORCE_SPLIT=3), dict(GRID=4, SMALL_PATH=0), dict(GRID=4, SMALL_PATH=0, FORCE_WARPS=3), dict(SMALL_PATH=1)):
         env(**kw)
         for form in (0, 1, 2):
             ops.knn_search(ref, qry, k, form, want_dist=True)
@@ -43,21 +43,24 @@ for B, N, S, k in ((2, 3000, 700, 16), (1, 513, 31, 3), (3, 1000, 777, 1), (1, 5
     env()
 bad_r, bad_q = a[:, :N].copy(), b[:, :S].copy()
 bad_r[0, 7] = np.nan; bad_r[0, 99, 2] = np.inf; bad_q[0, 3] = np.nan
-for kw in (dict(), dict(GRID=3, SMALL_PATH=0), dict(GRID=2, SMALL_PATH=0)):
+for kw in (dict(), dict(GRID=3, SMALL_PATH=0), dict(GRID=2, SMALL_PATH=0), dict(GRID=4, SMALL_PATH=0)):
     env(**kw); ops.knn_search(t(bad_r), t(bad_q), 16, 0, want_dist=True); P.query_ball_point(1.0, 16, t(bad_r), t(bad_q))
 # k above the finite count on the small path (rows end in -1), and a split range (tile 1 of the strided order, 2 tiles)
 # holding only non-finite refs; (+inf, 0, 0) is the query whose filter value is -inf for refs with x > 0
 few = bad_r[:1, :900].copy(); few[0, 8:] = np.nan
 half = bad_r[:1, :1000].copy(); half[0, 1::2] = np.inf
 bq = bad_q[:1, :64].copy(); bq[0, 5] = [np.inf, 0.0, 0.0]
-for kw, cloud in ((dict(SMALL_PATH=1), few), (dict(SMALL_PATH=0, GRID=0, FORCE_SPLIT=2), half), (dict(SMALL_PATH=0, GRID=3), half)):
+for kw, cloud in ((dict(SMALL_PATH=1), few), (dict(SMALL_PATH=0, GRID=0, FORCE_SPLIT=2), half), (dict(SMALL_PATH=0, GRID=3), half),
+                   (dict(SMALL_PATH=0, GRID=4), half), (dict(SMALL_PATH=0, GRID=4), few)):
     env(**kw)
     for form in (0, 1, 2):
         ops.knn_search(t(cloud), t(bq), 16, form, want_dist=True); ops.knn_search_i32(t(cloud), t(bq), 16, form)
     ops.chamfer(t(cloud), t(bq)); ops.fusion_group(t(bq), t(cloud), 16, t(cloud))
 env()
 same = np.repeat(np.array([[[1.5, -2.0, 0.25]]], np.float32), 900, axis=1)
-env(GRID=3, SMALL_PATH=0); ops.knn_search(t(same), t(b[:1, :100]), 7, 0); env()
+for grid in (3, 4):
+    env(GRID=grid, SMALL_PATH=0); ops.knn_search(t(same), t(b[:1, :100]), 7, 0)
+env()
 # forced plans (tests/test_gpu_plans.py): every split a range count can come from, short and ragged ranges, k above the refs
 # of a range, warps per CTA with empty trailing warps, two queries per thread, the broadcast filter and the natural order
 for (B, N, S, k), splits in (((1, 513, 77, 300), (2,)), ((2, 2048, 333, 600), (3, 4)), ((1, 5000, 700, 16), (3, 4, 5, 7, 8)),
