@@ -1718,7 +1718,9 @@ static int grid_mode(int B, int N, int S, int k) {
 bool plan_search(int B, int N, int S, int k, int mode, SearchPlan *pl) {
     const int sms = sm_count();
     const size_t qb = query_bytes(k, mode);
-    if (kFixedSmem + 32 * qb > kMaxSmem) return false;   // not even one warp of queries fits
+    // the pruned search keeps no ref tiles in shared memory and takes longer lists (k <= 876) than search_kernel (k <= 774)
+    const int gm = mode == MODE_TOPK ? grid_mode(B, N, S, k) : 0;
+    if (!(gm == 3 && pruned_fits(k)) && kFixedSmem + 32 * qb > kMaxSmem) return false;   // not even one warp of queries fits
     pl->n_pad = (int)align_up((size_t)N, TILE);
     pl->n_tiles = pl->n_pad / TILE;
 
@@ -1812,7 +1814,6 @@ bool plan_search(int B, int N, int S, int k, int mode, SearchPlan *pl) {
     pl->grid_bytes = 0;
     pl->grid_sorted = 0;
     pl->grid_pruned = 0;
-    const int gm = mode == MODE_TOPK ? grid_mode(B, N, S, k) : 0;
     if (gm) {
         pl->grid_bytes = grid_layout(B, N, S, pl->n_pad, nullptr, nullptr);
         pl->grid_sorted = gm >= 2;
