@@ -151,12 +151,15 @@ int b200pc_feature_propagation(const float *unknown, const float *known, const f
 
 /* ---- a3: farthest_point_sample(xyz, npoint)  Utils/Pointnet2Utils.py:64-85 --------------- */
 /* start [B] int64: the first centroid of each cloud (the facade draws it with torch.randint
- * on the CPU generator exactly as the reference does).  idx [B,npoint] int64.                */
+ * on the CPU generator exactly as the reference does).  idx [B,npoint] int64.
+ * N <= 262144 points per cloud (B200PC_EINVAL above; one thread-block cluster holds a cloud on
+ * chip).  The workspace arguments are ignored.                                              */
 int b200pc_fps(const float *xyz, int B, int N, int npoint, const int64_t *start, int64_t *idx, void *workspace,
                size_t workspace_bytes, b200pc_stream_t stream);
 
 /* a7: Sample.forward (Utils/Layers.py:23-27) = farthest_point_sample + index_points(points, ind) behind one call:
- * idx [B,npoint] and the picks' coordinates new_xyz [B,npoint,3] (the FPS kernel followed by the gather kernel).     */
+ * idx [B,npoint] and the picks' coordinates new_xyz [B,npoint,3] (the FPS kernel followed by the gather kernel).
+ * Same per-cloud limit as b200pc_fps: N <= 262144.                                                                  */
 int b200pc_fps_sample(const float *xyz, int B, int N, int npoint, const int64_t *start, int64_t *idx, float *new_xyz,
                       b200pc_stream_t stream);
 

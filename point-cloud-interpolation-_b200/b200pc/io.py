@@ -6,7 +6,7 @@ Dataset/InterpolationData.py:141-147, PolyPCI/Dataset/Dataset.py:165-172) or `.r
 PointINet20230424/data/interpolation_data.py:34) and down-sample every frame to `npoints` with open3d's
 `farthest_point_down_sample` on the host -- 2*field+3 frames per training sample, ~34 700 -> 16 000 points each, the input
 pipeline's bottleneck.  Here the sweep is uploaded once and the a3 kernel (one thread-block cluster per cloud, up to
-131 072 points) picks the samples; a batch of sweeps runs as one launch, one cluster per sweep.
+262 144 points: a full HDL-64 sweep of 133 312 returns, or a 128-beam x 2 048-column one) picks the samples; a batch of sweeps runs as one launch, one cluster per sweep.
 
 Arithmetic: the kernel computes what the reference's own `farthest_point_sample` computes (fp32,
 (dx*dx + dy*dy) + dz*dz, first arg-max) -- bit-exact against the strict CPU checker used by the tests.  open3d's implementation starts at point 0

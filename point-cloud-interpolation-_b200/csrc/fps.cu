@@ -5,6 +5,8 @@
 // thread-block CLUSTER owns one cloud for the whole loop:
 //   * every thread keeps P points (x,y,z,min-dist) in REGISTERS for all rounds; 512 threads x
 //     P<=16 = 8192 points per CTA, up to 16 CTAs per cluster (131072 points);
+//   * larger clouds, up to 262144 points, run the wide tier (fps_wide_kernel): every CTA holds up to
+//     8192 more points in shared memory, their running minima still in registers;
 //   * the update is packed fp32x2 math in the reference's exact rounding order
 //     d = ((dx*dx + dy*dy) + dz*dz), dx = x - cx, every product rounded on its own (SURVEY Appendix A.5);
 //   * arg-max: min-dists are >= +0, so their bit patterns order like unsigned ints:
@@ -35,6 +37,73 @@ struct __align__(16) FpsRecord {  // what a CTA tells its peers each round
     float x, y, z;      // its coordinates
     int pad[3];
 };
+
+// ---- round steps shared by the FPS kernels ----
+
+// running-min update of P points against the last pick, reference rounding order, two points per instruction; returns the
+// largest running minimum of the P points
+template <int P>
+__device__ __forceinline__ float fps_update(const float (&x)[P], const float (&y)[P], const float (&z)[P], float (&mind)[P],
+                                            float cx, float cy, float cz) {
+    float lmax = 0.f;
+    if (P >= 2) {
+        const f32x2 ncx = splat2(-cx), ncy = splat2(-cy), ncz = splat2(-cz);
+#pragma unroll
+        for (int p = 0; p < P; p += 2) {
+            const f32x2 dx = add2(pack2(x[p], x[p + 1]), ncx);
+            const f32x2 dy = add2(pack2(y[p], y[p + 1]), ncy);
+            const f32x2 dz = add2(pack2(z[p], z[p + 1]), ncz);
+            // Only the subtractions stay packed.  ptxas 12.9 contracts mul.rn.f32x2 feeding add.rn.f32x2 into FFMA2 (it even
+            // folds fma(d, d, -0.0) back to a product first), which would turn the reference's (dx*dx + dy*dy) + dz*dz into
+            // fma(dz,dz,fma(dy,dy,dx*dx)) and flip near-tied arg-max picks.  The scalar .rn intrinsics are never
+            // contracted (tests/test_abi.py and tests/test_gpu_fps_large.py check the SASS of every FPS kernel: no FFMA2, no
+            // FMUL2, no FFMA).
+            float ax, bx, ay, by, az, bz;
+            unpack2(dx, ax, bx); unpack2(dy, ay, by); unpack2(dz, az, bz);
+            const float d0 = __fadd_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay)), __fmul_rn(az, az));
+            const float d1 = __fadd_rn(__fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by)), __fmul_rn(bz, bz));
+            mind[p] = fminf(mind[p], d0);
+            mind[p + 1] = fminf(mind[p + 1], d1);
+            lmax = fmaxf(lmax, fmaxf(mind[p], mind[p + 1]));
+        }
+    } else {
+        const float dx = __fadd_rn(x[0], -cx), dy = __fadd_rn(y[0], -cy), dz = __fadd_rn(z[0], -cz);
+        const float d = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
+        mind[0] = fminf(mind[0], d);
+        lmax = mind[0];
+    }
+    return lmax;
+}
+
+// cluster arg-max: all-to-all of one 32-byte record through DSMEM.  Each record is pushed with st.async, which completes
+// bytes on the RECEIVER's mbarrier: no cluster-wide barrier and no membar per round, only the DSMEM latency.  rec / bar are
+// this round's slots (they alternate with round parity, `phase` = (round >> 1) & 1).  Every warp then picks the winner among
+// the C records in parallel: lane r holds record r, two REDUX give (max bits, lowest index), one ballot finds the lane that
+// owns it.  This CTA's candidate is point ci, local slot cl of the lookup copy sx / sy / sz.  -> the winner's index; its
+// coordinates in cx, cy, cz
+__device__ __forceinline__ int fps_cluster_argmax(FpsRecord *rec, unsigned long long *bar, uint32_t phase, int C, int rank, int t,
+                                                  int lane, unsigned int cbits, int ci, const float *sx, const float *sy,
+                                                  const float *sz, int cl, float &cx, float &cy, float &cz) {
+    const uint32_t my_bar = smem_u32(bar);
+    if (t == 0) mbar_expect_tx(my_bar, (uint32_t)(C * sizeof(FpsRecord)));   // C records will land here
+    if (t < C) {
+        const uint32_t dst = map_to_rank(smem_u32(&rec[rank]), (uint32_t)t);
+        const uint32_t rbar = map_to_rank(my_bar, (uint32_t)t);
+        st_async_v4(dst, cbits, (uint32_t)ci, __float_as_uint(sx[cl]), __float_as_uint(sy[cl]), rbar);
+        st_async_v4(dst + 16, __float_as_uint(sz[cl]), 0u, 0u, 0u, rbar);
+    }
+    mbar_wait_cluster(my_bar, phase);
+    const FpsRecord mine = rec[lane < C ? lane : 0];
+    const unsigned int vb = lane < C ? mine.bits : 0u;
+    const unsigned int bb = __reduce_max_sync(0xffffffffu, vb);
+    const unsigned int vinv = (lane < C && vb == bb) ? 0xffffffffu - (unsigned int)mine.idx : 0u;
+    const unsigned int binv = __reduce_max_sync(0xffffffffu, vinv);
+    const int src = __ffs(__ballot_sync(0xffffffffu, lane < C && vb == bb && vinv == binv)) - 1;
+    cx = __shfl_sync(0xffffffffu, mine.x, src);
+    cy = __shfl_sync(0xffffffffu, mine.y, src);
+    cz = __shfl_sync(0xffffffffu, mine.z, src);
+    return (int)(0xffffffffu - binv);
+}
 
 template <int P>
 __global__ void __launch_bounds__(FPS_T) fps_kernel(const float *__restrict__ xyz, int N, int npoint,
@@ -89,32 +158,7 @@ __global__ void __launch_bounds__(FPS_T) fps_kernel(const float *__restrict__ xy
         if (it == npoint - 1) break;  // the last pick needs no further update
 
         // ---- running-min update, reference rounding order, two points per instruction ----
-        float lmax = 0.f;
-        if (P >= 2) {
-            const f32x2 ncx = splat2(-cx), ncy = splat2(-cy), ncz = splat2(-cz);
-#pragma unroll
-            for (int p = 0; p < P; p += 2) {
-                const f32x2 dx = add2(pack2(x[p], x[p + 1]), ncx);
-                const f32x2 dy = add2(pack2(y[p], y[p + 1]), ncy);
-                const f32x2 dz = add2(pack2(z[p], z[p + 1]), ncz);
-                // Only the subtractions stay packed.  ptxas 12.9 contracts mul.rn.f32x2 feeding add.rn.f32x2 into FFMA2 (it even
-                // folds fma(d, d, -0.0) back to a product first), which would turn the reference's (dx*dx + dy*dy) + dz*dz into
-                // fma(dz,dz,fma(dy,dy,dx*dx)) and flip near-tied arg-max picks.  The scalar .rn intrinsics are never
-                // contracted (tests/test_abi.py checks the SASS of every fps_kernel: no FFMA2, no FMUL2, no FFMA).
-                float ax, bx, ay, by, az, bz;
-                unpack2(dx, ax, bx); unpack2(dy, ay, by); unpack2(dz, az, bz);
-                const float d0 = __fadd_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay)), __fmul_rn(az, az));
-                const float d1 = __fadd_rn(__fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by)), __fmul_rn(bz, bz));
-                mind[p] = fminf(mind[p], d0);
-                mind[p + 1] = fminf(mind[p + 1], d1);
-                lmax = fmaxf(lmax, fmaxf(mind[p], mind[p + 1]));
-            }
-        } else {
-            const float dx = __fadd_rn(x[0], -cx), dy = __fadd_rn(y[0], -cy), dz = __fadd_rn(z[0], -cz);
-            const float d = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
-            mind[0] = fminf(mind[0], d);
-            lmax = mind[0];
-        }
+        const float lmax = fps_update<P>(x, y, z, mind, cx, cy, cz);
 
         TICK(0)
         // ---- block arg-max (first index) with ONE barrier: the pair (max bits, ~index) is reduced as a
@@ -142,32 +186,9 @@ __global__ void __launch_bounds__(FPS_T) fps_kernel(const float *__restrict__ xy
             far = ci;
             cx = sx[cl]; cy = sy[cl]; cz = sz[cl];
         } else {
-            // ---- cluster arg-max: all-to-all of one 32-byte record through DSMEM.  Each record is pushed
-            // with st.async, which completes bytes on the RECEIVER's mbarrier: no cluster-wide barrier and
-            // no membar per round, only the DSMEM latency.  Slots / barriers alternate with round parity.
             const int par = it & 1;
-            const uint32_t my_bar = smem_u32(&xbar[par]);
-            if (t == 0) mbar_expect_tx(my_bar, (uint32_t)(C * sizeof(FpsRecord)));   // C records will land here
-            if (t < C) {
-                const uint32_t dst = map_to_rank(smem_u32(&rec[par][rank]), (uint32_t)t);
-                const uint32_t rbar = map_to_rank(my_bar, (uint32_t)t);
-                st_async_v4(dst, cbits, (uint32_t)ci, __float_as_uint(sx[cl]), __float_as_uint(sy[cl]), rbar);
-                st_async_v4(dst + 16, __float_as_uint(sz[cl]), 0u, 0u, 0u, rbar);
-            }
-            mbar_wait_cluster(my_bar, (uint32_t)((it >> 1) & 1));
-            // every warp picks the winner among the C records in parallel: lane r holds record r,
-            // two REDUX give (max bits, lowest index), one ballot finds the lane that owns it
-            const FpsRecord mine = rec[par][lane < C ? lane : 0];
-            const unsigned int vb = lane < C ? mine.bits : 0u;
-            const unsigned int bb = __reduce_max_sync(0xffffffffu, vb);
-            const unsigned int vinv = (lane < C && vb == bb) ? 0xffffffffu - (unsigned int)mine.idx : 0u;
-            const unsigned int binv = __reduce_max_sync(0xffffffffu, vinv);
-            const int src = __ffs(__ballot_sync(0xffffffffu, lane < C && vb == bb && vinv == binv)) - 1;
-            const int bi = (int)(0xffffffffu - binv);
-            cx = __shfl_sync(0xffffffffu, mine.x, src);
-            cy = __shfl_sync(0xffffffffu, mine.y, src);
-            cz = __shfl_sync(0xffffffffu, mine.z, src);
-            far = bi;
+            far = fps_cluster_argmax(rec[par], &xbar[par], (uint32_t)((it >> 1) & 1), C, rank, t, lane, cbits, ci, sx, sy, sz, cl,
+                                     cx, cy, cz);
         }
         TICK(4)
     }
@@ -236,29 +257,8 @@ __global__ void __launch_bounds__(FPS_T) fps_flat_kernel(const float *__restrict
         if (rank == 0 && t == 0) out[(size_t)b * npoint + it] = far;
         if (it == npoint - 1) break;  // the last pick needs no further update
 
-        // ---- running-min update, reference rounding order (every product rounded on its own: see fps_kernel) ----
-        float lmax = 0.f;
-        if (P >= 2) {
-            const f32x2 ncx = splat2(-cx), ncy = splat2(-cy), ncz = splat2(-cz);
-#pragma unroll
-            for (int p = 0; p < P; p += 2) {
-                const f32x2 dx = add2(pack2(x[p], x[p + 1]), ncx);
-                const f32x2 dy = add2(pack2(y[p], y[p + 1]), ncy);
-                const f32x2 dz = add2(pack2(z[p], z[p + 1]), ncz);
-                float ax, bx, ay, by, az, bz;
-                unpack2(dx, ax, bx); unpack2(dy, ay, by); unpack2(dz, az, bz);
-                const float d0 = __fadd_rn(__fadd_rn(__fmul_rn(ax, ax), __fmul_rn(ay, ay)), __fmul_rn(az, az));
-                const float d1 = __fadd_rn(__fadd_rn(__fmul_rn(bx, bx), __fmul_rn(by, by)), __fmul_rn(bz, bz));
-                mind[p] = fminf(mind[p], d0);
-                mind[p + 1] = fminf(mind[p + 1], d1);
-                lmax = fmaxf(lmax, fmaxf(mind[p], mind[p + 1]));
-            }
-        } else {
-            const float dx = __fadd_rn(x[0], -cx), dy = __fadd_rn(y[0], -cy), dz = __fadd_rn(z[0], -cz);
-            const float d = __fadd_rn(__fadd_rn(__fmul_rn(dx, dx), __fmul_rn(dy, dy)), __fmul_rn(dz, dz));
-            mind[0] = fminf(mind[0], d);
-            lmax = mind[0];
-        }
+        // ---- running-min update, reference rounding order (every product rounded on its own: see fps_update) ----
+        const float lmax = fps_update<P>(x, y, z, mind, cx, cy, cz);
         int lp = 0;
 #pragma unroll
         for (int p = P - 1; p >= 0; --p)
@@ -332,8 +332,149 @@ static int launch_fps(const float *xyz, int B, int N, int npoint, const int64_t 
     return B200PC_OK;
 }
 
-// cluster size and points-per-thread for a cloud of N points in a batch of B
-static void fps_shape(int B, int N, int *C_out, int *P_out) {
+// ------------------------------------------------------------------------------------------------------------------
+// Wide tier: clouds the registers of one cluster cannot hold (131 073 .. 262 144 points by default), still one cluster of
+// C CTAs per cloud, all state on chip and no workspace.  Every CTA owns a contiguous slice of S = ceil(N / C) points: the
+// first 8 192 live in registers as in fps_kernel<16>, the other S - 8 192 (at most 8 192, Q per thread) in shared memory.
+// Their coordinates are the tail of the x/y/z lookup copy every CTA keeps anyway (3 * 512 * (16 + Q) floats, 196 608 bytes
+// at Q = 16); their running minima stay in registers, Q more per thread.  Balancing the slices keeps the shared part small
+// for clouds just above the register capacity: a 133 312-point sweep puts 140 points per CTA there (Q = 1).
+// Slot s of thread t (s < 16: register point s, s >= 16: shared point s - 16) is point base + s * 512 + t of the cloud, so
+// a thread's slots are in index order and its first local arg-max is the lowest index.  Slots at or past the slice's end are
+// padding with min-dist 0: they tie only when every real point has min-dist 0, and then point 0 of the cloud wins.
+// Arithmetic (fps_update), tie rule and the two-level exchange are those of fps_kernel: the picks are identical.
+// ------------------------------------------------------------------------------------------------------------------
+constexpr int FPS_WIDE_P = 16;                          // register points per thread
+constexpr int FPS_WIDE_MAX_Q = 16;                      // shared-memory points per thread
+constexpr int FPS_MAX_N = FPS_MAX_CLUSTER * FPS_T * (FPS_WIDE_P + FPS_WIDE_MAX_Q);   // 262 144
+
+template <int Q>
+__global__ void __launch_bounds__(FPS_T) fps_wide_kernel(const float *__restrict__ xyz, int N, int npoint,
+                                                         const int64_t *__restrict__ start, int64_t *__restrict__ out) {
+    constexpr int P = FPS_WIDE_P, L = FPS_T * (P + Q);  // L: slots per CTA
+    cg::cluster_group cluster = cg::this_cluster();
+    const int C = (int)cluster.num_blocks();
+    const int rank = (int)cluster.block_rank();
+    const int b = blockIdx.y;
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    const int S = (N + C - 1) / C;
+    const int base = rank * S;                          // first point of this CTA's slice
+    const int len = min(S, N - base);                   // points in the slice; slots from len on are padding
+    B200PC_DEV_ASSERT(len > 0 && len <= L);
+
+    extern __shared__ __align__(16) float fps_smem[];
+    float *sx = fps_smem, *sy = sx + L, *sz = sy + L;
+    __shared__ uint2 warp_key[2][FPS_WARPS];
+    __shared__ FpsRecord rec[2][FPS_MAX_CLUSTER];
+    __shared__ __align__(8) unsigned long long xbar[2];
+
+    const float *cloud = xyz + (size_t)b * N * 3;
+    float x[P], y[P], z[P], mind[P], qmind[Q];
+#pragma unroll
+    for (int s = 0; s < P + Q; ++s) {
+        const int l = s * FPS_T + t;
+        float px = 0.f, py = 0.f, pz = 0.f, m = 0.f;
+        if (l < len) {
+            const int i = base + l;
+            B200PC_DEV_ASSERT(i < N);
+            px = cloud[i * 3 + 0]; py = cloud[i * 3 + 1]; pz = cloud[i * 3 + 2];
+            m = 1e10f;
+        }
+        sx[l] = px; sy[l] = py; sz[l] = pz;
+        if (s < P) { x[s] = px; y[s] = py; z[s] = pz; mind[s] = m; }
+        else qmind[s - P] = m;
+    }
+    if (t == 0) {
+        mbar_init(smem_u32(&xbar[0]), 1); mbar_init(smem_u32(&xbar[1]), 1);
+        mbar_fence_init();
+    }
+    int far = (int)start[b];
+    far = far < 0 ? 0 : (far >= N ? N - 1 : far);      // a bad start index must not read outside the cloud
+    float cx = cloud[far * 3 + 0], cy = cloud[far * 3 + 1], cz = cloud[far * 3 + 2];
+    if (C > 1) cluster.sync(); else __syncthreads();   // barriers initialised, shared points stored
+
+    for (int it = 0; it < npoint; ++it) {
+        B200PC_DEV_ASSERT(far >= 0 && far < N);
+        if (rank == 0 && t == 0) out[(size_t)b * npoint + it] = far;
+        if (it == npoint - 1) break;  // the last pick needs no further update
+
+        // ---- running-min update of the register points, then of the shared-memory points ----
+        float qx[Q], qy[Q], qz[Q];
+#pragma unroll
+        for (int q = 0; q < Q; ++q) {
+            const int l = (P + q) * FPS_T + t;
+            qx[q] = sx[l]; qy[q] = sy[l]; qz[q] = sz[l];
+        }
+        const float lmax = fmaxf(fps_update<P>(x, y, z, mind, cx, cy, cz), fps_update<Q>(qx, qy, qz, qmind, cx, cy, cz));
+
+        // ---- block arg-max over the global index (as in fps_kernel): shared slots follow the register slots of a thread ----
+        int ls = 0;
+#pragma unroll
+        for (int q = Q - 1; q >= 0; --q)
+            if (qmind[q] == lmax) ls = P + q;
+#pragma unroll
+        for (int p = P - 1; p >= 0; --p)
+            if (mind[p] == lmax) ls = p;                       // first local slot attaining the local max
+        const unsigned int lbits = __float_as_uint(lmax);
+        const unsigned int linv = 0xffffffffu - (unsigned int)(base + ls * FPS_T + t);   // larger = lower index
+        const unsigned int wbits = __reduce_max_sync(0xffffffffu, lbits);
+        const unsigned int winv = __reduce_max_sync(0xffffffffu, lbits == wbits ? linv : 0u);
+        if (lane == 0) warp_key[it & 1][warp] = make_uint2(wbits, winv);
+        __syncthreads();
+        const uint2 wk = warp_key[it & 1][lane & (FPS_WARPS - 1)];
+        const unsigned int cbits = __reduce_max_sync(0xffffffffu, wk.x);
+        const unsigned int cinv = __reduce_max_sync(0xffffffffu, wk.x == cbits ? wk.y : 0u);
+        const int ci = (int)(0xffffffffu - cinv);
+        const int cl = ci - base;
+        B200PC_DEV_ASSERT(cl >= 0 && cl < len);
+
+        if (C == 1) {
+            far = ci;
+            cx = sx[cl]; cy = sy[cl]; cz = sz[cl];
+        } else {
+            const int par = it & 1;
+            far = fps_cluster_argmax(rec[par], &xbar[par], (uint32_t)((it >> 1) & 1), C, rank, t, lane, cbits, ci, sx, sy, sz, cl,
+                                     cx, cy, cz);
+        }
+    }
+    if (C > 1) cluster.sync();  // nobody exits while a peer may still write into its shared memory
+}
+
+template <int Q>
+static int launch_fps_wide(const float *xyz, int B, int N, int npoint, const int64_t *start, int64_t *idx, int C,
+                           cudaStream_t st) {
+    auto kern = fps_wide_kernel<Q>;
+    const size_t smem = (size_t)3 * FPS_T * (FPS_WIDE_P + Q) * sizeof(float);
+    B200PC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (C > 8) B200PC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(C, B, 1);
+    cfg.blockDim = dim3(FPS_T, 1, 1);
+    cfg.dynamicSmemBytes = smem;
+    cfg.stream = st;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeClusterDimension;
+    attr[0].val.clusterDim.x = C; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+    cfg.attrs = attr; cfg.numAttrs = 1;
+    // one CTA per SM at this much shared memory: a device (or a partition of one) without C such SMs in one GPC cannot run
+    // the cluster at all, so ask before launching instead of failing at launch
+    int clusters = 0;
+    B200PC_CUDA(cudaOccupancyMaxActiveClusters(&clusters, kern, &cfg));
+    if (clusters < 1) {
+        set_error("fps: N=%d needs a cluster of %d CTAs with %zu bytes of dynamic shared memory each, which this device cannot "
+                  "schedule", N, C, smem);
+        return B200PC_ECUDA;
+    }
+    if (tuning().debug_plan)
+        fprintf(stderr, "b200pc fps wide tier: at most %d clusters of %d CTAs co-resident, %zu bytes of dynamic shared memory per CTA\n",
+                clusters, C, smem);
+    B200PC_CUDA(cudaLaunchKernelEx(&cfg, kern, xyz, N, npoint, start, idx));
+    return B200PC_OK;
+}
+
+// cluster size C, register points per thread P and shared-memory points per thread Q (0: fps_kernel / fps_flat_kernel,
+// >= 1: fps_wide_kernel) for a cloud of N points in a batch of B
+static void fps_shape(int B, int N, int *C_out, int *P_out, int *Q_out) {
     const int sms = sm_count();
     // Measured (tools/fps_timing_probe.py, tools/fps_time.py): a single CTA needs ~560 cycles per round plus ~12 per
     // point held by a thread; a cluster adds ~600-750 cycles of DSMEM exchange.  So one CTA whenever the cloud fits
@@ -343,13 +484,19 @@ static void fps_shape(int B, int N, int *C_out, int *P_out) {
     while (C < FPS_MAX_CLUSTER && (long)C * FPS_T * 16 < N) C *= 2;
     if (C > 1)
         while (C < 8 && (long)B * C * 4 <= sms && (long)C * FPS_T * 4 < N) C *= 2;
-    {   // tuning override (cached; not part of the ABI)
+    {   // tuning override (cached; not part of the ABI); a cluster too small for the cloud in registers runs the wide tier
         const int f = tuning().fps_cluster;
-        if (f >= 1 && f <= FPS_MAX_CLUSTER && (long)f * FPS_T * 16 >= N) C = f;
+        if (f >= 1 && f <= FPS_MAX_CLUSTER && (long)f * FPS_T * (FPS_WIDE_P + FPS_WIDE_MAX_Q) >= N) C = f;
     }
-    int P = 1;
-    while ((long)C * FPS_T * P < N) P *= 2;
-    *C_out = C; *P_out = P;
+    int P = 1, Q = 0;
+    if ((long)C * FPS_T * FPS_WIDE_P < N) {             // wide tier: 16 register points per thread, the rest of a slice shared
+        const int shared_points = (N + C - 1) / C - FPS_T * FPS_WIDE_P;
+        P = FPS_WIDE_P; Q = 1;
+        while (FPS_T * Q < shared_points) Q *= 2;
+    } else {
+        while ((long)C * FPS_T * P < N) P *= 2;
+    }
+    *C_out = C; *P_out = P; *Q_out = Q;
 }
 
 }  // namespace b200pc
@@ -361,21 +508,35 @@ extern "C" size_t b200pc_fps_workspace_bytes(int, int) { return 256; }
 extern "C" int b200pc_fps(const float *xyz, int B, int N, int npoint, const int64_t *start, int64_t *idx, void *,
                           size_t, b200pc_stream_t stream) {
     B200PC_REQUIRE(B >= 0 && N >= 1 && npoint >= 0, "fps: bad sizes B=%d N=%d npoint=%d", B, N, npoint);
-    B200PC_REQUIRE((long)N <= (long)FPS_MAX_CLUSTER * FPS_T * 16, "fps: N=%d exceeds the %d points one cluster can hold",
-                   N, FPS_MAX_CLUSTER * FPS_T * 16);
+    B200PC_REQUIRE(N <= FPS_MAX_N, "fps: N=%d exceeds the %d points one cluster can hold", N, FPS_MAX_N);
     if (B == 0 || npoint == 0) return B200PC_OK;
     B200PC_REQUIRE(xyz && start && idx, "fps: null pointer");
-    int C, P;
-    fps_shape(B, N, &C, &P);
+    int C, P, Q;
+    fps_shape(B, N, &C, &P, &Q);
     cudaStream_t st = as_stream(stream);
     // Measured at 16 384 points (tools/fps_sweep.py, us per round, two-level / flat): C=2 0.98 / 1.05, C=4 0.75 / 0.67,
     // C=8 0.62 / 0.68, C=16 0.63 / 0.94; one CTA 0.29 / 0.50.  The flat exchange wins exactly where the cluster is 4 CTAs
-    // (batches of >= 10 clouds, e.g. C3: 3.05 -> 2.70 ms); everywhere else the two-level kernel stays.
+    // (batches of >= 10 clouds, e.g. C3: 3.05 -> 2.70 ms); everywhere else the two-level kernel stays.  The wide tier
+    // always exchanges in two levels.
     const int flat = tuning().fps_flat;
-    const bool use_flat = flat > 0 || (flat < 0 && C == 4);
-    if (tuning().debug_plan)
-        fprintf(stderr, "b200pc fps plan: B=%d N=%d npoint=%d -> cluster %d, %d points/thread, exchange %s\n", B, N, npoint, C, P,
-                use_flat ? "flat" : "two-level");
+    const bool use_flat = Q == 0 && (flat > 0 || (flat < 0 && C == 4));
+    if (tuning().debug_plan) {
+        if (Q == 0)
+            fprintf(stderr, "b200pc fps plan: B=%d N=%d npoint=%d -> cluster %d, %d points/thread, exchange %s\n", B, N, npoint, C,
+                    P, use_flat ? "flat" : "two-level");
+        else
+            fprintf(stderr, "b200pc fps plan: B=%d N=%d npoint=%d -> cluster %d, %d points/thread, exchange two-level, shared %d "
+                    "points/thread\n", B, N, npoint, C, P, Q);
+    }
+    if (Q > 0) {
+        switch (Q) {
+            case 1: return launch_fps_wide<1>(xyz, B, N, npoint, start, idx, C, st);
+            case 2: return launch_fps_wide<2>(xyz, B, N, npoint, start, idx, C, st);
+            case 4: return launch_fps_wide<4>(xyz, B, N, npoint, start, idx, C, st);
+            case 8: return launch_fps_wide<8>(xyz, B, N, npoint, start, idx, C, st);
+            default: return launch_fps_wide<16>(xyz, B, N, npoint, start, idx, C, st);
+        }
+    }
     if (use_flat) {
         switch (P) {
             case 1: return launch_fps_flat<1>(xyz, B, N, npoint, start, idx, C, st);

@@ -100,6 +100,15 @@ for kw in (dict(), dict(FPS_FLAT=1), dict(FPS_FLAT=0), dict(FPS_CLUSTER=2), dict
     for n, m in ((16384, 300), (12000, 64), (3000, 128), (40, 7)):
         ops.fps(big[:, :n].contiguous(), m, torch.tensor([1, n - 1], device=dev))
 env()
+# the wide tier (registers + shared memory per CTA): the default plan just above 131 072 points and at the 262 144 limit,
+# then forced clusters at small N, every shared-memory width Q = 1 .. 16, ragged last slices, starts at both ends
+wide = t(np.concatenate([a.reshape(-1, 3), b.reshape(-1, 3)] * 5)[None, :262144])
+for n, m in ((140000, 300), (262144, 64)):
+    ops.fps(wide[:, :n].contiguous().expand(2, -1, -1).contiguous(), m, torch.tensor([0, n - 1], device=dev))
+for C, n in ((1, 8193), (1, 9000), (1, 10000), (1, 12288), (1, 12289), (1, 16384), (2, 20000), (3, 30001), (4, 60000), (8, 100000), (16, 262144)):
+    env(FPS_CLUSTER=C)
+    ops.fps(wide[:, :n].contiguous().expand(2, -1, -1).contiguous(), min(n, 5000), torch.tensor([1, n - 1], device=dev))
+env()
 ref = big[:, :3000].contiguous(); qry = t(b[:, :700])
 fi = ops.fps(ref, 64, torch.tensor([1, 2], device=dev))
 for C in (3, 32, 36, 128, 257):
