@@ -443,6 +443,8 @@ def _fusion_group(qry, ref, feat, k):
 def _channel_max(x):
     rows, Cc = x.shape
     out = _f32(rows, like=x)
+    if x.data_ptr() % 16:       # the kernel reads each row as float4s: a view that starts between 16-byte boundaries
+        x = x.clone()           # (a slice of a flat buffer) is copied into a fresh, aligned block first
     _call(x.device, _lib.load().b200pc_channel_max, _ptr(x), rows, Cc, _ptr(out), _stream(x.device))
     return out
 
@@ -739,7 +741,8 @@ def fusion_group(qry, ref, k, feat=None):
 
 def channel_max(x):
     """x [rows, C] (channels-last rows of PointsFusion's point-wise MLP) -> [rows] = max over the channels
-    (`torch.max(new_features, dim=1)`, Utils/Layers.py:276)"""
+    (`torch.max(new_features, dim=1)`, Utils/Layers.py:276).  Any storage offset: the op copies a view that is not
+    16-byte aligned before its vector kernel reads it."""
     x = _prep(x, "x")
     if x.dim() != 2 or x.shape[1] % 4:
         return x.max(dim=1)[0]

@@ -48,8 +48,8 @@ def knn_points(p1, p2, lengths1=None, lengths2=None, norm=2, K=1, version=-1, re
     K = min(int(K), p2.shape[1])
     if K <= 0 or p1.shape[1] == 0:
         B, P1 = p1.shape[0], p1.shape[1]
-        z = p1.new_zeros(B, P1, 0)
-        return _KNN(z, z.long(), p1.new_zeros(B, P1, 0, 3) if return_nn else None)
+        z = torch.zeros(B, P1, 0, dtype=torch.float32, device=p1.device)             # fp32 out, like every other path
+        return _KNN(z, z.long(), torch.zeros(B, P1, 0, 3, dtype=torch.float32, device=p1.device) if return_nn else None)
     grad = torch.is_grad_enabled() and (p1.requires_grad or p2.requires_grad)
     if lengths1 is None and lengths2 is None:
         idx, dists = ops.knn_search(p2.detach(), p1.detach(), K, ops.FORM_DIRECT, want_dist=True)

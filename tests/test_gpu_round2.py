@@ -176,24 +176,6 @@ def test_loader_fps_on_device(cuda_dev, tmp_path):
             np.testing.assert_array_equal(idx[i].cpu().numpy(), want)
 
 
-def test_torch_ops_pass_opcheck(cuda_dev):
-    """torch.library.opcheck on the registered ops: schema, fake kernel and autograd registration agree with what the CUDA
-    implementation (the C-ABI call) really returns"""
-    g = torch.Generator().manual_seed(11)
-    ref = torch.randn(2, 300, 3, generator=g).to(cuda_dev); qry = torch.randn(2, 70, 3, generator=g).to(cuda_dev)
-    feat = torch.randn(2, 300, 16, generator=g).to(cuda_dev)
-    idx = torch.ops.b200pc.knn(ref, qry, 4, 0, False)[0]
-    tests = ("test_schema", "test_faketensor", "test_autograd_registration")
-    torch.library.opcheck(torch.ops.b200pc.knn, (ref, qry, 4, 0, True), test_utils=tests)
-    torch.library.opcheck(torch.ops.b200pc.ball_query, (ref, qry, 0.5, 8), test_utils=tests)
-    torch.library.opcheck(torch.ops.b200pc.gather, (feat.clone().requires_grad_(True), idx.reshape(2, -1), False), test_utils=tests)
-    torch.library.opcheck(torch.ops.b200pc.group_points, (ref, qry, feat.clone().requires_grad_(True), idx, True), test_utils=tests)
-    torch.library.opcheck(torch.ops.b200pc.fusion_group, (qry, ref, feat, 4), test_utils=tests)
-    sf = torch.randn(2, 70, 8, generator=g).to(cuda_dev).requires_grad_(True)
-    torch.library.opcheck(torch.ops.b200pc.feature_propagation, (ref, qry, sf, 0), test_utils=tests)
-    torch.library.opcheck(torch.ops.b200pc.chamfer_fwd, (ref.clone().requires_grad_(True), qry.clone().requires_grad_(True)), test_utils=tests)
-
-
 def test_error_behaviour_of_the_new_entries(cuda_dev):
     ref = torch.randn(1, 10, 3, device=cuda_dev); qry = torch.randn(1, 4, 3, device=cuda_dev)
     # fusion_group clamps k to the number of refs like pytorch3d.knn_points (K = min(K, P2))
